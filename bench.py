@@ -6,15 +6,16 @@ Workload (config C4 of BASELINE.json, one GPU's share): 125,000 columns x 8760 h
 config C3 instead (Bushland record, 100,000-member parameter ensemble, forward only).  Weak scaling: every
 rank draws its own shard; no data-path collective (columns are independent).
 
-A bench "step" is ONE TIME SEGMENT of the record: the whole shard advanced through ceil(T / steps)
-consecutive forcing rows by one persistent launch (`lgar_problem.step_begin/step_end`, continuing from the
-column state the previous launch left in the workspace -- the way the reference's training loop feeds
+A bench "step" is ONE TIME SEGMENT of the record: the whole shard advanced through ceil(T / steps) or
+floor(T / steps) consecutive forcing rows (steps <= T) by one persistent launch (`lgar_problem.step_begin/step_end`,
+continuing from the column state the previous launch left in the workspace -- the way the reference's training loop feeds
 dpLGAR.forward one row after the other, agents/DifferentiableLGAR.py:117-125).  The K timed steps together
 are exactly ONE pass over the full record (results bit-identical to a single launch: tests/test_gpu_bench_path.py);
 the W warm-up steps run the first W segments and the timed pass then restarts from the initial state.
 
   python bench.py --gpus 1 --steps K --warmup W            # CUDA path (this repo)
   python bench.py --impl reference ...                     # the reference on the box's host cores
+  python bench.py ... --dump-outputs DIR                   # + what the last timed step returned, as DIR/*.npy
 
 `value`   : whole-job column-timesteps/s, inputs resident in HBM, CUDA-event time, max over ranks.  Only
             column-steps that were actually simulated count: a column the reference would abort with an
@@ -76,7 +77,16 @@ def parse():
                     help="A/B: every rank draws its own site records too (shards then differ in work by several per cent)")
     ap.add_argument("--grad-columns", type=int, default=-1,
                     help="columns of the shard used for the forward+gradient figure (-1 = the whole shard, 0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (at most 64 MB in all, a sample "
+                         "with a fixed seed where the shard does not fit, sampled indices beside it); rank 0's shard")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl b200)")
+    if args.impl == "b200" and args.steps > args.nsteps:
+        ap.error("--steps must not exceed --nsteps: every timed step advances the shard by at least one forcing row")
     if args.columns <= 0:
         args.columns = 125_000 if args.workload == "c4" else 100_000
     if args.workload == "c3":
@@ -85,7 +95,6 @@ def parse():
             args.grad_columns = 0  # C3 is forward only (BASELINE.json configs[2])
     if args.grad_columns < 0:
         args.grad_columns = args.columns
-    args.steps = max(1, args.steps)
     return args
 
 
@@ -109,8 +118,63 @@ def make_workload(args, rank):
 
 
 def segments(T, steps):
-    seg = -(-T // steps)
-    return [(i * seg, min(T, (i + 1) * seg)) for i in range(steps) if i * seg < T]
+    """min(steps, T) consecutive non-empty windows [t0, t1) that cover the record once; the first is the longest."""
+    k = min(steps, T)
+    b = [-(-i * T // k) for i in range(k + 1)]
+    return list(zip(b[:-1], b[1:]))
+
+
+DUMP_BYTES = 63 * 10**6  # array data; the .npy headers fit in what is left of 64 MB
+
+
+def _sample(n, k, seed):
+    """Sorted indices of k of range(n), drawn with a fixed seed; all of range(n) when k >= n."""
+    if k >= n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, max(k, 1), replace=False))
+
+
+def dump_outputs(path, res, window, outs):
+    """--dump-outputs: what the last timed step returned to its caller, as .npy files of at most DUMP_BYTES in all.
+    Per column (indices in `columns`): `status`, `crash_step`, `start_volume` and `sums` [10, C] (running totals of all
+    outputs since row 0).  Per step: the series `outs` over the step's window, one [rows, C'] file each (absolute rows
+    in `series_rows`, columns in `series_columns`).  Where a whole array does not fit, a sample drawn from the shape
+    alone with a fixed seed stands for it, so that two builds run with the same arguments write the same elements
+    whatever their results.  A column the reference aborts has no values from its crash step on, which the library
+    marks NaN: every float array is written as float64 with such entries set to 0, beside a float32 `<name>_nonfinite`
+    that is 1 exactly there, so the files hold finite numbers and lose nothing."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    dev = res.status.device
+    B, nout = res.status.numel(), res.sums.shape[0]
+
+    def save(name, v, dtype=torch.float64):
+        np.save(os.path.join(path, f"{name}.npy"), v.to(dtype).cpu().numpy())
+
+    def save_values(name, v):
+        finite = torch.isfinite(v)
+        save(name, torch.where(finite, v, torch.zeros_like(v)))
+        save(f"{name}_nonfinite", ~finite, torch.float32)
+
+    def sample(n, k, seed):
+        return torch.from_numpy(_sample(n, k, seed)).to(dev)
+
+    per_column = 8 * (3 + nout + 1) + 4 * (1 + nout)  # status, crash step, start volume, sums, index; two masks
+    cols = sample(B, DUMP_BYTES // 2 // per_column, seed=1)
+    save("columns", cols)
+    save("status", res.status.index_select(0, cols))
+    save("crash_step", res.crash_step.index_select(0, cols))
+    save_values("start_volume", res.start_volume.index_select(0, cols))
+    save_values("sums", res.sums.index_select(1, cols))
+    left = DUMP_BYTES - per_column * cols.numel()
+    t0, t1 = window
+    per_element = 12 * len(outs)  # float64 value + float32 mask of every series
+    rows = t0 + sample(t1 - t0, (left - 8) // (per_element + 8), seed=2)  # leaves room for at least one column
+    series_cols = sample(B, (left - 8 * rows.numel()) // (per_element * rows.numel() + 8), seed=3)
+    save("series_rows", rows)
+    save("series_columns", series_cols)
+    for name in outs:
+        save_values(name, res[name].index_select(0, rows).index_select(1, series_cols))
 
 
 def alive_steps_of(status, crash, T):
@@ -435,6 +499,8 @@ def main():
     alive_steps = int(alive_cols.sum())
     hist = {lgar_b200.STATUS_NAMES[s]: int((status == s).sum()) for s in np.unique(status)}
     flop_per_pass = flop_per_col_step * alive_steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, segs[-1], outs)
 
     # ---- parity of the first columns against the oracle results of the cpu_baseline leg ----------------------------
     parity = None

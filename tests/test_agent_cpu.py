@@ -1,9 +1,8 @@
 """CPU tests of the calibration agent's host logic (lgar_b200.agent, SURVEY 8f N2): the derived time configuration,
-the loss functions and NSE against the reference's own (imported when /root/reference is present, pinned numbers
-otherwise), the mass-balance report, checkpoint save / load, and the world-size-2 gloo gradient all-reduce.  The
-model is a small differentiable stand-in with the dpLGAR surface (the kernels need a GPU: tests/test_gpu_agent.py)."""
+the loss functions and NSE against numbers worked out by hand from the reference's definitions, the mass-balance
+report, checkpoint save / load, and the world-size-2 gloo gradient all-reduce.  The model is a small differentiable
+stand-in with the dpLGAR surface (the kernels need a GPU: tests/test_gpu_agent.py)."""
 import os
-import sys
 from types import SimpleNamespace
 
 import numpy as np
@@ -81,14 +80,6 @@ def test_losses_and_nse():
     y, t = torch.tensor([0.1, 0.4, 0.2]), torch.tensor([0.0, 0.5, 0.1])
     assert float(A.mse_loss(y, t)) == pytest.approx(0.01)
     assert A.calculate_nse(y.numpy(), t.numpy()) == pytest.approx(1 - 0.03 / float(((t - t.mean()) ** 2).sum()))
-    if os.path.isdir("/root/reference/dpLGAR"):  # the reference's own functions, when available (build container)
-        sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "pyref_stub"))
-        sys.path.insert(0, "/root/reference")
-        from dpLGAR.models.functions.loss import RangeBoundLoss as RefRB, MSE_loss
-        from dpLGAR.data.metrics import calculate_nse as ref_nse
-        assert float(RefRB(LB, UB)([alpha, n, ks, pdm])) == pytest.approx(got, rel=1e-14)
-        assert float(MSE_loss(y, t)) == pytest.approx(float(A.mse_loss(y, t)), rel=1e-15)
-        assert ref_nse(y.numpy(), t.numpy()) == pytest.approx(A.calculate_nse(y.numpy(), t.numpy()), rel=1e-15)
 
 
 def test_reference_observations_are_the_seeded_series():

@@ -1,8 +1,5 @@
 """CPU: forcing loader formats (SURVEY 8f N3)."""
-import os
-
 import numpy as np
-import pytest
 
 import lgar_b200
 from lgar_b200 import forcing
@@ -20,13 +17,3 @@ def test_three_formats(tmp_path):
     np.testing.assert_allclose(forcing.read_forcing(str(c)), [[0, 0], [5.0, 0.05]])
     s = forcing.stack_sites([forcing.read_forcing(str(a)), forcing.read_forcing(str(b))], pin=False)
     assert tuple(s.shape) == (2, 2, 2)
-
-
-@pytest.mark.skipif(not os.path.exists("/root/reference/data"), reason="reference data only in the build container")
-def test_matches_golden_forcing():
-    from conftest import load_golden
-    g = load_golden("phil_year")
-    x = forcing.read_forcing("/root/reference/data/forcing_data_resampled_uniform_Phillipsburg.csv")
-    np.testing.assert_array_equal(x[:8760], g["forcing"])
-    g = load_golden("synth_1")
-    np.testing.assert_array_equal(forcing.read_forcing("/root/reference/data/forcing_data_synth_1.txt"), g["forcing"])

@@ -3,6 +3,7 @@
 * A record advanced window by window (lgar_problem.step_begin / step_end, the bench's "steps") gives the bits of ONE
   launch over the whole record: per-step series, sums, status, crash step -- for windows that do not align with the
   scheduler's chunks, and for the window sizes the bench uses.
+* bench.py --dump-outputs writes the bits of the timed pass's last window.
 * lgar_forward_host (the host-pointer entry of the C ABI) gives the bits of the device-pointer entry.
 * The C ABI rejects windows that cannot work (no resume, keep_checkpoints, out of range)."""
 import ctypes as C
@@ -72,6 +73,52 @@ def test_pipelined_windows_equal_one_launch(B, chunk):
         assert torch.equal(res.per_step.view(torch.int64), full.per_step.view(torch.int64))
         c = res.crash_step.cpu().numpy()
         np.testing.assert_array_equal(np.where(c <= -2, -2 - c, c), full.crash_step.cpu().numpy())
+
+
+def test_bench_steps_and_dumped_outputs(tmp_path):
+    """bench.py --steps K times K launches, and --dump-outputs writes what the last one returned: the rows of its window
+    and the per-column results, equal to one launch over the whole record of the same shard and placement."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from lgar_b200 import forward_raw, workloads, ColumnEnsemble
+    import bench
+    B, T, K, sites = 4096, 240, 7, 4
+    root = os.path.dirname(os.path.abspath(bench.__file__))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", str(K), "--warmup", "2",
+                          "--columns", str(B), "--nsteps", str(T), "--sites", str(sites), "--no-cpu-baseline", "--no-e2e",
+                          "--grad-columns", "0", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900, cwd=root)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == K and line["gpu_launches"] == K
+    we = workloads.synthetic_sites_ensemble(B=B, T=T, sites=sites, rank=0, shared_sites=True)
+    ens = ColumnEnsemble(theta_r=we.theta_r, theta_e=we.theta_e, thickness=we.thickness, forcing=we.forcing,
+                         site_index=we.site_index, max_fronts=16, chunk_steps=64, device="cuda:0")
+    ksat = torch.from_numpy(we.ksat).cuda()
+    ens.balance(ksat)
+    full, _ = forward_raw(ens, we.alpha, we.n, ksat, outputs=("runoff", "AET"))
+    torch.cuda.synchronize()
+    t0 = bench.segments(T, K)[-1][0]
+    bits = lambda a: np.ascontiguousarray(a).view(np.int64)
+    load = lambda f: np.load(tmp_path / f"{f}.npy")
+    assert all(np.isfinite(np.load(f)).all() for f in tmp_path.iterdir())
+    status = full.status.cpu().numpy()
+    assert 0 < (status == 0).sum() < B, "the case must contain crashing columns"
+    # all 4096 columns and every row of the last window fit
+    np.testing.assert_array_equal(load("columns"), np.arange(B))
+    np.testing.assert_array_equal(load("series_columns"), np.arange(B))
+    np.testing.assert_array_equal(load("series_rows"), np.arange(t0, T))
+    np.testing.assert_array_equal(load("status"), status)
+    c = load("crash_step")
+    np.testing.assert_array_equal(np.where(c <= -2, -2 - c, c), full.crash_step.cpu().numpy())
+    for name, want in (("start_volume", full.start_volume), ("sums", full.sums),
+                       ("runoff", full["runoff"][t0:]), ("AET", full["AET"][t0:])):
+        want = want.cpu().numpy()
+        missing = load(f"{name}_nonfinite") == 1
+        np.testing.assert_array_equal(missing, ~np.isfinite(want))  # the NaN after a crash step, exactly there
+        np.testing.assert_array_equal(bits(load(name)[~missing]), bits(want[~missing]))
 
 
 def test_window_argument_checks():
