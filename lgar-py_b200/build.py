@@ -36,8 +36,6 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
     if not force and not _stale():
         return LIB
     flags = list(NVCC_FLAGS)
-    if os.path.exists(os.path.join(CSRC, "lgar_backward.cuh")):
-        flags += ["-DLGAR_WITH_BACKWARD"]
     if verbose:
         flags += ["-Xptxas", "-v"]
     flags += os.environ.get("LGAR_EXTRA_NVCC_FLAGS", "").split()  # developer A/B switches

@@ -21,9 +21,10 @@
 // Tapes and adjoints live in global memory (L2), laid out lane-fastest so the 32 lanes of a warp
 // touch consecutive addresses when they are at the same entry.  The root finders are
 // straight-through (they never appear on the tape); Geff is one macro entry whose partials are
-// evaluated cooperatively by the warp.  (A first version recomputed the chunk in plain fp64 and
-// replayed each sub-step on the tape afterwards; carrying both code paths made the kernel 50k
-// instructions and instruction-fetch bound: `no_instruction` 3.8 stalls per issue in ncu.)
+// evaluated together with its value, one request per lane (geff_batch_eval_taped).  (A first
+// version recomputed the chunk in plain fp64 and replayed each sub-step on the tape afterwards;
+// carrying both code paths made the kernel 50k instructions and instruction-fetch bound:
+// `no_instruction` 3.8 stalls per issue in ncu.)
 // =====================================================================================
 #pragma once
 #include "lgar_forward.cuh"
@@ -119,8 +120,8 @@ template <int FM, int GM>
 __global__ void __launch_bounds__(NT, 2) lgar_backward_kernel(const BParams P) {  // 2 CTAs per SM: up to 255 registers
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* sm_fields = reinterpret_cast<double*>(smem_raw);                       // [5*FM][NT]
-  double* sm_nodes = sm_fields + 5 * FM * NT;                                    // [WARPS][NODEBUF_TAPED]
-  short* sm_ids = reinterpret_cast<short*>(sm_nodes + WARPS * NODEBUF_TAPED);          // [5*FM][NT]
+  double* sm_nodes = sm_fields + 5 * FM * NT;                                    // [WARPS][NODEBUF]
+  short* sm_ids = reinterpret_cast<short*>(sm_nodes + WARPS * NODEBUF);          // [5*FM][NT]
   uint8_t* sm_flags = reinterpret_cast<uint8_t*>(sm_ids + 5 * FM * NT);          // [FM][NT]
   __shared__ unsigned long long sm_item[WARPS];
   pow_tables_to_shared();
@@ -130,7 +131,7 @@ __global__ void __launch_bounds__(NT, 2) lgar_backward_kernel(const BParams P) {
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   const int slot = blockIdx.x * WARPS + warp;  // resident-warp scratch slot
-  double* nodebuf = sm_nodes + warp * NODEBUF_TAPED;
+  double* nodebuf = sm_nodes + warp * NODEBUF;
   const int Tn = p.num_steps, S = p.num_subcycles;
   const size_t B = p.num_columns;
   constexpr int NL = num_leaves<FM>();

@@ -25,7 +25,7 @@ template <int FM, int GM>
 static int launch_backward(BParams& P, int S, int chunk, int slots, int arena_cap, int step_cap, int num_sms,
                            unsigned char* scratch, cudaStream_t st, char* err, size_t errlen) {
   auto kern = lgar_backward_kernel<FM, GM>;
-  const size_t smem = (size_t)5 * FM * NT * sizeof(double) + (size_t)WARPS * NODEBUF_TAPED * sizeof(double) +
+  const size_t smem = (size_t)5 * FM * NT * sizeof(double) + (size_t)WARPS * NODEBUF * sizeof(double) +
                       (size_t)5 * FM * NT * sizeof(short) + (size_t)FM * NT;
   BW_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;

@@ -8,9 +8,7 @@
 #include <vector>
 
 #include "lgar_forward.cuh"
-#ifdef LGAR_WITH_BACKWARD
 #include "lgar_backward.cuh"
-#endif
 
 namespace {
 
@@ -216,11 +214,9 @@ struct DevBuf {
 }  // namespace
 
 
-#ifdef LGAR_WITH_BACKWARD
 // the reverse kernel is compiled in its own translation unit (lgar_backward_launch.cu)
 int lgar_reverse_unit_launch(int FM, void* params, int S, int chunk, int slots, int arena_cap, int step_cap, int num_sms,
                              unsigned char* scratch, void* stream, char* err, size_t errlen);
-#endif
 
 extern "C" {
 
@@ -250,10 +246,8 @@ size_t lgar_workspace_bytes(const lgar_problem* p, int with_grad) {
     return 0;
   }
   size_t total = carve(s, with_grad).total;
-#ifdef LGAR_WITH_BACKWARD
   if (with_grad)
     total += lgar::backward_scratch_bytes(s.S, s.FM, s.chunk, backward_slots(s), backward_arena_cap(s), LGAR_TAPE_CAP, s.ntiles);
-#endif
   return total;
 }
 
@@ -339,7 +333,6 @@ int lgar_forward(const lgar_problem* p, const lgar_outputs* out, void* workspace
   return rc;
 }
 
-#ifdef LGAR_WITH_BACKWARD
 int lgar_backward_ex(const lgar_problem* p, const lgar_gradients* g, void* workspace_dev, size_t workspace_bytes,
                      void* stream) {
   Shape s;
@@ -411,17 +404,6 @@ int lgar_backward(const lgar_problem* p, const double* grad_per_step, uint32_t g
   g.grad_ksat = grad_ksat;
   return lgar_backward_ex(p, &g, workspace_dev, workspace_bytes, stream);
 }
-#endif
-
-#ifndef LGAR_WITH_BACKWARD
-int lgar_backward(const lgar_problem*, const double*, uint32_t, const double*, double*, double*, double*, void*,
-                  size_t, void*) {
-  return fail(LGAR_E_INVALID, "library built without the reverse-mode kernel");
-}
-int lgar_backward_ex(const lgar_problem*, const lgar_gradients*, void*, size_t, void*) {
-  return fail(LGAR_E_INVALID, "library built without the reverse-mode kernel");
-}
-#endif
 
 int lgar_forward_host(const lgar_problem* ph, const lgar_outputs* oh) {
   Shape s;

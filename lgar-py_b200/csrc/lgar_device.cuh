@@ -11,10 +11,10 @@
 // crosses a layer boundary (physics/layers/Layer.py:965-1008 then :951-963).
 //
 // The Green-Ampt capillary drive Geff (physics/lgar/green_ampt.py:19-99; 120-interval
-// trapezoid = 480 pow) is evaluated WARP-COOPERATIVELY: lanes = trapezoid nodes, so its cost
-// does not depend on how many lanes of the warp need it (divergent front counts).  The
-// node conductivities are then summed by the requesting lane in the reference's sequential
-// order, so the result is bit-identical to a scalar evaluation.
+// trapezoid = 480 pow) is evaluated ONE REQUEST PER LANE: the requests of a phase are written
+// to a per-warp queue (GeffQueue) and every lane runs one whole request through the
+// reference's literal loop, so the result is bit-identical to a scalar evaluation and the
+// cost does not depend on which lanes of the warp own the requests (divergent front counts).
 //
 // All citations are relative to /root/reference/dpLGAR/.  Quirk numbers (Qn) refer to
 // SURVEY.md section 8(a).
@@ -32,8 +32,10 @@ namespace lgar {
 
 constexpr int NT = 128;          // threads per CTA (4 warps, each warp an independent tile)
 constexpr int WARPS = NT / 32;
-constexpr int NODEBUF = 136;     // doubles of per-warp scratch: Geff request queue (forward), node buffer of the A/B path
-constexpr int NODEBUF_TAPED = NODEBUF;  // (the taped pass returns its five partials per request through global scratch)
+// doubles of per-warp scratch, which holds the Geff request queue.  The queue needs 96; the other 40 are kept because
+// the size sets the kernels' shared-memory layout and L1 carve-out, so shrinking it is a change to measure on its own.
+// (The taped pass returns its five partials per request through global scratch.)
+constexpr int NODEBUF = 136;
 constexpr int MAXL = LGAR_MAX_LAYERS;
 constexpr int NGIUH = LGAR_MAX_GIUH;
 constexpr int NOUT = LGAR_NUM_OUTPUTS;
@@ -89,24 +91,14 @@ __device__ __noinline__ double2 pow_log_f64(double a, double b) {
   if (!ok[0]) return pow_log_slow(a, b);
   return make_double2(r[0], lg[0]);
 }
-// two INDEPENDENT pows issued interleaved from one basic block (ILP: pow is one long dependent chain)
+// two INDEPENDENT pows from one call (fewer calls; ptxas keeps the two chains back to back, see DESIGN.md 4.1)
 __device__ __noinline__ double2 pow_x2(double x0, double y0, double x1, double y1) {
-#ifdef LGAR_POW_X2_VECTOR  // A/B: source-interleaved pair (ptxas serialises it again; measured 0.4 % slower)
-  const double xv[2] = {x0, x1}, yv[2] = {y0, y1};
-  double r[2];
-  bool ok[2];
-  pow_core_v<2>(xv, yv, r, ok);  // chains interleaved statement by statement (lgar_pow.cuh)
-  if (!ok[0]) r[0] = pow_slow(x0, y0);
-  if (!ok[1]) r[1] = pow_slow(x1, y1);
-  return make_double2(r[0], r[1]);
-#else
   bool ok0, ok1;
   double a = pow_core(x0, y0, ok0);
   double b = pow_core(x1, y1, ok1);
   if (!ok0) a = pow_slow(x0, y0);
   if (!ok1) b = pow_slow(x1, y1);
   return make_double2(a, b);
-#endif
 }
 
 struct D4 {
@@ -303,148 +295,8 @@ __device__ __forceinline__ double tmin(double a, double b) {
 }
 
 // ------------------------------------------------------------------------------------
-// Warp-cooperative Geff (green_ampt.py:19-99, trapezoid branch).
-// Must be called by all 32 lanes of the warp (convergent).  Lanes with need==true get
-// Geff(theta_1, theta_2) for their own soil `s`; the others get 0.
-//   stage A (per lane): Se, h at both ends, dh, K at node 0 -- exactly the reference's scalars
-//   stage B (per request, all lanes): node k = 1..nint has h2_k = h_i + dh + dh ... (k adds, the
-//            same accumulated rounding as `h2 = h2 + dh`), K_k = K(Se(h2_k)); lane j takes
-//            nodes j, j+32, j+64, ...
-//   stage C (requesting lane): geff = sum_i (K_{i-1} + K_i) * (dh / 2) in the reference's order.
-// ------------------------------------------------------------------------------------
-// Trapezoid terms of one Geff request, evaluated by all lanes: nodebuf[i] := (K_{i-1} + K_i) * (dh / 2) for
-// i = 1..nint (the same two operations as the reference's loop body), staged through registers so that the buffer
-// is rewritten in place.  The requesting lane then only carries the sequential `geff = geff + term_i` chain
-// (one DADD per node instead of DADD + DMUL + DADD at 1 active lane of 32).  Warp-convergent.
-__device__ __forceinline__ void geff_terms_inplace(double* nodebuf, int nint, double half) {
-  const int lane = threadIdx.x & 31;
-  double t[4];
-#pragma unroll
-  for (int r = 0; r < 4; r++) {
-    const int i = lane + 1 + 32 * r;
-    t[r] = (i <= nint) ? (nodebuf[i - 1] + nodebuf[i]) * half : 0.0;
-  }
-  __syncwarp();
-#pragma unroll
-  for (int r = 0; r < 4; r++) {
-    const int i = lane + 1 + 32 * r;
-    if (i <= nint) nodebuf[i] = t[r];
-  }
-  __syncwarp();
-}
-struct GeffRet {
-  double v;
-  int st;
-};
-// Out of line, arguments by value: one copy of the code for the three call sites of a sub-step, and
-// neither the status block nor the soil parameters are forced into local memory by the call.
-__device__ __noinline__ GeffRet geff_warp_core(bool need, double theta_1, double theta_2, Soil s, int nint,
-                                               double* nodebuf) {
-  Ctx c;
-  c.st = 0;
-  const int lane = threadIdx.x & 31;
-  double h_i = 0.0, dh = 0.0, k0 = 0.0;
-  if (need) {
-    double se_i = se_from_theta(theta_1, s, c);
-    double se_f = se_from_theta(theta_2, s, c);
-    const double2 hh = h_from_se_x2(se_i, se_f, s, c);
-    h_i = hh.x;
-    const double h_f = hh.y;
-    // "Checkpoint" calls green_ampt.py:61-63: results unused, only their guards can matter
-    if (fabs(h_i) >= 0.1 && s.alpha * h_i < 0.0) raise(c, LGAR_ST_NEG_POW);
-    if (fabs(h_f) >= 0.1 && s.alpha * h_f < 0.0) raise(c, LGAR_ST_NEG_POW);
-    dh = (h_f - h_i) / (double)nint;
-    k0 = k_from_se(se_i, s.ksat, s.m, s.inv_m, c);
-  }
-  unsigned mask = __ballot_sync(0xffffffffu, need);
-  double result = 0.0;
-  while (mask) {
-    const int src = __ffs(mask) - 1;
-    mask &= mask - 1;
-    // broadcast the request
-    Soil q;
-    q.alpha = shfl_d(s.alpha, src);
-    q.n = shfl_d(s.n, src);
-    q.m = shfl_d(s.m, src);
-    q.inv_m = shfl_d(s.inv_m, src);
-    q.ksat = shfl_d(s.ksat, src);
-    const double qh = shfl_d(h_i, src);
-    const double qdh = shfl_d(dh, src);
-    const double qk0 = shfl_d(k0, src);
-    int cc_st = 0;  // guards raised while evaluating nodes are reported to the requesting lane
-    // node t has h = h_i + dh + dh + ... (t rounded additions): advance_rounded() gives exactly that
-    // value without walking the chain; lanes take nodes lane, lane+32, lane+64, lane+96 in two pairs
-    double hn[4];
-    {
-      double h = qh;
-      int done = 0;
-#pragma unroll
-      for (int rdx = 0; rdx < 4; rdx++) {
-        const int target = lane + 32 * rdx;
-        if (target <= nint && target > done) {
-          const double h0 = h;
-          h = advance_rounded(h0, qdh, target - done);
-          if (!(h > 0.0)) {  // outside the positive range of the exact jump: walk the chain
-            h = h0;
-            for (int w = done; w < target; w++) h = h + qdh;
-          }
-          done = target;
-        }
-        hn[rdx] = h;
-      }
-    }
-#pragma unroll
-    for (int pr = 0; pr < 2; pr++) {
-      const int ta = lane + 64 * pr, tb = ta + 32;
-      if (ta <= nint) {
-        const bool both = tb <= nint;
-        int bad;
-        const double2 kk = k_nodes_core_x2(hn[2 * pr], both ? hn[2 * pr + 1] : hn[2 * pr], q.alpha, q.n, q.m, q.inv_m,
-                                           q.ksat, &bad);
-        if (bad == 0 && (isnan(kk.x) || isnan(kk.y))) bad = LGAR_ST_NAN;
-        if (bad && cc_st == 0) cc_st = bad;
-        nodebuf[ta] = (ta == 0) ? qk0 : kk.x;
-        if (both) nodebuf[tb] = kk.y;
-      }
-    }
-    unsigned badmask = __ballot_sync(0xffffffffu, cc_st != 0);
-    int st_any = 0;
-    if (badmask) {
-      int b = __ffs(badmask) - 1;  // lowest node raises first in the sequential reference
-      st_any = __shfl_sync(0xffffffffu, cc_st, b);
-    }
-    __syncwarp();
-    geff_terms_inplace(nodebuf, nint, qdh / 2.0);
-    if (lane == src) {
-      if (st_any) raise(c, st_any);
-      double geff = 0.0;
-#pragma unroll 8
-      for (int i = 1; i <= nint; i++) geff = geff + nodebuf[i];
-      result = fabs(geff / s.ksat);
-    }
-    __syncwarp();
-  }
-  GeffRet r;
-  r.v = result;
-  r.st = c.st;
-  return r;
-}
-__device__ __forceinline__ double geff_warp(bool need, double theta_1, double theta_2, const Soil& s, int nint,
-                                            double* nodebuf, Ctx& c) {
-  const GeffRet r = geff_warp_core(need, theta_1, theta_2, s, nint, nodebuf);
-  if (need) {
-    c.cnt[C_GEFF]++;
-    c.cnt[C_H_SE] += 2;
-    c.cnt[C_K_SE] += 1 + nint;
-    c.cnt[C_SE_H] += nint;
-    if (r.st) raise(c, r.st);
-  }
-  return r.v;
-}
-
-// ------------------------------------------------------------------------------------
-// Closed-form capillary drive (cfg.data.use_closed_form_G, green_ampt.py:85-98), per lane (three pows, no warp
-// cooperation needed).  Literal restatement, including the swapped roles of theta_1 / theta_2 and the operator
+// Closed-form capillary drive (cfg.data.use_closed_form_G, green_ampt.py:85-98), per lane (three pows, no queue
+// needed).  Literal restatement, including the swapped roles of theta_1 / theta_2 and the operator
 // precedence of the published line (sic):
 //   se_f = Se(theta_1), se_i = Se(theta_2);  h_c = psib (2 + 3 lambda) / (1 + 3 lambda);  e = 3 + 1 / lambda
 //   geff = h_c * se_i^e - se_f^e / (1 - se_f^e);  inf or NaN -> h_c
@@ -452,7 +304,7 @@ __device__ __forceinline__ double geff_warp(bool need, double theta_1, double th
 //   p = 1 + 2/m;  lambda = 2 / (p - 3);  psib = (p + 3)(147.8 + 8.1 p + 0.092 p^2) / (2 alpha p (p - 1)(55.6 + 7.4 p + p^2))
 // P == true also returns the partials w.r.t. theta_1, theta_2, alpha and m (reference autograd: gradient flows
 // through lambda(m) and psib(alpha, m); torch's pow has zero exponent-gradient at base 0).
-// Selected by nint < 0 at the geff_warpR call sites (substep passes nint = -1 when the flag is set).
+// Evaluated through geff_closedR where nint < 0 (substep passes nint = -1 when the flag is set).
 // ------------------------------------------------------------------------------------
 struct GeffClosed {
   double v, d_t1, d_t2, d_alpha, d_m;
@@ -672,32 +524,29 @@ __device__ __forceinline__ Pair<Var> psi_kR(const Var& se, const SoilT<Var>& s, 
   return p;
 }
 
-// ---- Geff: value from the forward routine (bit-identical), partials cooperatively (lanes = nodes).
-//      G = dh sum_k w_k K_k, geff = |G / ksat|; K_k = K(Se(h_k)), h_k = h_i + k dh, node 0 uses K(Se_i).
-//      d geff / d ksat = 0 (K is proportional to ksat).
-// GM (Geff mode) = 0: trapezoid only (the production forward kernel: the closed-form branch is compiled out of
-// its three call sites); GM = 2: run-time switch, nint < 0 selects the closed form.
-template <int GM>
-__device__ __forceinline__ double geff_warpR(bool need, double theta_1, double theta_2, const SoilT<double>& s, int nint,
-                                            double* nodebuf, Ctx& c) {
-  if (GM == 2 && nint < 0) {  // closed form (warp-uniform switch)
-    if (!need) return 0.0;
-    const GeffClosed g = geff_closed_core<false>(theta_1, theta_2, s.alpha, s.m, s.the, s.thr);
-    if (g.st) raise(c, g.st);
-    return g.v;
-  }
-  return geff_warp(need, theta_1, theta_2, s, nint, nodebuf, c);
+// ---- closed-form Geff of this lane's request (0 when need == false); the taped form records one entry with the
+//      partials w.r.t. theta_1, theta_2, alpha and m
+__device__ __forceinline__ double geff_closedR(bool need, double theta_1, double theta_2, const SoilT<double>& s, Ctx& c) {
+  if (!need) return 0.0;
+  const GeffClosed g = geff_closed_core<false>(theta_1, theta_2, s.alpha, s.m, s.the, s.thr);
+  if (g.st) raise(c, g.st);
+  return g.v;
 }
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
-  return v;
+__device__ Var geff_closedR(bool need, const Var& theta_1, const Var& theta_2, const SoilT<Var>& s, Ctx& c) {
+  if (!need) return Var(0.0);
+  const GeffClosed g = geff_closed_core<true>(theta_1.v, theta_2.v, s.alpha, s.m, s.the, s.thr);
+  if (g.st) raise(c, g.st);
+  const int ids[4] = {theta_1.id, theta_2.id, s.id_alpha, s.id_m};
+  const double d[4] = {g.d_t1, g.d_t2, g.d_alpha, g.d_m};
+  return tape_record_n(g.v, 4, ids, d);
 }
-// One trapezoid node with everything the reverse kernel needs, from ONE evaluation of the four pows: K (the same
-// operations as k_nodes_core_x2, hence the same bits as the forward kernel's node) and the partials of
-// K(Se(h; alpha, n, m); ksat, m); the logs come out of the pow cores.  node0: K_0 = K(Se_i) is a direct function of
-// Se_i in the reference graph (green_ampt.py:75), so Se is overridden by se0 after the guards of the first half
-// and the partial w.r.t. Se is reported instead of the h / alpha / n ones.
+
+// Node 0 of a taped Geff request (geff_batch_eval_taped), from ONE evaluation of the four pows: K (the same
+// operations as k_nodes_core_x2, hence the same bits as the forward kernel) and the partials of
+// K(Se(h; alpha, n, m); ksat, m); the logs come out of the pow cores.  K_0 = K(Se_i) is a direct function of Se_i in
+// the reference graph (green_ampt.py:75), so with node0 Se is overridden by se0 after the guards of the first half
+// and the partial w.r.t. Se is reported instead of the h / alpha / n ones.  The other nodes of the request go
+// through k_node_full_x2, two at a time.
 struct NodeFull {
   double K, dk_se, dk_h, dk_a, dk_n, dk_m;
   int bad;
@@ -754,130 +603,18 @@ __device__ __noinline__ NodeFull k_node_full(double h, bool node0, double se0, d
   return r;
 }
 
-// Fused value + gradient pass of the reverse kernel: the node loop of geff_warp_core with k_node_full, i.e. four
-// pows per node for the value AND the partials (a separate partial pass cost four more pows and four logs).
-template <int GM>
-__device__ Var geff_warpR(bool need, const Var& theta_1, const Var& theta_2, const SoilT<Var>& s, int nint,
-                          double* nodebuf, Ctx& c) {
-  if (GM == 2 && nint < 0) {  // closed form (warp-uniform switch): one tape entry with four partials
-    if (!need) return Var(0.0);
-    const GeffClosed g = geff_closed_core<true>(theta_1.v, theta_2.v, s.alpha, s.m, s.the, s.thr);
-    if (g.st) raise(c, g.st);
-    const int ids[4] = {theta_1.id, theta_2.id, s.id_alpha, s.id_m};
-    const double d[4] = {g.d_t1, g.d_t2, g.d_alpha, g.d_m};
-    return tape_record_n(g.v, 4, ids, d);
-  }
-  const int lane = threadIdx.x & 31;
-  // stage A: the scalars of geff_warp_core, plus the end-point partials of h(Se) for every requesting lane at once
-  Ctx ca;
-  ca.st = 0;
-  double se_i = 1.0, se_f = 1.0, h_i = 0.0, h_f = 0.0, dh = 0.0, k0 = 0.0;
-  P4 pi, pf;
-  pi.a = pi.b = pi.c = pi.d = pf.a = pf.b = pf.c = pf.d = 0.0;
-  if (need) {
-    se_i = se_from_theta(theta_1.v, s, ca);
-    se_f = se_from_theta(theta_2.v, s, ca);
-    const double2 hh = h_from_se_x2(se_i, se_f, s, ca);
-    h_i = hh.x;
-    h_f = hh.y;
-    if (fabs(h_i) >= 0.1 && s.alpha * h_i < 0.0) raise(ca, LGAR_ST_NEG_POW);  // "Checkpoint" calls, green_ampt.py:61-63
-    if (fabs(h_f) >= 0.1 && s.alpha * h_f < 0.0) raise(ca, LGAR_ST_NEG_POW);
-    dh = (h_f - h_i) / (double)nint;
-    k0 = k_from_se(se_i, s.ksat, s.m, s.inv_m, ca);
-    pi = h_se_partials_core(se_i, s.alpha, s.ninv_m, s.inv_m, s.inv_n, h_i);
-    pf = h_se_partials_core(se_f, s.alpha, s.ninv_m, s.inv_m, s.inv_n, h_f);
-    c.cnt[C_GEFF]++;
-    c.cnt[C_H_SE] += 2;
-    c.cnt[C_K_SE] += 1 + nint;
-    c.cnt[C_SE_H] += nint;
-  }
-  unsigned mask = __ballot_sync(0xffffffffu, need);
-  Var result(0.0);
-  while (mask) {
-    const int src = __ffs(mask) - 1;
-    mask &= mask - 1;
-    Soil q;
-    q.alpha = shfl_d(s.alpha, src);
-    q.n = shfl_d(s.n, src);
-    q.m = shfl_d(s.m, src);
-    q.inv_m = shfl_d(s.inv_m, src);
-    q.ksat = shfl_d(s.ksat, src);
-    const double qh = shfl_d(h_i, src), qdh = shfl_d(dh, src), qk0 = shfl_d(k0, src), qsei = shfl_d(se_i, src);
-    int cc_st = 0;
-    double S = 0.0, Ahi = 0.0, Ahf = 0.0, Ca = 0.0, Cn = 0.0, Cm = 0.0, Csei = 0.0;
-    double h = qh;
-    int done = 0;
-    for (int rdx = 0; rdx < 4; rdx++) {
-      const int target = lane + 32 * rdx;
-      if (target <= nint) {
-        if (target > done) {  // node abscissa: the rounded chain of the value pass (advance_rounded)
-          const double h0 = h;
-          h = advance_rounded(h0, qdh, target - done);
-          if (!(h > 0.0)) {
-            h = h0;
-            for (int w = done; w < target; w++) h = h + qdh;
-          }
-          done = target;
-        }
-        const NodeFull nf = k_node_full(h, target == 0, qsei, q.alpha, q.n, q.m, q.inv_m, q.ksat);
-        if (nf.bad && cc_st == 0) cc_st = nf.bad;
-        const double kk = (target == 0) ? qk0 : nf.K;
-        nodebuf[target] = kk;
-        const double w = (target == 0 || target == nint) ? 0.5 : 1.0;
-        const double frac = (double)target / (double)nint;
-        S += w * kk;
-        if (target == 0) Csei += w * nf.dk_se;
-        Ahi += w * nf.dk_h * (1.0 - frac);
-        Ahf += w * nf.dk_h * frac;
-        Ca += w * nf.dk_a;
-        Cn += w * nf.dk_n;
-        Cm += w * nf.dk_m;
-      }
-    }
-    const unsigned badmask = __ballot_sync(0xffffffffu, cc_st != 0);
-    int st_any = 0;
-    if (badmask) st_any = __shfl_sync(0xffffffffu, cc_st, __ffs(badmask) - 1);
-    S = warp_sum(S); Ahi = warp_sum(Ahi); Ahf = warp_sum(Ahf); Ca = warp_sum(Ca); Cn = warp_sum(Cn);
-    Cm = warp_sum(Cm); Csei = warp_sum(Csei);
-    __syncwarp();
-    geff_terms_inplace(nodebuf, nint, qdh / 2.0);
-    if (lane == src) {
-      if (st_any) raise(ca, st_any);
-      double geff = 0.0;
-#pragma unroll 8
-      for (int i = 1; i <= nint; i++) geff = geff + nodebuf[i];
-      const double value = fabs(geff / s.ksat);
-      const double G = qdh * S;
-      const double sg = (G / q.ksat > 0.0) ? 1.0 : ((G / q.ksat < 0.0) ? -1.0 : 0.0);
-      const double f = sg / q.ksat;
-      const double dG_dhi = -S / (double)nint + qdh * Ahi;
-      const double dG_dhf = S / (double)nint + qdh * Ahf;
-      const double inv_span = 1.0 / (s.the - s.thr);
-      const int ids[5] = {theta_1.id, theta_2.id, s.id_alpha, s.id_n, s.id_m};
-      const double d[5] = {f * (dG_dhi * pi.a + qdh * Csei) * inv_span, f * (dG_dhf * pf.a) * inv_span,
-                           f * (qdh * Ca + dG_dhi * pi.b + dG_dhf * pf.b), f * (qdh * Cn + dG_dhi * pi.c + dG_dhf * pf.c),
-                           f * (qdh * Cm + dG_dhi * pi.d + dG_dhf * pf.d)};
-      result = tape_record_n(value, 5, ids, d);
-    }
-    __syncwarp();
-  }
-  if (need && ca.st) raise(c, ca.st);
-  return result;
-}
-
 // ------------------------------------------------------------------------------------
 // Batched Geff: ONE LANE PER REQUEST (green_ampt.py:19-84, trapezoid branch).
 //
 // A sub-step of a 32-column tile issues ~60 independent Geff(theta_1, theta_2; layer) requests in calc_dzdt (one
 // per moving front of every column) -- ~90 % of all requests -- plus at most one per column in insert_water and in
 // calc_dry_depth.  The requests of a phase are known before any of them is evaluated, so they are written to a
-// per-warp queue of 32 slots and every lane evaluates ONE whole request: the literal loop of the reference
-// (`h2 = h2 + dh`, `geff = geff + (k1 + k2) * (dh / 2)`), four nodes at a time so that four independent pow
-// chains are in flight (pow_core_v<4>).  Against the earlier lanes-as-nodes scheme (geff_warp_core, kept for the
-// A/B build -DLGAR_GEFF_COOP) this needs no reconstruction of the node abscissae (advance_rounded), no node
-// buffer, no closing sum on one lane of 32, and its cost no longer depends on which lanes own the requests: the
-// queue spreads them evenly.  Values are bit-identical (same operations on the same operands in the same order).
-// The soil parameters of the requesting column are fetched with warp shuffles (owner lane, list layer).
+// per-warp queue of 32 slots (calc_dzdt: batches of 32 in queue order; the other two: slot = lane, through
+// geff_one_per_lane) and every lane evaluates ONE whole request with the literal loop of the reference
+// (`h2 = h2 + dh`, `geff = geff + (k1 + k2) * (dh / 2)`), two nodes per pass through the out-of-line pair evaluator
+// k_nodes_core_x2.  Values are bit-identical to a scalar evaluation (same operations on the same operands in the
+// same order), and the cost of a batch does not depend on which lanes own the requests.  The soil parameters of
+// the requesting column are fetched with warp shuffles (owner lane, list layer).
 // ------------------------------------------------------------------------------------
 struct GeffQueue {         // SoA over the 32 slots of a batch; lives in the per-warp scratch
   double a[32];            // in: theta_1                    out: Geff
@@ -890,58 +627,6 @@ static_assert(sizeof(GeffQueue) <= NODEBUF * sizeof(double), "the queue lives in
 // scratch (the warp's adjoint array, idle during the taped recompute): 1.25 KB more shared memory per warp would cost
 // the reverse kernel its second CTA per SM.
 __shared__ double* g_geffq_partials[NT / 32];
-
-struct K4 {
-  double k[4];
-  int bad[4];
-};
-// K(Se(h)) at four consecutive trapezoid nodes (the operations of k_nodes_core_x2, four chains interleaved)
-__device__ __forceinline__ void k_nodes_x4(const double (&h)[4], double alpha, double n, double m, double inv_m, double ksat,
-                                           double (&kout)[4], int (&bad)[4]) {
-  bool w[4], ok[4];
-  double x[4], y[4], p[4], u[4], d[4], se[4], sp[4], base[4], o[4];
-#pragma unroll
-  for (int e = 0; e < 4; e++) {
-    w[e] = fabs(h[e]) < 1.0e-01;
-    x[e] = w[e] ? 1.0 : alpha * h[e];
-    bad[e] = isnan(x[e]) ? LGAR_ST_NAN : (x[e] < 0.0 ? LGAR_ST_NEG_POW : 0);
-    y[e] = n;
-  }
-  pow_core_v<4>(x, y, p, ok);
-#pragma unroll
-  for (int e = 0; e < 4; e++) {
-    if (!ok[e]) p[e] = pow_slow(x[e], n);
-    u[e] = 1.0 + p[e];
-    y[e] = m;
-  }
-  pow_core_v<4>(u, y, d, ok);
-#pragma unroll
-  for (int e = 0; e < 4; e++) {
-    if (!ok[e]) d[e] = pow_slow(u[e], m);
-    se[e] = 1.0 / d[e];
-    if (!bad[e] && isnan(se[e])) bad[e] = LGAR_ST_NAN;
-    if (w[e]) se[e] = 1.0;
-    y[e] = inv_m;
-  }
-  pow_core_v<4>(se, y, sp, ok);
-#pragma unroll
-  for (int e = 0; e < 4; e++) {
-    if (!ok[e]) sp[e] = pow_slow(se[e], inv_m);
-    base[e] = 1.0 - sp[e];
-    if (fabs(base[e]) <= 1e-8) base[e] = base[e] + 1e-12;
-    if (!bad[e]) bad[e] = isnan(base[e]) ? LGAR_ST_NAN : (base[e] < 0.0 ? LGAR_ST_NEG_POW : 0);
-    y[e] = m;
-  }
-  pow_core_v<4>(base, y, o, ok);
-#pragma unroll
-  for (int e = 0; e < 4; e++) {
-    if (!ok[e]) o[e] = pow_slow(base[e], m);
-    const double t = 1.0 - o[e];
-    if (!bad[e]) bad[e] = isnan(t) ? LGAR_ST_NAN : (t < 0.0 ? LGAR_ST_NEG_POW : 0);
-    kout[e] = ksat * sqrt(se[e]) * (t * t);
-    if (!bad[e] && isnan(kout[e])) bad[e] = LGAR_ST_NAN;
-  }
-}
 
 // gather the soil of (owner lane, list layer) from the lanes' own parameter arrays; warp-convergent
 template <class ST>
@@ -984,26 +669,6 @@ __device__ __noinline__ void geff_batch_eval(GeffQueue* q, const ST* soil, int L
     double geff = 0.0;
     double h2 = h_i + dh;
     int st = c.st;
-#ifdef LGAR_GEFF_X4
-    for (int i = 0; i < nint; i += 4) {
-      double h[4], kk[4];
-      int bad[4];
-      h[0] = h2;
-      h[1] = h[0] + dh;
-      h[2] = h[1] + dh;
-      h[3] = h[2] + dh;
-      h2 = h[3] + dh;
-      k_nodes_x4(h, s.alpha, s.n, s.m, s.inv_m, s.ksat, kk, bad);
-#pragma unroll
-      for (int e = 0; e < 4; e++) {
-        if (i + e < nint) {
-          if (st == 0 && bad[e]) st = bad[e];
-          geff = geff + ((k1 + kk[e]) * half);
-          k1 = kk[e];
-        }
-      }
-    }
-#else
     // two nodes per pass through the SAME out-of-line pair evaluator as everything else (k_nodes_core_x2 -> pow_x2):
     // the kernel is instruction-fetch sensitive (DESIGN.md), so the hot loops share one small body of pow code
 #pragma unroll 1
@@ -1023,7 +688,6 @@ __device__ __noinline__ void geff_batch_eval(GeffQueue* q, const ST* soil, int L
         else if (isnan(kk.x) || (i + 1 < nint && isnan(kk.y))) st = LGAR_ST_NAN;
       }
     }
-#endif
     q->a[lane] = fabs(geff / s.ksat);
     q->st[lane] = st;
   }
@@ -1184,237 +848,6 @@ __device__ __noinline__ void geff_batch_eval_taped(GeffQueue* q, const ST* soil,
   __syncwarp();
 }
 
-#ifndef LGAR_GEFF_SPLIT_UP_TO
-#define LGAR_GEFF_SPLIT_UP_TO 0
-#endif
-#if LGAR_GEFF_SPLIT_UP_TO > 0
-// ------------------------------------------------------------------------------------
-// Split batches: EIGHT lanes per request, at most four requests per batch.  A full batch costs the latency of one
-// whole request (~480 dependent pows) however many of its 32 slots are filled, so the remainder of a phase's
-// requests (R mod 32, when it is small) goes through split batches instead: sub-lane p of a group evaluates the
-// nodes p*npl+1 .. (p+1)*npl (npl = ceil(nint / 8) = 15), whose abscissae h_i + dh + ... + dh (the rounded chain of
-// the reference) come from advance_rounded(); the trapezoid terms stay in registers, and the closing sum -- which
-// must be added up in the reference's order to give the same bits -- is handed from sub-lane to sub-lane.
-// Latency: 60 pows + 120 dependent adds instead of 480 pows.  Values are bit-identical to the full batch.
-// MEASURED SLOWER and therefore compiled out by default (-DLGAR_GEFF_SPLIT_UP_TO=8 enables it): 933 ms against 866 ms
-// at 125,000 x 640 -- the fixed part of a batch (soil gather, end points, six pows, the hand-over of the sum) and the
-// extra code in the instruction cache outweigh the shorter node loop; with it the gradients also depend on the
-// placement in the last bits (different summation order of the partials in split and full batches).
-// ------------------------------------------------------------------------------------
-constexpr int GEFF_SPLIT_SLOTS = 4;
-constexpr int GEFF_SPLIT_MAX_NODES = 16;  // per sub-lane (nint <= 128)
-
-__device__ __forceinline__ double geff_split_start(double h_i, double dh, int first) {
-  double h = advance_rounded(h_i, dh, first);
-  if (!(h > 0.0)) {  // outside the positive range of the exact jump: walk the chain
-    h = h_i;
-    for (int w = 0; w < first; w++) h = h + dh;
-  }
-  return h;
-}
-
-template <class ST>
-__device__ __noinline__ void geff_batch_eval_split(GeffQueue* q, const ST* soil, int L, int nint) {
-  const unsigned FULL = 0xffffffffu;
-  const int lane = threadIdx.x & 31, grp = lane >> 3, sub = lane & 7, base = lane & ~7;
-  const int meta = q->meta[grp];
-  const bool have = meta >= 0;
-  const Soil s = gather_soil(soil, L, have ? (meta & 31) : lane, have ? ((meta >> 8) & 7) : 0);
-  double h_i = 0.0, dh = 0.0, k0 = 0.0;
-  int st = 0;
-  if (have) {  // stage A, redundantly in the eight lanes of the group (same operands, same bits)
-    Ctx c;
-    c.st = 0;
-    const double se_i = se_from_theta(q->a[grp], s, c);
-    const double se_f = se_from_theta(q->b[grp], s, c);
-    const double2 hh = h_from_se_x2(se_i, se_f, s, c);
-    h_i = hh.x;
-    const double h_f = hh.y;
-    if (fabs(h_i) >= 0.1 && s.alpha * h_i < 0.0) raise(c, LGAR_ST_NEG_POW);
-    if (fabs(h_f) >= 0.1 && s.alpha * h_f < 0.0) raise(c, LGAR_ST_NEG_POW);
-    dh = (h_f - h_i) / (double)nint;
-    k0 = k_from_se(se_i, s.ksat, s.m, s.inv_m, c);
-    st = c.st;
-  }
-  const int npl = (nint + 7) >> 3;
-  const int first = sub * npl + 1;
-  const int cnt = have ? max(0, min(npl, nint - first + 1)) : 0;
-  double kk[GEFF_SPLIT_MAX_NODES];
-  double klast = 0.0;
-  int bad_first = 0;
-  if (cnt > 0) {
-    double h = geff_split_start(h_i, dh, first);
-#pragma unroll
-    for (int i = 0; i < GEFF_SPLIT_MAX_NODES; i += 2) {
-      kk[i] = kk[i + 1] = 0.0;
-      if (i < cnt) {
-        const double ha = h, hb = ha + dh;
-        h = hb + dh;
-        int bad;
-        // (an odd share ends with half a pair: the second element repeats the first, so that no abscissa beyond the
-        // request's range is ever evaluated and `bad` only reflects real nodes)
-        const double2 k2 = k_nodes_core_x2(ha, (i + 1 < cnt) ? hb : ha, s.alpha, s.n, s.m, s.inv_m, s.ksat, &bad);
-        kk[i] = k2.x;
-        kk[i + 1] = k2.y;
-        klast = (i + 1 < cnt) ? k2.y : k2.x;
-        if (bad_first == 0) {
-          if (bad) bad_first = bad;
-          else if (isnan(k2.x) || (i + 1 < cnt && isnan(k2.y))) bad_first = LGAR_ST_NAN;
-        }
-      }
-    }
-  }
-  // K of the node in front of this sub-lane's first node
-  double kin = __shfl_up_sync(FULL, klast, 1);
-  if (sub == 0) kin = k0;
-  const double half = dh / 2.0;
-  double acc = 0.0;
-#pragma unroll 1
-  for (int p = 0; p < 8; p++) {
-    if (sub == p && cnt > 0) {
-      double k1 = kin;
-#pragma unroll
-      for (int i = 0; i < GEFF_SPLIT_MAX_NODES; i++) {
-        if (i < cnt) {
-          acc = acc + ((k1 + kk[i]) * half);
-          k1 = kk[i];
-        }
-      }
-    }
-    acc = __shfl_sync(FULL, acc, base + p);  // the running sum goes to the next sub-lane (and, at the end, to all)
-    const int v = __shfl_sync(FULL, bad_first, base + p);
-    if (st == 0 && v) st = v;  // guards in node order: the first node that raises wins
-  }
-  if (have && sub == 0) {
-    q->a[grp] = fabs(acc / s.ksat);
-    q->st[grp] = st;
-  }
-  __syncwarp();
-}
-
-// taped variant: value as above + the partials (plain sums over the nodes: each sub-lane adds up its share, then a
-// butterfly over the group)
-template <class ST>
-__device__ __noinline__ void geff_batch_eval_split_taped(GeffQueue* q, const ST* soil, int L, int nint) {
-  const unsigned FULL = 0xffffffffu;
-  const int lane = threadIdx.x & 31, grp = lane >> 3, sub = lane & 7, base = lane & ~7;
-  const int meta = q->meta[grp];
-  const bool have = meta >= 0;
-  const Soil s = gather_soil(soil, L, have ? (meta & 31) : lane, have ? ((meta >> 8) & 7) : 0);
-  double h_i = 0.0, dh = 0.0, k0 = 0.0, se_i = 1.0, se_f = 1.0, h_f = 0.0;
-  int st = 0;
-  if (have) {
-    Ctx c;
-    c.st = 0;
-    se_i = se_from_theta(q->a[grp], s, c);
-    se_f = se_from_theta(q->b[grp], s, c);
-    const double2 hh = h_from_se_x2(se_i, se_f, s, c);
-    h_i = hh.x;
-    h_f = hh.y;
-    if (fabs(h_i) >= 0.1 && s.alpha * h_i < 0.0) raise(c, LGAR_ST_NEG_POW);
-    if (fabs(h_f) >= 0.1 && s.alpha * h_f < 0.0) raise(c, LGAR_ST_NEG_POW);
-    dh = (h_f - h_i) / (double)nint;
-    k0 = k_from_se(se_i, s.ksat, s.m, s.inv_m, c);
-    st = c.st;
-  }
-  const int npl = (nint + 7) >> 3;
-  const int first = sub * npl + 1;
-  const int cnt = have ? max(0, min(npl, nint - first + 1)) : 0;
-  const double inv_nint = 1.0 / (double)nint;
-  double kk[GEFF_SPLIT_MAX_NODES];
-  double klast = 0.0;
-  int bad_first = 0;
-  double S = 0.0, Csei = 0.0, Ahi = 0.0, Ahf = 0.0, Ca = 0.0, Cn = 0.0, Cm = 0.0;
-  if (have && sub == 0) {  // node 0: K(Se_i), a direct function of Se_i
-    const NodeFull n0 = k_node_full(h_i, true, se_i, s.alpha, s.n, s.m, s.inv_m, s.ksat);
-    if (st == 0 && n0.bad) st = n0.bad;
-    S = 0.5 * k0;
-    Csei = 0.5 * n0.dk_se;
-    Cm = 0.5 * n0.dk_m;
-  }
-  if (cnt > 0) {
-    double h = geff_split_start(h_i, dh, first);
-#pragma unroll
-    for (int i = 0; i < GEFF_SPLIT_MAX_NODES; i += 2) {
-      kk[i] = kk[i + 1] = 0.0;
-      if (i < cnt) {
-        const double ha = h, hb = ha + dh;
-        h = hb + dh;
-        const NodeFull2 nf = k_node_full_x2(ha, (i + 1 < cnt) ? hb : ha, s.alpha, s.n, s.m, s.inv_m, s.ksat);
-        kk[i] = nf.K[0];
-        kk[i + 1] = nf.K[1];
-        klast = (i + 1 < cnt) ? nf.K[1] : nf.K[0];
-#pragma unroll
-        for (int e = 0; e < 2; e++) {
-          if (i + e < cnt) {
-            if (bad_first == 0 && nf.bad[e]) bad_first = nf.bad[e];
-            const int node = first + i + e;
-            const double wgt = (node == nint) ? 0.5 : 1.0;
-            const double frac = (double)node * inv_nint;
-            S += wgt * nf.K[e];
-            Ahi += wgt * nf.dk_h[e] * (1.0 - frac);
-            Ahf += wgt * nf.dk_h[e] * frac;
-            Ca += wgt * nf.dk_a[e];
-            Cn += wgt * nf.dk_n[e];
-            Cm += wgt * nf.dk_m[e];
-          }
-        }
-      }
-    }
-  }
-  double kin = __shfl_up_sync(FULL, klast, 1);
-  if (sub == 0) kin = k0;
-  const double half = dh / 2.0;
-  double acc = 0.0;
-#pragma unroll 1
-  for (int p = 0; p < 8; p++) {
-    if (sub == p && cnt > 0) {
-      double k1 = kin;
-#pragma unroll
-      for (int i = 0; i < GEFF_SPLIT_MAX_NODES; i++) {
-        if (i < cnt) {
-          acc = acc + ((k1 + kk[i]) * half);
-          k1 = kk[i];
-        }
-      }
-    }
-    acc = __shfl_sync(FULL, acc, base + p);
-    const int v = __shfl_sync(FULL, bad_first, base + p);
-    if (st == 0 && v) st = v;
-  }
-#pragma unroll
-  for (int d = 1; d < 8; d <<= 1) {  // sums over the eight sub-lanes of the group
-    S += __shfl_xor_sync(FULL, S, d);
-    Csei += __shfl_xor_sync(FULL, Csei, d);
-    Ahi += __shfl_xor_sync(FULL, Ahi, d);
-    Ahf += __shfl_xor_sync(FULL, Ahf, d);
-    Ca += __shfl_xor_sync(FULL, Ca, d);
-    Cn += __shfl_xor_sync(FULL, Cn, d);
-    Cm += __shfl_xor_sync(FULL, Cm, d);
-  }
-  if (have && sub == 0) {
-    const P4 pi = h_se_partials_core(se_i, s.alpha, s.ninv_m, s.inv_m, s.inv_n, h_i);
-    const P4 pf = h_se_partials_core(se_f, s.alpha, s.ninv_m, s.inv_m, s.inv_n, h_f);
-    const double G = dh * S;
-    const double sg = (G / s.ksat > 0.0) ? 1.0 : ((G / s.ksat < 0.0) ? -1.0 : 0.0);
-    const double f = sg / s.ksat;
-    const double dG_dhi = -S * inv_nint + dh * Ahi;
-    const double dG_dhf = S * inv_nint + dh * Ahf;
-    const double inv_span = 1.0 / (s.the - s.thr);
-    q->a[grp] = fabs(acc / s.ksat);
-    q->st[grp] = st;
-    double* dq = g_geffq_partials[threadIdx.x >> 5] + grp;
-    dq[0 * 32] = f * (dG_dhi * pi.a + dh * Csei) * inv_span;
-    dq[1 * 32] = f * (dG_dhf * pf.a) * inv_span;
-    dq[2 * 32] = f * (dh * Ca + dG_dhi * pi.b + dG_dhf * pf.b);
-    dq[3 * 32] = f * (dh * Cn + dG_dhi * pi.c + dG_dhf * pf.c);
-    dq[4 * 32] = f * (dh * Cm + dG_dhi * pi.d + dG_dhf * pf.d);
-  }
-  __syncwarp();
-}
-
-#endif  // LGAR_GEFF_SPLIT_UP_TO > 0
-
 // ---- queue protocol shared by the three call sites of a sub-step ------------------------------------------------
 __device__ __forceinline__ void geffq_put(GeffQueue* q, int slot, int owner, int layer, double t1, double t2) {
   q->a[slot] = t1;
@@ -1445,154 +878,22 @@ __device__ __forceinline__ Var geffq_get(GeffQueue* q, int slot, const Var& t1, 
   const double d[5] = {dq[0 * 32], dq[1 * 32], dq[2 * 32], dq[3 * 32], dq[4 * 32]};
   return tape_record_n(q->a[slot], 5, ids, d);
 }
-// ------------------------------------------------------------------------------------
-// Dealt batches: P = 2, 4 or 8 LANES PER REQUEST for the last, partly filled batch of a phase (forward values only).
-// A batch costs the latency of one whole request (60 passes of the pair evaluator) however many of its 32 slots are
-// filled, and the bench ensemble fills 77 % of them (the requests of a warp-step, ~50, rarely come in multiples of 32).
-// When at most 32 / P requests are left they are dealt over all lanes instead: the nodes of a request go round-robin,
-// in pairs, to the P lanes of its group (lane `sub` takes the pairs sub, sub + P, ...), so a batch takes
-// ceil(nint / 2P) passes.  Bits are those of the literal loop: every lane walks the SAME chain of rounded additions
-// `h = h + dh` (and skips the nodes that are not its own: 2 (P - 1) additions per pass), and the running sum
-// `geff = geff + (k1 + k2) * (dh / 2)` travels through the P lanes in node order once per pass (two shuffles per
-// hand-over) -- nothing is buffered and the node evaluation is the one out-of-line pair evaluator of everything else.
-// The guards keep the reference's order: the first node (in node order) that raises wins.
-// MEASURED SLOWER and therefore compiled out by default (-DLGAR_GEFF_DEAL=1 enables it): bit-identical results (all 101
-// GPU tests green, incl. the bit-exact full-year columns), but the full-year forward pass of the C4 shard took 19.61 s
-// against 19.27 s (48.4 M against 49.3 M column-steps/s, profiles/bench_r2c_ab_deal.json).  Like the eight-lanes-per-
-// request split above: a partly filled batch is cheaper than its pass count suggests (the pair evaluator's FP64
-// instructions of the other resident warps fill the pipe while this warp waits), and the hand-over + redundant end
-// points are not free.  Kept as the A/B that closes the "fill the remainder batch" question.
-// ------------------------------------------------------------------------------------
-#ifndef LGAR_GEFF_DEAL
-#define LGAR_GEFF_DEAL 0
-#endif
-template <class ST>
-__device__ __noinline__ void geff_batch_eval_deal(GeffQueue* q, const ST* soil, int L, int nint, int P) {
-  const unsigned FULL = 0xffffffffu;
-  const int lane = threadIdx.x & 31;
-  const int sub = lane & (P - 1), base = lane - sub;
-  const int slot = lane / P;
-  const int meta = q->meta[slot];
-  const bool have = meta >= 0;
-  const Soil s = gather_soil(soil, L, have ? (meta & 31) : lane, have ? ((meta >> 8) & 7) : 0);
-  double h_i = 0.0, dh = 0.0, k_last = 0.0;
-  int st_a = 0;
-  if (have) {  // end points, redundantly in the P lanes of the group (same operands, same bits)
-    Ctx c;
-    c.st = 0;
-    const double se_i = se_from_theta(q->a[slot], s, c);
-    const double se_f = se_from_theta(q->b[slot], s, c);
-    const double2 hh = h_from_se_x2(se_i, se_f, s, c);
-    h_i = hh.x;
-    const double h_f = hh.y;
-    if (fabs(h_i) >= 0.1 && s.alpha * h_i < 0.0) raise(c, LGAR_ST_NEG_POW);
-    if (fabs(h_f) >= 0.1 && s.alpha * h_f < 0.0) raise(c, LGAR_ST_NEG_POW);
-    dh = (h_f - h_i) / (double)nint;
-    k_last = k_from_se(se_i, s.ksat, s.m, s.inv_m, c);
-    st_a = c.st;
-  }
-  __syncwarp();  // every lane has read its request before any result is written back into the queue
-  const double half = dh / 2.0;
-  double h2 = h_i + dh;                                 // node 1 ...
-  for (int w = 0; w < 2 * sub; w++) h2 = h2 + dh;       // ... node 2 sub + 1: this lane's first node
-  double geff = 0.0;
-  int bad_st = 0, bad_key = 0x7fffffff;                 // first raising node of this lane: status, (pass, sub)
-  const int npass = (nint + 2 * P - 1) / (2 * P);
-#pragma unroll 1
-  for (int pass = 0; pass < npass; pass++) {            // (warp-uniform)
-    const int n0 = (pass * P + sub) * 2 + 1;            // this lane's nodes: n0, n0 + 1
-    const bool va = have && n0 <= nint, vb = have && n0 + 1 <= nint;
-    double2 kk = make_double2(0.0, 0.0);
-    if (va) {
-      const double ha = h2, hb = ha + dh;
-      int bad;
-      kk = k_nodes_core_x2(ha, vb ? hb : ha, s.alpha, s.n, s.m, s.inv_m, s.ksat, &bad);
-      h2 = hb + dh;
-      for (int w = 0; w < 2 * (P - 1); w++) h2 = h2 + dh;
-      if (bad_st == 0) {
-        const int b = bad ? bad : ((isnan(kk.x) || (vb && isnan(kk.y))) ? LGAR_ST_NAN : 0);
-        if (b) {
-          bad_st = b;
-          bad_key = pass * P + sub;
-        }
-      }
-    }
-    // the running sum and the K of the node before go through the group in node order
-#pragma unroll 1
-    for (int qd = 0; qd < P; qd++) {
-      const int src = base + ((qd + P - 1) & (P - 1));
-      const double g_in = shfl_d(geff, src), k_in = shfl_d(k_last, src);
-      if (sub == qd) {
-        double g = geff, k1 = k_last;
-        if (pass > 0 || qd > 0) {
-          g = g_in;
-          k1 = k_in;
-        }
-        if (va) {
-          g = g + ((k1 + kk.x) * half);
-          k1 = kk.x;
-        }
-        if (vb) {
-          g = g + ((k1 + kk.y) * half);
-          k1 = kk.y;
-        }
-        geff = g;
-        k_last = k1;
-      }
-    }
-  }
-  const double g_fin = shfl_d(geff, base + P - 1);      // the lane that closed the last pass holds the sum
-  for (int d = 1; d < P; d <<= 1) {                     // earliest raising node of the group
-    const int ok = __shfl_xor_sync(FULL, bad_key, d), os = __shfl_xor_sync(FULL, bad_st, d);
-    if (ok < bad_key) {
-      bad_key = ok;
-      bad_st = os;
-    }
-  }
-  if (have && sub == 0) {
-    q->a[slot] = fabs(g_fin / s.ksat);
-    q->st[slot] = st_a ? st_a : bad_st;
-  }
-  __syncwarp();
-}
-
-__device__ __forceinline__ void geffq_eval(GeffQueue* q, const SoilT<double>* soil, int L, int nint, bool split = false, int deal = 1) {
-#if LGAR_GEFF_SPLIT_UP_TO > 0
-  if (split) {
-    geff_batch_eval_split(q, soil, L, nint);
-    return;
-  }
-#endif
-  (void)split;
-  if (LGAR_GEFF_DEAL && deal > 1) {
-    geff_batch_eval_deal(q, soil, L, nint, deal);
-    return;
-  }
+// evaluate the batch in the queue: values (forward) or values and partials (taped pass)
+__device__ __forceinline__ void geffq_eval(GeffQueue* q, const SoilT<double>* soil, int L, int nint) {
   geff_batch_eval(q, soil, L, nint);
 }
-__device__ __forceinline__ void geffq_eval(GeffQueue* q, const SoilT<Var>* soil, int L, int nint, bool split = false, int /*deal*/ = 1) {
-#if LGAR_GEFF_SPLIT_UP_TO > 0
-  if (split) {
-    geff_batch_eval_split_taped(q, soil, L, nint);
-    return;
-  }
-#endif
-  (void)split;
+__device__ __forceinline__ void geffq_eval(GeffQueue* q, const SoilT<Var>* soil, int L, int nint) {
   geff_batch_eval_taped(q, soil, L, nint);
 }
-// remainder rule of a phase: up to this many left-over requests go through split batches (4 per batch, ~1/7 of the
-// latency of a full batch each); more than that fill one full batch
-constexpr int GEFF_SPLIT_UP_TO = LGAR_GEFF_SPLIT_UP_TO;
-#if LGAR_GEFF_SPLIT_UP_TO == 0
-constexpr int GEFF_SPLIT_SLOTS = 4;
-#endif
 
 // At most one request per lane (insert_water, calc_dry_depth): slot = lane.  Warp-convergent.
+// GM (Geff mode) = 0: trapezoid only (the production forward kernel: the closed form is compiled out of the call
+// sites); GM = 2: run-time switch, nint < 0 selects the closed form.
 template <int GM, class R>
 __device__ __forceinline__ R geff_one_per_lane(bool need, const R& theta_1, const R& theta_2, int layer, const SoilT<R>* soil,
                                                int L, int nint, GeffQueue* q, Ctx& c) {
-  if (GM == 2 && nint < 0)  // closed form: per lane, no cooperation (geff_warpR handles it)
-    return geff_warpR<GM>(need, theta_1, theta_2, soil[need ? layer : 0], nint, reinterpret_cast<double*>(q), c);
+  if (GM == 2 && nint < 0)  // closed form: per lane, no queue
+    return geff_closedR(need, theta_1, theta_2, soil[need ? layer : 0], c);
   if (!__any_sync(0xffffffffu, need)) return R(0.0);
   const int lane = threadIdx.x & 31;
   q->meta[lane] = -1;

@@ -11,7 +11,8 @@
 // the chunk-start states double as the checkpoints of the reverse-mode kernel.
 //
 // One sub-step follows models/dpLGAR.py:154-299 exactly; the three places that evaluate Geff
-// (insert_water, calc_dry_depth, calc_dzdt) are warp-convergent call sites of geff_warp().
+// (insert_water, calc_dry_depth, calc_dzdt) are warp-convergent: their requests go through the
+// per-warp queue, one request per lane (GeffQueue, lgar_device.cuh).
 // =====================================================================================
 #pragma once
 #include "lgar_device.cuh"
@@ -122,14 +123,14 @@ __device__ void init_column(Tile<FM, R, LM>& T, double initial_psi, bool closed_
 }
 
 // ---- one sub-step: models/dpLGAR.py:176-298.  Warp-convergent: every lane of the warp calls it;
-//      lanes with act == false only take part in the cooperative Geff evaluations.
+//      lanes with act == false only take part in the warp's Geff batches.
 template <int FM, class R, int GM, int LM>
 __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double pet_rate, const KParams& K,
                         double* nodebuf) {
   Column<FM, R, LM>& C = T.col;
   Ctx& c = T.ctx;
   const double dt = K.p.subcycle_length_h;
-  const int nint = (GM == 2 && K.p.use_closed_form_G) ? -1 : K.p.nint;  // nint < 0 selects the closed-form Geff (geff_warpR)
+  const int nint = (GM == 2 && K.p.use_closed_form_G) ? -1 : K.p.nint;  // nint < 0 selects the closed-form Geff (geff_closedR)
   const int L = C.L;
   GeffQueue* const gq = reinterpret_cast<GeffQueue*>(nodebuf);
   act = act && (c.st == 0);
@@ -174,11 +175,7 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
         theta_2 = R(C.soil[lfp].the);
       }
     }
-#ifdef LGAR_GEFF_COOP
-    const R geff = geff_warpR<GM>(needG, theta_1, theta_2, C.soil[needG ? lfp : 0], nint, nodebuf, c);
-#else
     const R geff = geff_one_per_lane<GM, R>(needG, theta_1, theta_2, lfp, C.soil, K.p.num_layers, nint, gq, c);
-#endif
     if (brB && c.st == 0) {
       const R h_p = clamp_min_((ponded_depth_sub - precip_sub) * dt, 0.0);  // clamp(min=0)
       const R fd_depth = C.g(F_DEPTH, fd);
@@ -248,11 +245,7 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
       theta_1 = C.g(F_THETA, 0);
       theta_2 = R(C.soil[0].the);
     }
-#ifdef LGAR_GEFF_COOP
-    const R geff = geff_warpR<GM>(needG, theta_1, theta_2, C.soil[0], nint, nodebuf, c);
-#else
     const R geff = geff_one_per_lane<GM, R>(needG, theta_1, theta_2, 0, C.soil, K.p.num_layers, nint, gq, c);
-#endif
     if (needG && c.st == 0) {
       const SoilT<R>& s = C.soil[0];
       const R cur_theta = C.g(F_THETA, 0);
@@ -303,7 +296,6 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
   // ---- phase 4: Layer.calc_dzdt (Layer.py:1176-1252): one Geff per moving front of every column.  All requests of
   //      the tile are known here, so they go through the per-warp queue in batches of 32, one lane per request
   //      (geff_batch_eval); each lane then finishes dzdt of its own fronts in front order.
-#ifndef LGAR_GEFF_COOP
   if (!(GM == 2 && nint < 0)) {
     const unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31;
@@ -343,14 +335,7 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
     int cur = 0;           // next front to look at
     int rem = nreq;
     for (int lo = 0; lo < total;) {
-      const bool split = (total - lo) <= GEFF_SPLIT_UP_TO;  // warp-uniform
-      // the last, partly filled batch of the phase is dealt over all lanes (forward values only: geff_batch_eval_deal)
-      int deal = 1;
-      if (LGAR_GEFF_DEAL && !Column<FM, R, LM>::TAPED && !split) {
-        const int left = total - lo;
-        deal = (left <= 4) ? 8 : ((left <= 8) ? 4 : ((left <= 16) ? 2 : 1));
-      }
-      const int hi = lo + (split ? GEFF_SPLIT_SLOTS : (32 / deal));
+      const int hi = lo + 32;
       gq->meta[lane] = -1;
       __syncwarp();
       {
@@ -365,7 +350,7 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
         }
       }
       __syncwarp();
-      geffq_eval(gq, C.soil, K.p.num_layers, nint, split, deal);
+      geffq_eval(gq, C.soil, K.p.num_layers, nint);
       while (rem > 0 && g < hi) {
         const int i = cur++;
         if (C.tb(i)) continue;
@@ -396,9 +381,7 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
       lo = hi;
     }
     if (go && c.st == 0 && pre_err) raise(c, pre_err);
-  } else
-#endif
-  {  // closed-form Geff (per lane) or the A/B build with lanes-as-nodes: one request at a time
+  } else {  // closed-form Geff (geff_closedR): per lane, no queue; each lane takes its own fronts in front order
     const bool go = act && c.st == 0;
     const int my_n = go ? C.n - 1 : 0;  // the deepest front of the domain is excluded
     int nmax = my_n;
@@ -428,7 +411,7 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
           needG = (c.st == 0);
         }
       }
-      const R geff = geff_warpR<GM>(needG, theta_1, theta_2, C.soil[needG ? l : 0], nint, nodebuf, c);
+      const R geff = geff_closedR(needG, theta_1, theta_2, C.soil[needG ? l : 0], c);
       if (needG && c.st == 0) {
         const SoilT<R>& s = C.soil[l];
         const R depth = C.g(F_DEPTH, i);

@@ -54,28 +54,12 @@ __device__ const PowExpEntry g_pow_exp_table[LGAR_POW_N] = {LGAR_POW_EXP_TABLE};
 // per CTA, before its first pow); the 4 KB log table stays in global memory / L1: a shared-memory copy shortens a
 // lone warp's pow by ~3 % but costs 5 % THROUGHPUT at full occupancy (two 16-byte LDS per pow with random rows
 // serialise on bank conflicts), and throughput is what the ensemble runs are bound by.
-// LGAR_POW_LOG_SHARED / LGAR_POW_EXP_GLOBAL select the other placements (A/B builds).
-#ifdef LGAR_POW_LOG_SHARED
-__shared__ double2 s_pow_log_table[2 * LGAR_POW_N];
-#define LGAR_POW_LOG_ROW(i2) s_pow_log_table[i2]
-#else
-#define LGAR_POW_LOG_ROW(i2) __ldg(reinterpret_cast<const double2*>(g_pow_log_table) + (i2))
-#endif
-#ifndef LGAR_POW_EXP_GLOBAL
 __shared__ double2 s_pow_exp_table[LGAR_POW_N];
+#define LGAR_POW_LOG_ROW(i2) __ldg(reinterpret_cast<const double2*>(g_pow_log_table) + (i2))
 #define LGAR_POW_EXP_ROW(j) s_pow_exp_table[j]
-#else
-#define LGAR_POW_EXP_ROW(j) __ldg(reinterpret_cast<const double2*>(g_pow_exp_table) + (j))
-#endif
 __device__ __forceinline__ void pow_tables_to_shared() {
-#ifdef LGAR_POW_LOG_SHARED
-  for (int i = threadIdx.x; i < 2 * LGAR_POW_N; i += blockDim.x)
-    s_pow_log_table[i] = reinterpret_cast<const double2*>(g_pow_log_table)[i];
-#endif
-#ifndef LGAR_POW_EXP_GLOBAL
   for (int i = threadIdx.x; i < LGAR_POW_N; i += blockDim.x)
     s_pow_exp_table[i] = reinterpret_cast<const double2*>(g_pow_exp_table)[i];
-#endif
   __syncthreads();
 }
 #endif
@@ -130,10 +114,8 @@ LGAR_HD double pow_fma(double a, double b, double c) {
 // lg (optional): log(x[k]) to double precision -- a by-product of the log stage, used by the derivative weights of
 // the reverse kernel (d x^y / dy = x^y log x) instead of a separate log() call.
 template <int N>
-// rs (optional): X - res[k], the rounding residual of the final operation (X = scale + scale * tmp2 before rounding),
-// NaN where it is not defined (|y log x| < 2^-60); used by pow_inverse_root() below.
 LGAR_HD void pow_core_v(const double (&x)[N], const double (&y)[N], double (&res)[N], bool (&ok)[N],
-                        double* lg = nullptr, double* rs = nullptr) {
+                        double* lg = nullptr) {
   bool x_ok[N];
   int ki_[N];
   double z[N], kd[N], invc[N], logc[N], logctail[N];
@@ -228,34 +210,7 @@ LGAR_HD void pow_core_v(const double (&x)[N], const double (&y)[N], double (&res
   LGAR_V(tmp2[e] = tailj[e] + (rr[e] + (rr2[e] * e2[e] + (rr2[e] * rr2[e]) * e4[e])))
   // |y log x| tiny: pow = 1 + y log x to well below half an ulp
   LGAR_V(res[e] = (aeh[e] < 0x1p-60) ? (1.0 + ehi[e]) : pow_fma(scale[e], tmp2[e], scale[e]))
-  if (rs) {  // scale - res is exact (Sterbenz: res / scale is within 0.4 % of 1), so the fma returns X - res rounded once
-    LGAR_V(rs[e] = (aeh[e] < 0x1p-60) ? (0.0 / 0.0) : pow_fma(scale[e], tmp2[e], scale[e] - res[e]))
-  }
 #undef LGAR_V
-}
-
-// The third pow of a trapezoid node (green_ampt.py:75-81 -> utils.py:115-156):
-//     d = pow(u, m);  se = 1 / d;  sp = pow(se, inv_m)        with u = 1 + (alpha h)^n, inv_m = fl(1 / m)
-// sp is mathematically 1/u up to the rounding errors of d, se and inv_m, all of which are known EXACTLY:
-//     d  = X (1 - resid / X)      resid = rounding residual of the pow core's last operation (rs above)
-//     se = (1 / d)(1 + eps)       eps = fma(se, d, -1)
-//     inv_m = (1 / m)(1 + tau)    tau = fma(inv_m, m, -1)
-//   => pow(se, inv_m) = (1 / u) (1 + (eps + resid / d) inv_m - tau log u)  (1 + O(2^-61 / m))
-// (X differs from the true u^m by the pow core's internal error, <= 2^-61.7 relative in 60,000 samples; log u is the
-// core's own logarithm).  1/u is formed as a two-term quotient, so the result carries 0.5 ulp of final rounding plus
-// ~(0.004 + 0.003 / m) ulp -- the accuracy class of glibc's pow (0.52 ulp), at a quarter of the cost of a pow.
-// Checked against mpmath by tools/pow_inverse_root_accuracy.py.
-LGAR_HD double pow_inverse_root(double u, double d, double se, double resid, double log_u, double m, double inv_m) {
-  const double eps = pow_fma(se, d, -1.0);
-  const double tau = pow_fma(inv_m, m, -1.0);
-  const double c = (eps + resid * se) * inv_m - tau * log_u;  // resid / d = resid * se (1 + O(2^-53)), resid is ~2^-53 d
-#ifdef __CUDA_ARCH__
-  const double w_hi = __drcp_rn(u);  // IEEE reciprocal: cheaper than the general division
-#else
-  const double w_hi = 1.0 / u;
-#endif
-  const double w_lo = -pow_fma(w_hi, u, -1.0) * w_hi;
-  return w_hi + (w_lo + w_hi * c);
 }
 
 // scalar form (the CPU accuracy harness and the single-evaluation closures)
