@@ -83,41 +83,20 @@ struct BParams {
   unsigned long long* counters; // [8] diagnostics (lgar_gradients.counters)
 };
 
-// second stage of the shared-parameter reduction: block q sums partials[.][q] over the tiles in a fixed order
-// (lane j takes tiles j, j+32, ... sequentially, then a butterfly over the 32 lane sums)
-__global__ void lgar_reduce_tile_partials(const double* partials, int ntiles, int L, double* grad_alpha, double* grad_n,
-                                          double* grad_ksat, double* grad_pdm) {
-  const int q = blockIdx.x;  // 3 l + {0: alpha, 1: n, 2: ksat}
-  double s = 0.0;
-  for (int t = threadIdx.x; t < ntiles; t += 32) s += partials[(size_t)t * NPAR_IDS + q];
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d);
-  if (threadIdx.x == 0) {
-    const int l = q / 3;
-    if (q == ID_PDM) {
-      if (grad_pdm) grad_pdm[0] = s;
-    } else if (l < L) {
-      double* out = (q % 3 == 0) ? grad_alpha : ((q % 3 == 1) ? grad_n : grad_ksat);
-      out[l] = s;
-    }
-  }
-}
+// resident CTAs per SM of lgar_backward_kernel: sets its register cap (2: up to 255 registers) and bounds the number of
+// resident warps that need a scratch slot (lgar_backward_launch.cu)
+constexpr int BACKWARD_CTAS_PER_SM = 2;
 
-__host__ inline size_t backward_meta_bytes(int FM) {
-  return FM == 16 ? sizeof(StepMeta<16>) : (FM == 12 ? sizeof(StepMeta<12>) : sizeof(StepMeta<8>));
-}
-__host__ inline size_t backward_scratch_bytes(int S, int FM, int chunk, int slots, int arena_cap, int step_cap, int ntiles) {
-  const size_t ring_steps = (size_t)chunk * S;
-  const size_t nl = NPAR_IDS + 5 * (size_t)FM + 2 + NGIUH;
-  size_t per = (size_t)arena_cap * 32 * sizeof(TapeEntry) + ring_steps * 32 * backward_meta_bytes(FM) +
-               (nl + step_cap) * 32 * 8;
-  size_t per_tile = nl * 32 * 8 + (size_t)NPAR_IDS * 32 * 8 + 32 * 4 + 4;
-  return per * slots + per_tile * ntiles + 16384;
+// dynamic shared memory of lgar_backward_kernel<FM>: the carve at the top of the kernel
+template <int FM>
+constexpr size_t backward_smem_bytes() {
+  return (size_t)5 * FM * NT * sizeof(double) + (size_t)WARPS * NODEBUF * sizeof(double) +
+         (size_t)5 * FM * NT * sizeof(short) + (size_t)FM * NT;
 }
 
 // GM = 0: trapezoid Geff only (closed-form branch compiled out of the taped sub-step); GM = 2: run-time switch
 template <int FM, int GM>
-__global__ void __launch_bounds__(NT, 2) lgar_backward_kernel(const BParams P) {  // 2 CTAs per SM: up to 255 registers
+__global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel(const BParams P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* sm_fields = reinterpret_cast<double*>(smem_raw);                       // [5*FM][NT]
   double* sm_nodes = sm_fields + 5 * FM * NT;                                    // [WARPS][NODEBUF]

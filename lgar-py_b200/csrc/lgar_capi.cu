@@ -3,12 +3,18 @@
 // Host-side only does argument checking, workspace carving and ONE kernel launch per call.
 // There is no CPU fallback: without an sm_100 device every compute entry point fails.
 // =====================================================================================
+#include <algorithm>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <vector>
 
 #include "lgar_forward.cuh"
 #include "lgar_backward.cuh"
+
+// the reverse kernel is compiled in its own translation unit (lgar_backward_launch.cu)
+size_t lgar_reverse_unit_scratch(int FM, void* params, unsigned char* scratch);
+int lgar_reverse_unit_launch(int FM, const void* params, int num_sms, void* stream, char* err, size_t errlen);
 
 namespace {
 
@@ -32,7 +38,13 @@ struct Shape {
   int t_begin, t_end;  // window of forcing rows (whole record: 0, T)
 };
 
-int shape_of(const lgar_problem* p, Shape& s) {
+enum Entry { WORKSPACE_BYTES, FORWARD, BACKWARD };
+
+// The argument rules of lgar_workspace_bytes, lgar_forward and lgar_backward_ex, checked before the device and before
+// anything is enqueued.  `with_grad`: the call sizes, writes or reads checkpoints.  Fills s; returns the first rule
+// the call breaks (0: none).
+int check_args(Entry entry, const lgar_problem* p, int with_grad, const lgar_outputs* out, const lgar_gradients* g,
+               Shape& s) {
   if (!p) return fail(LGAR_E_INVALID, "problem is NULL");
   if (p->abi_version != LGAR_ABI_VERSION) return fail(LGAR_E_INVALID, "abi_version mismatch");
   if (p->num_columns < 1 || p->num_steps < 1 || p->num_subcycles < 1) return fail(LGAR_E_INVALID, "empty problem");
@@ -60,10 +72,35 @@ int shape_of(const lgar_problem* p, Shape& s) {
   }
   s.nchunks = (s.t_end - s.t_begin + s.chunk - 1) / s.chunk;
   s.ntiles = s.Bp / 32;
+  if (with_grad && (long long)s.chunk * s.S > 512)
+    return fail(LGAR_E_INVALID, "chunk_steps * num_subcycles > 512 with checkpoints: the tape arena of the reverse "
+                                "pass (one chunk of sub-steps per resident warp) would not fit; use chunk_steps = 0 "
+                                "(default) or a smaller value");
+  if (entry == WORKSPACE_BYTES) return 0;
+  if (s.FM == 32 && with_grad) return fail(LGAR_E_INVALID, "max_fronts = 32 is forward-only (no checkpoints)");
+  if (with_grad && (s.t_begin != 0 || s.t_end != s.T))
+    return fail(LGAR_E_INVALID, "a step window (step_begin, step_end) is forward-only: checkpoints and lgar_backward "
+                                "need the whole record");
+  if (entry == BACKWARD) {
+    if (!g) return fail(LGAR_E_INVALID, "gradients is NULL");
+    if (!g->grad_alpha || !g->grad_n || !g->grad_ksat)
+      return fail(LGAR_E_INVALID, "a gradient output array (grad_alpha, grad_n, grad_ksat) is NULL");
+    if (g->reduce && !g->partials) return fail(LGAR_E_INVALID, "reduce needs the partials scratch array");
+    return 0;
+  }
+  if (!out) return fail(LGAR_E_INVALID, "outputs is NULL");
+  if (!p->alpha || !p->n || !p->ksat || !p->theta_r || !p->theta_e || !p->thickness || !p->initial_psi ||
+      !p->ponded_depth_max || !p->forcing)
+    return fail(LGAR_E_INVALID, "a required problem array is NULL");
+  if (p->num_sites < 1) return fail(LGAR_E_INVALID, "num_sites < 1");
+  if (p->resume && with_grad) return fail(LGAR_E_INVALID, "resume is not available with keep_checkpoints");
+  if (s.t_begin != 0 && !p->resume) return fail(LGAR_E_INVALID, "step_begin > 0 needs resume = 1");
+  if (p->pipeline_seq < 0 || p->pipeline_seq >= (1 << 23)) return fail(LGAR_E_INVALID, "pipeline_seq out of range");
+  if (p->pipeline_seq > 0 && with_grad) return fail(LGAR_E_INVALID, "pipeline_seq > 0 is forward-only");
+  if (p->pipeline_seq > 1 && !p->resume) return fail(LGAR_E_INVALID, "pipeline_seq > 1 needs resume = 1");
+  if (out->fronts && s.FM != 16) return fail(LGAR_E_INVALID, "front dumps (outputs.fronts) need max_fronts = 16");
   return 0;
 }
-
-size_t align_up(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
 
 struct Carve {
   size_t off_d, off_i, off_f, off_slog, off_slogc, off_done, off_item, total;
@@ -74,6 +111,7 @@ struct Carve {
 #define LGAR_SLOG_AVG 5
 
 Carve carve(const Shape& s, int with_grad) {
+  using lgar::align_up;
   const size_t nck = with_grad ? (size_t)s.nchunks + 1 : 1;
   const size_t nd = 5 * (size_t)s.FM + lgar::S_COUNT;
   Carve c;
@@ -90,46 +128,63 @@ Carve carve(const Shape& s, int with_grad) {
   return c;
 }
 
+// the kernel parameters both passes share; the settings of one pass are made by its caller
+lgar::KParams kparams(const lgar_problem* p, const Shape& s, const Carve& c, unsigned char* w) {
+  lgar::KParams K;
+  std::memset(&K, 0, sizeof(K));
+  K.p = *p;
+  K.state_d = lgar::at<double>(w, c.off_d);
+  K.state_i = lgar::at<int32_t>(w, c.off_i);
+  K.state_f = lgar::at<uint8_t>(w, c.off_f);
+  K.done = lgar::at<int32_t>(w, c.off_done);
+  K.next_item = lgar::at<unsigned long long>(w, c.off_item);
+  K.Bp = s.Bp;
+  K.ntiles = s.ntiles;
+  K.nchunks = s.nchunks;
+  K.chunk_steps = s.chunk;
+  K.iter_cap = p->iter_cap > 0 ? p->iter_cap : 1000000;
+  return K;
+}
+
 int g_dev_checked = -2;
 int g_num_sms = 0;
 
-// reverse kernel: resident warps that own scratch (ring, tape, adjoints).  Sized without a device
-// query so that lgar_workspace_bytes works on a host without a GPU: <= 160 SMs, CTAs per SM bounded by
-// the shared-memory footprint of the value + id arrays.
-#define LGAR_TAPE_CAP_MAX 6144  /* + leaves must stay below 32768: ids are stored as 16 bit in shared memory */
-// entries one sub-step may record.  LGAR_DEBUG_TAPE_CAP (environment, tests only) shrinks it to provoke the
-// overflow path: tests/test_gpu_gradients.py::test_tape_overflow_is_reported
-#include <cstdlib>
-static int tape_cap() {
-  const char* e = std::getenv("LGAR_DEBUG_TAPE_CAP");
-  if (e) {
-    const int v = std::atoi(e);
-    if (v >= 16 && v <= LGAR_TAPE_CAP_MAX) return v;
-  }
-  return LGAR_TAPE_CAP_MAX;
-}
-#define LGAR_TAPE_CAP tape_cap()
-int backward_ctas_per_sm(const Shape&) { return 2; }  // __launch_bounds__(NT, 2) of lgar_backward_kernel
-// tape arena of one chunk: average budget of LGAR_TAPE_AVG entries per sub-step (a sub-step may use up to
-// LGAR_TAPE_CAP); exhaustion flags the column (NaN gradient + tape_overflow)
-#define LGAR_TAPE_AVG 640  /* bench ensemble: 83 entries per sub-step on average, heavy-tailed (320 overflows 0.1 % of the columns) */
-int backward_arena_cap(const Shape& s) {
-  long long c = (long long)s.chunk * s.S * LGAR_TAPE_AVG;  // chunk * S <= 512 (checked): fits an int
-  if (std::getenv("LGAR_DEBUG_TAPE_CAP")) c = LGAR_TAPE_CAP;
-  if (c < LGAR_TAPE_CAP) c = LGAR_TAPE_CAP;
-  return (int)c;
-}
-int backward_slots(const Shape& s) {
-  long long want = ((long long)s.ntiles * s.nchunks + lgar::WARPS - 1) / lgar::WARPS;
-  long long grid = 160LL * backward_ctas_per_sm(s);
-  if (grid > want) grid = want;
-  return (int)grid * lgar::WARPS;
+int ensure_device() {
+  int dev = -1;
+  if (cudaGetDevice(&dev) == cudaSuccess && dev == g_dev_checked) return 0;
+  return lgar_device_check();
 }
 
-template <int FM>
-size_t smem_bytes() {
-  return (size_t)5 * FM * lgar::NT * sizeof(double) + (size_t)lgar::WARPS * lgar::NODEBUF * sizeof(double) +
-         (size_t)FM * lgar::NT;
+// Tape budget of the reverse pass.  step_cap: entries one sub-step may record; step_cap + leaves must stay below 32768
+// because tape ids are stored as 16 bit in shared memory.  arena_cap: entries of one chunk per lane, on average 640 per
+// sub-step (bench ensemble: 83 per sub-step on average, heavy-tailed; 320 overflows 0.1 % of the columns), and at
+// least step_cap.  An exhausted arena flags the column (NaN gradient + tape_overflow).  LGAR_DEBUG_TAPE_CAP (tests
+// only) sets step_cap and shrinks the arena to it, to provoke the overflow path
+// (tests/test_gpu_gradients.py::test_tape_overflow_is_reported).
+void set_tape_budget(lgar::BParams& P, const Shape& s) {
+  constexpr int TAPE_CAP_MAX = 6144, TAPE_AVG = 640;
+  const char* e = std::getenv("LGAR_DEBUG_TAPE_CAP");
+  const int v = e ? std::atoi(e) : 0;
+  P.step_cap = (v >= 16 && v <= TAPE_CAP_MAX) ? v : TAPE_CAP_MAX;
+  P.arena_cap = e ? P.step_cap : std::max(s.chunk * s.S * TAPE_AVG, P.step_cap);  // chunk * S <= 512 (checked)
+}
+
+// Everything the reverse kernel reads except the caller's gradient arguments, over workspace w (nullptr: sizing only).
+// Returns the bytes of workspace the reverse pass needs.
+size_t backward_params(const lgar_problem* p, const Shape& s, unsigned char* w, lgar::BParams& P) {
+  const Carve c = carve(s, 1);
+  std::memset(&P, 0, sizeof(P));
+  lgar::KParams& K = P.K;
+  K = kparams(p, s, c, w);
+  K.t_begin = 0;
+  K.t_end = s.T;
+  K.keep_ckpt = 1;
+  K.slog = lgar::at<double>(w, c.off_slog);
+  K.slog_count = lgar::at<int32_t>(w, c.off_slogc);
+  K.slog_cap = c.slog_cap;
+  P.ring_steps = s.chunk * s.S;
+  set_tape_budget(P, s);
+  return c.total + lgar_reverse_unit_scratch(s.FM, &P, lgar::at<unsigned char>(w, c.total));
 }
 
 // Launch plan of one lgar_forward call.  `pipeline_seq` k > 1 asks for a programmatic dependent launch behind
@@ -141,14 +196,13 @@ struct Plan {
   const Carve* carve;
   unsigned char* w;
   int pipeline_seq;
-  bool counters_reset;
 };
 
 template <int FM, bool COUNT, bool DUMP, bool LOGW = false>
 int launch_forward(Plan& P, cudaStream_t st) {
   lgar::KParams& K = P.K;
   auto kern = lgar::lgar_forward_kernel<FM, COUNT, DUMP, LOGW>;
-  const size_t smem = smem_bytes<FM>();
+  constexpr size_t smem = lgar::forward_smem_bytes<FM>();
   CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, lgar::NT, smem));
@@ -180,12 +234,11 @@ int launch_forward(Plan& P, cudaStream_t st) {
   return 0;
 }
 
-}  // namespace
-
 // ---- host-buffer variant ------------------------------------------------------------
-namespace {
 struct DevBuf {
   std::vector<void*> ptrs;
+  struct Download { void* host; const void* dev; size_t bytes; };
+  std::vector<Download> downloads;
   ~DevBuf() {
     for (void* p : ptrs) cudaFree(p);
   }
@@ -200,23 +253,25 @@ struct DevBuf {
     *dev_out = (const T*)d;
     return 0;
   }
+  // device buffer for an output, copied back to `host` by download()
   template <class T>
-  int alloc(const T* host, size_t count, T** dev_out) {
+  int out(T* host, size_t count, T** dev_out) {
     *dev_out = nullptr;
     if (!host) return 0;
     void* d = nullptr;
     CUDA_TRY(cudaMalloc(&d, count * sizeof(T)));
     ptrs.push_back(d);
+    downloads.push_back({host, d, count * sizeof(T)});
     *dev_out = (T*)d;
     return 0;
   }
+  int download() {
+    for (const Download& x : downloads) CUDA_TRY(cudaMemcpy(x.host, x.dev, x.bytes, cudaMemcpyDeviceToHost));
+    return 0;
+  }
 };
+
 }  // namespace
-
-
-// the reverse kernel is compiled in its own translation unit (lgar_backward_launch.cu)
-int lgar_reverse_unit_launch(int FM, void* params, int S, int chunk, int slots, int arena_cap, int step_cap, int num_sms,
-                             unsigned char* scratch, void* stream, char* err, size_t errlen);
 
 extern "C" {
 
@@ -239,65 +294,25 @@ int lgar_device_check(void) {
 
 size_t lgar_workspace_bytes(const lgar_problem* p, int with_grad) {
   Shape s;
-  if (shape_of(p, s)) return 0;
-  if (with_grad && (long long)s.chunk * s.S > 512) {
-    fail(LGAR_E_INVALID, "chunk_steps * num_subcycles > 512: the tape arena of the reverse pass (one chunk of sub-steps per "
-                         "resident warp) would not fit; use chunk_steps = 0 (default) or a smaller value");
-    return 0;
-  }
-  size_t total = carve(s, with_grad).total;
-  if (with_grad)
-    total += lgar::backward_scratch_bytes(s.S, s.FM, s.chunk, backward_slots(s), backward_arena_cap(s), LGAR_TAPE_CAP, s.ntiles);
-  return total;
+  if (check_args(WORKSPACE_BYTES, p, with_grad, nullptr, nullptr, s)) return 0;
+  if (!with_grad) return carve(s, 0).total;
+  lgar::BParams P;
+  return backward_params(p, s, nullptr, P);
 }
 
 int lgar_forward(const lgar_problem* p, const lgar_outputs* out, void* workspace_dev, size_t workspace_bytes,
                  int keep_checkpoints, void* stream) {
   Shape s;
-  int rc = shape_of(p, s);
-  if (rc) return rc;
-  if (!out) return fail(LGAR_E_INVALID, "outputs is NULL");
-  if (!p->alpha || !p->n || !p->ksat || !p->theta_r || !p->theta_e || !p->thickness || !p->initial_psi ||
-      !p->ponded_depth_max || !p->forcing)
-    return fail(LGAR_E_INVALID, "a required problem array is NULL");
-  if (p->num_sites < 1) return fail(LGAR_E_INVALID, "num_sites < 1");
-  if (p->resume && keep_checkpoints) return fail(LGAR_E_INVALID, "resume is not available with keep_checkpoints");
-  if (keep_checkpoints && (long long)s.chunk * s.S > 512)
-    return fail(LGAR_E_INVALID, "chunk_steps * num_subcycles > 512 with keep_checkpoints (reverse-pass tape arena)");
-  if (s.FM == 32 && keep_checkpoints) return fail(LGAR_E_INVALID, "max_fronts = 32 is forward-only (no checkpoints)");
-  if (keep_checkpoints && (s.t_begin != 0 || s.t_end != s.T))
-    return fail(LGAR_E_INVALID, "a step window is forward-only (keep_checkpoints needs the whole record)");
-  if (s.t_begin != 0 && !p->resume) return fail(LGAR_E_INVALID, "a window that does not start at row 0 needs resume = 1");
-  int dev = -1;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev != g_dev_checked) {
-    rc = lgar_device_check();
-    if (rc) return rc;
-  }
+  int rc = check_args(FORWARD, p, keep_checkpoints, out, nullptr, s);
+  if (rc || (rc = ensure_device())) return rc;
   const Carve c = carve(s, keep_checkpoints);
   if (!workspace_dev || workspace_bytes < c.total) return fail(LGAR_E_WORKSPACE, "workspace too small");
   cudaStream_t st = (cudaStream_t)stream;
   unsigned char* w = (unsigned char*)workspace_dev;
 
-  Plan plan;
+  Plan plan{kparams(p, s, c, w), &c, w, p->pipeline_seq};
   lgar::KParams& K = plan.K;
-  std::memset(&K, 0, sizeof(K));
-  plan.carve = &c;
-  plan.w = w;
-  plan.pipeline_seq = p->pipeline_seq;
-  if (p->pipeline_seq < 0 || p->pipeline_seq >= (1 << 23)) return fail(LGAR_E_INVALID, "pipeline_seq out of range");
-  if (p->pipeline_seq > 0 && keep_checkpoints) return fail(LGAR_E_INVALID, "pipelined windows are forward-only");
-  if (p->pipeline_seq > 1 && !p->resume) return fail(LGAR_E_INVALID, "pipeline_seq > 1 needs resume = 1");
-  K.p = *p;
   K.o = *out;
-  K.state_d = (double*)(w + c.off_d);
-  K.state_i = (int32_t*)(w + c.off_i);
-  K.state_f = (uint8_t*)(w + c.off_f);
-  K.done = (int32_t*)(w + c.off_done);
-  K.next_item = (unsigned long long*)(w + c.off_item);
-  K.Bp = s.Bp;
-  K.ntiles = s.ntiles;
-  K.nchunks = s.nchunks;
-  K.chunk_steps = s.chunk;
   K.t_begin = s.t_begin;
   K.t_end = s.t_end;
   K.keep_ckpt = keep_checkpoints ? 1 : 0;
@@ -310,7 +325,6 @@ int lgar_forward(const lgar_problem* p, const lgar_outputs* out, void* workspace
     K.slog_cap = c.slog_cap;
     if (!logw) CUDA_TRY(cudaMemsetAsync(K.slog_count, 0, (size_t)s.nchunks * s.Bp * sizeof(int32_t), st));
   }
-  K.iter_cap = p->iter_cap > 0 ? p->iter_cap : 1000000;
   if (p->pipeline_seq <= 1) {  // (a memset between two kernels of a pipelined sequence would serialise them)
     if (out->counters) CUDA_TRY(cudaMemsetAsync(out->counters, 0, 16 * sizeof(unsigned long long), st));
     if (out->tile_cycles)
@@ -318,61 +332,23 @@ int lgar_forward(const lgar_problem* p, const lgar_outputs* out, void* workspace
   }
   // the kernels without work counters are trapezoid-only (closed-form branch compiled out of the hot path)
   const bool count = out->counters != nullptr || p->use_closed_form_G != 0;
-  const bool dump = out->fronts != nullptr;
-  if (dump && s.FM != 16) return fail(LGAR_E_INVALID, "front dumps need max_fronts = 16");
-#define LGAR_DISPATCH(FM_)                                                         \
-  if (count) rc = launch_forward<FM_, true, false>(plan, st);                      \
-  else rc = launch_forward<FM_, false, false>(plan, st);
-  if (dump) rc = launch_forward<16, true, true>(plan, st);
-  else if (s.FM == 8) { LGAR_DISPATCH(8) }
-  else if (s.FM == 12) { LGAR_DISPATCH(12) }
-  else if (s.FM == 32) rc = launch_forward<32, true, false>(plan, st);  // large-capacity fallback (1 CTA per SM)
-  else if (logw) rc = launch_forward<16, false, false, true>(plan, st);
-  else { LGAR_DISPATCH(16) }
-#undef LGAR_DISPATCH
-  return rc;
+  if (out->fronts) return launch_forward<16, true, true>(plan, st);
+  if (s.FM == 8) return count ? launch_forward<8, true, false>(plan, st) : launch_forward<8, false, false>(plan, st);
+  if (s.FM == 12) return count ? launch_forward<12, true, false>(plan, st) : launch_forward<12, false, false>(plan, st);
+  if (s.FM == 32) return launch_forward<32, true, false>(plan, st);  // large-capacity fallback (1 CTA per SM)
+  if (logw) return launch_forward<16, false, false, true>(plan, st);
+  return count ? launch_forward<16, true, false>(plan, st) : launch_forward<16, false, false>(plan, st);
 }
 
 int lgar_backward_ex(const lgar_problem* p, const lgar_gradients* g, void* workspace_dev, size_t workspace_bytes,
                      void* stream) {
   Shape s;
-  int rc = shape_of(p, s);
-  if (rc) return rc;
-  if (!g) return fail(LGAR_E_INVALID, "gradients is NULL");
-  if (!g->grad_alpha || !g->grad_n || !g->grad_ksat) return fail(LGAR_E_INVALID, "gradient output array is NULL");
-  if (g->reduce && !g->partials) return fail(LGAR_E_INVALID, "reduce needs the partials scratch array");
-  if (s.FM == 32) return fail(LGAR_E_INVALID, "max_fronts = 32 is forward-only");
-  int dev = -1;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev != g_dev_checked) {
-    rc = lgar_device_check();
-    if (rc) return rc;
-  }
-  const Carve c = carve(s, 1);
-  const size_t need = lgar_workspace_bytes(p, 1);
-  if (!workspace_dev || workspace_bytes < need) return fail(LGAR_E_WORKSPACE, "workspace too small for lgar_backward");
-  cudaStream_t st = (cudaStream_t)stream;
+  int rc = check_args(BACKWARD, p, 1, nullptr, g, s);
+  if (rc || (rc = ensure_device())) return rc;
   unsigned char* w = (unsigned char*)workspace_dev;
   lgar::BParams P;
-  std::memset(&P, 0, sizeof(P));
-  lgar::KParams& K = P.K;
-  K.p = *p;
-  K.state_d = (double*)(w + c.off_d);
-  K.state_i = (int32_t*)(w + c.off_i);
-  K.state_f = (uint8_t*)(w + c.off_f);
-  K.done = (int32_t*)(w + c.off_done);
-  K.next_item = (unsigned long long*)(w + c.off_item);
-  K.Bp = s.Bp;
-  K.ntiles = s.ntiles;
-  K.nchunks = s.nchunks;
-  K.chunk_steps = s.chunk;
-  K.t_begin = 0;
-  K.t_end = s.T;
-  if (s.t_begin != 0 || s.t_end != s.T) return fail(LGAR_E_INVALID, "lgar_backward needs the whole record (no step window)");
-  K.keep_ckpt = 1;
-  K.slog = std::getenv("LGAR_DEBUG_NO_SEARCH_LOG") ? nullptr : (double*)(w + c.off_slog);
-  K.slog_count = (int32_t*)(w + c.off_slogc);
-  K.slog_cap = c.slog_cap;
-  K.iter_cap = p->iter_cap > 0 ? p->iter_cap : 1000000;
+  if (!w || workspace_bytes < backward_params(p, s, w, P))
+    return fail(LGAR_E_WORKSPACE, "workspace too small for lgar_backward");
   P.grad_per_step = g->grad_per_step;
   P.grad_mask = g->grad_per_step ? g->grad_mask : 0;
   P.grad_sums = g->grad_sums;
@@ -384,11 +360,9 @@ int lgar_backward_ex(const lgar_problem* p, const lgar_gradients* g, void* works
   P.reduce = g->reduce ? 1 : 0;
   P.partials = g->partials;
   P.counters = g->counters;
-  K.time_phases = g->counters ? 1 : 0;
-  if (g->counters) CUDA_TRY(cudaMemsetAsync(g->counters, 0, 8 * sizeof(unsigned long long), st));
-  unsigned char* scratch = w + c.total;
-  return lgar_reverse_unit_launch(s.FM, &P, s.S, s.chunk, backward_slots(s), backward_arena_cap(s), LGAR_TAPE_CAP, g_num_sms,
-                                  scratch, (void*)st, g_err, sizeof(g_err));
+  P.K.time_phases = g->counters ? 1 : 0;
+  if (g->counters) CUDA_TRY(cudaMemsetAsync(g->counters, 0, 8 * sizeof(unsigned long long), (cudaStream_t)stream));
+  return lgar_reverse_unit_launch(s.FM, &P, g_num_sms, stream, g_err, sizeof(g_err));
 }
 
 int lgar_backward(const lgar_problem* p, const double* grad_per_step, uint32_t grad_mask, const double* grad_sums,
@@ -407,11 +381,8 @@ int lgar_backward(const lgar_problem* p, const double* grad_per_step, uint32_t g
 
 int lgar_forward_host(const lgar_problem* ph, const lgar_outputs* oh) {
   Shape s;
-  int rc = shape_of(ph, s);
-  if (rc) return rc;
-  if (!oh) return fail(LGAR_E_INVALID, "outputs is NULL");
-  rc = lgar_device_check();
-  if (rc) return rc;
+  int rc = check_args(FORWARD, ph, 0, oh, nullptr, s);
+  if (rc || (rc = lgar_device_check())) return rc;
   DevBuf db;
   lgar_problem p = *ph;
   lgar_outputs o = *oh;
@@ -420,12 +391,12 @@ int lgar_forward_host(const lgar_problem* ph, const lgar_outputs* oh) {
   UP(alpha, LB) UP(n, LB) UP(ksat, LB) UP(theta_r, LB) UP(theta_e, LB) UP(thickness, LB)
   UP(initial_psi, B) UP(ponded_depth_max, B) UP(forcing, (size_t)ph->num_sites * T * 2) UP(site_index, B) UP(column_order, B)
 #undef UP
-#define AL(field, count) if ((rc = db.alloc(oh->field, (count), &o.field))) return rc;
-  AL(per_step, (size_t)__builtin_popcount(oh->per_step_mask) * T * B) AL(sums, (size_t)LGAR_NUM_OUTPUTS * B) AL(start_volume, B)
-  AL(status, B) AL(crash_step, B) AL(num_fronts, T * B) AL(fronts, T * LGAR_MAX_FRONTS * 5 * B)
-  AL(front_layer, T * LGAR_MAX_FRONTS * B) AL(front_to_bottom, T * LGAR_MAX_FRONTS * B) AL(counters, 16)
-  AL(tile_cycles, (size_t)(oh->tile_diag_rows == 3 ? 3 : 1) * s.ntiles)
-#undef AL
+#define OUT(field, count) if ((rc = db.out(oh->field, (count), &o.field))) return rc;
+  OUT(per_step, (size_t)__builtin_popcount(oh->per_step_mask) * T * B) OUT(sums, (size_t)LGAR_NUM_OUTPUTS * B)
+  OUT(start_volume, B) OUT(status, B) OUT(crash_step, B) OUT(num_fronts, T * B) OUT(fronts, T * LGAR_MAX_FRONTS * 5 * B)
+  OUT(front_layer, T * LGAR_MAX_FRONTS * B) OUT(front_to_bottom, T * LGAR_MAX_FRONTS * B) OUT(counters, 16)
+  OUT(tile_cycles, (size_t)(oh->tile_diag_rows == 3 ? 3 : 1) * s.ntiles)
+#undef OUT
   const size_t wsb = lgar_workspace_bytes(&p, 0);
   void* ws = nullptr;
   CUDA_TRY(cudaMalloc(&ws, wsb));
@@ -433,14 +404,7 @@ int lgar_forward_host(const lgar_problem* ph, const lgar_outputs* oh) {
   rc = lgar_forward(&p, &o, ws, wsb, 0, nullptr);
   if (rc) return rc;
   CUDA_TRY(cudaDeviceSynchronize());
-#define DOWN(field, count) \
-  if (oh->field) CUDA_TRY(cudaMemcpy(oh->field, o.field, (count) * sizeof(*oh->field), cudaMemcpyDeviceToHost));
-  DOWN(per_step, (size_t)__builtin_popcount(oh->per_step_mask) * T * B) DOWN(sums, (size_t)LGAR_NUM_OUTPUTS * B) DOWN(start_volume, B)
-  DOWN(status, B) DOWN(crash_step, B) DOWN(num_fronts, T * B) DOWN(fronts, T * LGAR_MAX_FRONTS * 5 * B)
-  DOWN(front_layer, T * LGAR_MAX_FRONTS * B) DOWN(front_to_bottom, T * LGAR_MAX_FRONTS * B) DOWN(counters, 16)
-  DOWN(tile_cycles, (size_t)(oh->tile_diag_rows == 3 ? 3 : 1) * s.ntiles)
-#undef DOWN
-  return 0;
+  return db.download();
 }
 
 }  // extern "C"

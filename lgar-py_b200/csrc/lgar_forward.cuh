@@ -56,6 +56,12 @@ struct KParams {
   long long iter_cap;
 };
 
+// host: every region of the workspace starts on a 256-byte boundary; without a workspace (sizing only) the region
+// pointers stay null
+inline size_t align_up(size_t x) { return (x + 255) / 256 * 256; }
+template <class T>
+T* at(unsigned char* w, size_t off) { return w ? reinterpret_cast<T*>(w + off) : nullptr; }
+
 template <int FM, class R, int LM = 0>
 struct Tile {
   Column<FM, R, LM> col;
@@ -564,6 +570,12 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       "}\n" ::"r"(smem_addr(bar)),
       "r"(parity)
       : "memory");
+}
+
+// dynamic shared memory of lgar_forward_kernel<FM>: the carve at the top of the kernel
+template <int FM>
+constexpr size_t forward_smem_bytes() {
+  return (size_t)5 * FM * NT * sizeof(double) + (size_t)WARPS * NODEBUF * sizeof(double) + (size_t)FM * NT;
 }
 
 // resident CTAs per SM are bounded by the shared-memory front lists: 1 (FM = 32, the fallback for the rare columns
