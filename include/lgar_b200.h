@@ -40,12 +40,27 @@
 extern "C" {
 #endif
 
-#define LGAR_ABI_VERSION 2
+#define LGAR_ABI_VERSION 3     /* 3: soil-moisture outputs (num_depths, moisture_depths, moisture, layer_water) */
 #define LGAR_MAX_LAYERS 4      /* soil layers per column (all reference configs use 3)            */
 #define LGAR_MAX_FRONTS 16     /* capacity of the wetting-front list of one column                */
 #define LGAR_MAX_GIUH 8        /* GIUH ordinates (reference: 5, data/config/Phillipsburg.yaml)    */
 #define LGAR_NUM_OUTPUTS 10
+#define LGAR_MAX_DEPTHS 8      /* sensor depths of the soil-moisture output (lgar_problem.moisture_depths)   */
 
+/* Soil moisture (lgar_outputs.moisture / layer_water), read off the column state at the END of every forcing
+ * step (after its last sub-step), the same point the rows of per_step are read at.  "The list of layer l" is the
+ * l-th block of the front list, cnt(l) fronts long (Layer.wetting_fronts of the reference).
+ *   layer water W_l (cm): the per-layer term of Layer.mass_balance (Layer.py:795-824) in its exact operation order:
+ *       top_l = 0 for l = 0, else cum_l - thickness_l (cum_l = thickness_0 + ... + thickness_l, summed in that order);
+ *       W_l = 0 + sum over the fronts i of the list except the last of (depth_i - top_l) * (theta_i - theta_{i+1}),
+ *             then + (depth_last - top_l) * theta_last.
+ *     W_0 + (W_1 + (W_2 ...)) is the column's mass balance, so on every step of an OK column it equals the
+ *     ENDING_VOLUME output bit for bit.  The layer-average water content is W_l / thickness_l.
+ *   theta at depth z (cm below the surface, z > 0): the layer l with cum_{l-1} < z <= cum_l (a depth on a layer
+ *     bottom belongs to the upper layer); theta(z) is the theta of the FIRST front of layer l's list, in list order,
+ *     whose depth >= z.  A selection, bit-identical to that front's theta; NaN if z > cum_{L-1} or no front of the
+ *     list qualifies.  Its gradient flows into the theta of the selected front; the selection carries none.
+ *   A column that crashed gets NaN from its crash step on (like per_step); earlier steps keep their values.   */
 /* per-forcing-step output variables (index into the [NOUT][T][B] output array); the same
  * accumulators MassBalance.change_mass reads and zeroes (physics/MassBalance.py:31-53)          */
 enum lgar_output {
@@ -120,7 +135,8 @@ typedef struct lgar_problem {
                               longer idle the GPU before the next.  Nothing else may be enqueued on the
                               stream between two calls of a sequence (it would serialise them again); the
                               results of all windows are complete when the stream has drained.           */
-  int32_t reserved1;
+  int32_t num_depths;      /* 0..LGAR_MAX_DEPTHS sensor depths of lgar_outputs.moisture (0 = none); was reserved (0)
+                              before ABI 3                                                                  */
   int64_t iter_cap;        /* root-finder iteration cap (0 = default 1,000,000)                 */
   double subcycle_length_h;   /* dt in hours                 cfg.models.subcycle_length_h       */
   double wilting_point_psi;   /* cm                          cfg.data.wilting_point_psi         */
@@ -145,6 +161,9 @@ typedef struct lgar_problem {
                               depend on it).  A warp advances its 32 columns in lock step, so grouping columns of
                               similar cost (e.g. sorted by top-layer ksat) raises lane utilisation.  lgar_backward
                               and resumed calls must pass the order of the lgar_forward they follow.           */
+  double moisture_depths[LGAR_MAX_DEPTHS]; /* cm below the surface, each finite and > 0; the first num_depths are
+                              used.  Shared by all columns; read by lgar_forward (moisture) and by
+                              lgar_backward_ex (grad_moisture)                                              */
 } lgar_problem;
 
 /* Output buffers.  Any pointer may be NULL (that output is skipped).                           */
@@ -176,6 +195,9 @@ typedef struct lgar_outputs {
    * spent WAITING for their predecessor chunk (a resident warp blocked on the per-tile progress counter), and the
    * global timer (ns) at the end of the tile's last chunk of this launch -- the scheduler's idle time and tail */
   unsigned long long* tile_cycles; /* [tile_diag_rows][ceil(B/32)]                              */
+  /* soil moisture after every step (definitions above LGAR_MAX_DEPTHS); may be NULL                        */
+  double* moisture;        /* [num_depths][T][B] theta at moisture_depths[d]; needs num_depths > 0            */
+  double* layer_water;     /* [L][T][B] water stored in each layer, cm                                        */
 } lgar_outputs;
 
 /* Library / device probe.  Returns 0 if an sm_100 device is current and usable.               */
@@ -235,6 +257,8 @@ typedef struct lgar_gradients {
                                     declares it as a parameter in a commented-out line (models/dpLGAR.py:48-49); as a
                                     leaf it reaches the loss through update_ponded_depth (models/dpLGAR.py:369-382) and
                                     insert_water (Layer.py:1509-1532)                                              */
+  const double* grad_moisture;    /* [num_depths][T][B] dL/d(lgar_outputs.moisture) or NULL (needs num_depths > 0)  */
+  const double* grad_layer_water; /* [L][T][B] dL/d(lgar_outputs.layer_water) or NULL                              */
 } lgar_gradients;
 int lgar_backward_ex(const lgar_problem* p, const lgar_gradients* g, void* workspace_dev, size_t workspace_bytes,
                      void* stream);

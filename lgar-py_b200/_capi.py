@@ -13,8 +13,9 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # LGAR_B200_LIB: developer override used to A/B two builds of the same library on one GPU box
 LIB_PATH = os.environ.get("LGAR_B200_LIB") or os.path.join(_HERE, "liblgar_b200.so")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 MAX_LAYERS, MAX_FRONTS, MAX_GIUH, NUM_OUTPUTS = 4, 16, 8, 10
+MAX_DEPTHS = 8  # sensor depths of the soil-moisture output (lgar_problem.moisture_depths)
 OUT_NAMES = ("runoff", "percolation", "AET", "infiltration", "ending_volume", "ponded_water",
              "giuh_runoff", "precip", "PET", "discharge")
 STATUS_NAMES = ("OK", "NEG_POW", "NAN", "THETA_ORDER", "BOTTOM_REACHED", "NULL_NEIGHBOUR",
@@ -31,13 +32,14 @@ class Problem(C.Structure):
         ("num_steps", C.c_int32), ("num_subcycles", C.c_int32), ("num_sites", C.c_int32),
         ("nint", C.c_int32), ("num_giuh", C.c_int32), ("max_fronts", C.c_int32),
         ("chunk_steps", C.c_int32), ("resume", C.c_int32), ("use_closed_form_G", C.c_int32),
-        ("step_begin", C.c_int32), ("step_end", C.c_int32), ("pipeline_seq", C.c_int32), ("reserved1", C.c_int32),
+        ("step_begin", C.c_int32), ("step_end", C.c_int32), ("pipeline_seq", C.c_int32), ("num_depths", C.c_int32),
         ("iter_cap", C.c_int64),
         ("subcycle_length_h", C.c_double), ("wilting_point_psi", C.c_double),
         ("frozen_factor", C.c_double), ("giuh_ordinates", C.c_double * MAX_GIUH),
         ("alpha", _dp), ("n", _dp), ("ksat", _dp), ("theta_r", _dp), ("theta_e", _dp),
         ("thickness", _dp), ("initial_psi", _dp), ("ponded_depth_max", _dp),
         ("forcing", _dp), ("site_index", _dp), ("column_order", _dp),
+        ("moisture_depths", C.c_double * MAX_DEPTHS),
     ]
 
 
@@ -46,7 +48,7 @@ class Outputs(C.Structure):
         ("per_step", _dp), ("per_step_mask", C.c_uint32), ("tile_diag_rows", C.c_int32),
         ("sums", _dp), ("start_volume", _dp), ("status", _dp), ("crash_step", _dp),
         ("num_fronts", _dp), ("fronts", _dp), ("front_layer", _dp), ("front_to_bottom", _dp),
-        ("counters", _dp), ("tile_cycles", _dp),
+        ("counters", _dp), ("tile_cycles", _dp), ("moisture", _dp), ("layer_water", _dp),
     ]
 
 
@@ -54,7 +56,7 @@ class Gradients(C.Structure):
     _fields_ = [
         ("grad_per_step", _dp), ("grad_mask", C.c_uint32), ("reduce", C.c_int32), ("grad_sums", _dp),
         ("grad_alpha", _dp), ("grad_n", _dp), ("grad_ksat", _dp), ("partials", _dp), ("tape_overflow", _dp),
-        ("counters", _dp), ("grad_ponded_depth_max", _dp),
+        ("counters", _dp), ("grad_ponded_depth_max", _dp), ("grad_moisture", _dp), ("grad_layer_water", _dp),
     ]
 
 

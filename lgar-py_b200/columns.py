@@ -14,13 +14,14 @@ arrive on the host, and the call fails loudly if the library or an sm_100 GPU is
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass, field
 from typing import Optional, Sequence
 
 import torch
 
 from . import _capi
-from ._capi import NUM_OUTPUTS, OUT_NAMES, MAX_FRONTS
+from ._capi import NUM_OUTPUTS, OUT_NAMES, MAX_FRONTS, MAX_DEPTHS
 
 F64 = torch.float64
 
@@ -63,6 +64,9 @@ class ColumnEnsemble:
     last_reverse_counters: Optional[torch.Tensor] = field(default=None, repr=False)
     device: object = "cuda"
     _keep: list = field(default_factory=list, repr=False)
+    # sensor depths (cm below the surface, at most 8, each > 0) of the soil-moisture output theta(z), shared by all
+    # columns (lgar_problem.moisture_depths; definition in lgar_b200.h).  Last, so positional arguments keep their meaning
+    moisture_depths: Optional[Sequence[float]] = None
 
     def __post_init__(self):
         dev = torch.device(self.device)
@@ -86,6 +90,7 @@ class ColumnEnsemble:
             assert self.column_order.shape == (B,)
         self.initial_psi = _dev_f64(self.initial_psi, dev, (B,))
         self.ponded_depth_max = _dev_f64(self.ponded_depth_max, dev, (B,))
+        self.moisture_depths = check_moisture_depths(self.moisture_depths)
 
     @property
     def num_layers(self): return self.theta_r.shape[0]
@@ -93,6 +98,8 @@ class ColumnEnsemble:
     def num_columns(self): return self.theta_r.shape[1]
     @property
     def num_steps(self): return self.forcing.shape[1]
+    @property
+    def num_depths(self): return len(self.moisture_depths)
 
     def problem(self, alpha, n, ksat, ponded_depth_max=None) -> _capi.Problem:
         p = _capi.Problem()
@@ -115,6 +122,9 @@ class ColumnEnsemble:
         p.forcing = self.forcing.data_ptr()
         p.site_index = self.site_index.data_ptr() if self.site_index is not None else None
         p.column_order = self.column_order.data_ptr() if self.column_order is not None else None
+        p.num_depths = self.num_depths
+        for i, z in enumerate(self.moisture_depths):
+            p.moisture_depths[i] = z
         return p
 
     def check_tape_overflow(self, raise_error=True) -> int:
@@ -145,6 +155,19 @@ class ColumnEnsemble:
         return self
 
 
+def check_moisture_depths(depths) -> tuple:
+    """The sensor depths as a tuple of floats; raises ValueError for more than MAX_DEPTHS depths or a depth that is not
+    finite and > 0 (before anything is launched)."""
+    if depths is None:
+        return ()
+    z = tuple(float(v) for v in torch.as_tensor(depths, dtype=F64).reshape(-1).tolist())
+    if len(z) > MAX_DEPTHS:
+        raise ValueError(f"moisture_depths: at most {MAX_DEPTHS} depths, got {len(z)}")
+    if not all(math.isfinite(v) and v > 0.0 for v in z):
+        raise ValueError(f"moisture_depths: every depth must be finite and > 0 cm, got {z}")
+    return z
+
+
 def output_mask(names) -> int:
     m = 0
     for nme in names:
@@ -166,6 +189,8 @@ class ForwardResult:
     front_to_bottom: Optional[torch.Tensor] = None # [T,16,B]
     counters: Optional[torch.Tensor] = None        # [16] int64: 8 work counters + phase timers (lgar_b200.h)
     tile_cycles: Optional[torch.Tensor] = None     # [ceil(B/32)] int64 (diagnostics); [3, ceil(B/32)] with counters
+    moisture: Optional[torch.Tensor] = None        # [D,T,B] theta at ens.moisture_depths (lgar_b200.h)
+    layer_water: Optional[torch.Tensor] = None     # [L,T,B] water stored in each layer, cm
     overflow_reruns: int = 0                       # columns rerun with the 32-front kernel (overflow_fallback)
 
     def __getitem__(self, name) -> torch.Tensor:
@@ -184,7 +209,8 @@ def _param(x, ens: ColumnEnsemble):
 FRONT_OVERFLOW = 6  # lgar_status: more than max_fronts wetting fronts (capacity of the library, not a reference state)
 
 
-def _rerun_overflowed(ens: ColumnEnsemble, alpha, n, ksat, res: "ForwardResult", outputs, per_step) -> int:
+def _rerun_overflowed(ens: ColumnEnsemble, alpha, n, ksat, res: "ForwardResult", outputs, per_step, moisture=False,
+                      layer_water=False) -> int:
     """The reference's front lists are unbounded; the production kernels hold 16 fronts per column in shared memory.
     The (rare: ~0.07 % of the bench ensemble over a year) columns that overflow are run again with the 32-front
     instantiation (one CTA per SM) and their results scattered into `res`.  Returns the number of columns rerun."""
@@ -197,11 +223,17 @@ def _rerun_overflowed(ens: ColumnEnsemble, alpha, n, ksat, res: "ForwardResult",
         ponded_depth_max=ens.ponded_depth_max[idx], subcycle_length_h=ens.subcycle_length_h,
         num_subcycles=ens.num_subcycles, nint=ens.nint, wilting_point_psi=ens.wilting_point_psi,
         frozen_factor=ens.frozen_factor, use_closed_form_G=ens.use_closed_form_G, giuh_ordinates=ens.giuh_ordinates,
-        max_fronts=32, chunk_steps=ens.chunk_steps, iter_cap=ens.iter_cap, device=ens.device)
+        max_fronts=32, chunk_steps=ens.chunk_steps, iter_cap=ens.iter_cap, moisture_depths=ens.moisture_depths,
+        device=ens.device)
     r2, _ = forward_raw(sub, alpha[:, idx].contiguous(), n[:, idx].contiguous(), ksat[:, idx].contiguous(), outputs=outputs,
-                        per_step=per_step, num_fronts=res.num_fronts is not None, overflow_fallback=False)
+                        per_step=per_step, num_fronts=res.num_fronts is not None, overflow_fallback=False,
+                        moisture=moisture, layer_water=layer_water)
     if res.per_step is not None:
         res.per_step[:, :, idx] = r2.per_step
+    if moisture:
+        res.moisture[:, :, idx] = r2.moisture
+    if layer_water:
+        res.layer_water[:, :, idx] = r2.layer_water
     res.sums[:, idx] = r2.sums
     res.start_volume[idx] = r2.start_volume
     res.status[idx] = r2.status
@@ -214,7 +246,8 @@ def _rerun_overflowed(ens: ColumnEnsemble, alpha, n, ksat, res: "ForwardResult",
 def forward_raw(ens: ColumnEnsemble, alpha, n, ksat, outputs=("runoff", "percolation"), per_step=True,
                 num_fronts=False, dump_fronts=False, counters=False, tile_cycles=False, keep_checkpoints=False,
                 workspace: Optional[torch.Tensor] = None, overflow_fallback=False, window=None,
-                into: Optional[ForwardResult] = None, pipeline_seq: int = 0, ponded_depth_max=None) -> tuple[ForwardResult, torch.Tensor]:
+                into: Optional[ForwardResult] = None, pipeline_seq: int = 0, ponded_depth_max=None, moisture=False,
+                layer_water=False) -> tuple[ForwardResult, torch.Tensor]:
     """One persistent launch over all columns and all forcing steps (no autograd).
     overflow_fallback: rerun the columns that overflowed the front list with the 32-front kernel (synchronises:
     the status array is inspected on the host).
@@ -225,9 +258,14 @@ def forward_raw(ens: ColumnEnsemble, alpha, n, ksat, outputs=("runoff", "percola
     reports crash_step = -2 - t (t = the absolute step).
     pipeline_seq=k (1, 2, ...): the k-th consecutive window of a pipelined sequence (lgar_problem.pipeline_seq):
     windows k > 1 start on the SMs the previous window has drained (programmatic dependent launch); enqueue nothing
-    else on the stream between them."""
+    else on the stream between them.
+    moisture / layer_water: also store the soil-moisture outputs of every step, `res.moisture[D,T,B]` (theta at
+    ens.moisture_depths) and `res.layer_water[L,T,B]` (cm); definitions in lgar_b200.h.  Windows fill their rows like
+    per_step."""
     L_ = _capi.lib()
     dev = ens.device
+    if moisture and ens.num_depths == 0:
+        raise ValueError("moisture=True needs ColumnEnsemble(moisture_depths=...)")
     alpha, n, ksat = _param(alpha, ens), _param(n, ens), _param(ksat, ens)
     B, T = ens.num_columns, ens.num_steps
     if ponded_depth_max is not None:  # [B] override of ens.ponded_depth_max (e.g. a learnable one)
@@ -259,6 +297,14 @@ def forward_raw(ens: ColumnEnsemble, alpha, n, ksat, outputs=("runoff", "percola
     o.per_step_mask = mask
     o.sums, o.start_volume = res.sums.data_ptr(), res.start_volume.data_ptr()
     o.status, o.crash_step = res.status.data_ptr(), res.crash_step.data_ptr()
+    if moisture:
+        if res.moisture is None:
+            res.moisture = torch.empty((ens.num_depths, T, B), dtype=F64, device=dev)
+        o.moisture = res.moisture.data_ptr()
+    if layer_water:
+        if res.layer_water is None:
+            res.layer_water = torch.empty((ens.num_layers, T, B), dtype=F64, device=dev)
+        o.layer_water = res.layer_water.data_ptr()
     if num_fronts or dump_fronts:
         if res.num_fronts is None:
             res.num_fronts = torch.empty((T, B), dtype=torch.int32, device=dev)
@@ -285,17 +331,19 @@ def forward_raw(ens: ColumnEnsemble, alpha, n, ksat, outputs=("runoff", "percola
     _capi.check(rc, "lgar_forward")
     res._keep = (alpha, n, ksat, ens, ponded_depth_max)  # keep inputs alive until the stream has consumed them
     if overflow_fallback and not keep_checkpoints and not dump_fronts:
-        res.overflow_reruns = _rerun_overflowed(ens, alpha, n, ksat, res, outputs, per_step)
+        res.overflow_reruns = _rerun_overflowed(ens, alpha, n, ksat, res, outputs, per_step, moisture, layer_water)
     return res, workspace
 
 
 class _LGARFunction(torch.autograd.Function):
     """autograd bridge: forward = lgar_forward (stores chunk checkpoints), backward = lgar_backward_ex.
     Parameters given as `[L]` vectors are SHARED by all columns: their gradient (the sum over columns) is reduced
-    inside the library in a fixed order (no torch reduction kernel, bit-reproducible)."""
+    inside the library in a fixed order (no torch reduction kernel, bit-reproducible).  The soil-moisture outputs
+    (moisture, layer_water) are outputs of their own, empty when not requested."""
 
     @staticmethod
-    def forward(ctx, alpha, n, ksat, pdm, ens: ColumnEnsemble, mask: int):
+    def forward(ctx, alpha, n, ksat, pdm, ens: ColumnEnsemble, mask: int, moisture: bool = False,
+                layer_water: bool = False):
         outputs = [OUT_NAMES[k] for k in range(NUM_OUTPUTS) if (mask >> k) & 1]
         need_grad = any(ctx.needs_input_grad[:4])
         B = ens.num_columns
@@ -304,7 +352,8 @@ class _LGARFunction(torch.autograd.Function):
             pdm_b = pdm.detach().to(ens.device, F64)
             pdm_b = (pdm_b.reshape(1).expand(B) if pdm_b.numel() == 1 else pdm_b.reshape(B)).contiguous()
         res, ws = forward_raw(ens, alpha.detach(), n.detach(), ksat.detach(), outputs=outputs,
-                              keep_checkpoints=need_grad, ponded_depth_max=pdm_b)
+                              keep_checkpoints=need_grad, ponded_depth_max=pdm_b, moisture=moisture,
+                              layer_water=layer_water)
         ctx.ens, ctx.mask, ctx.ws = ens, mask, ws
         ctx.save_for_backward(*res._keep[:3])
         ctx.pdm_b = res._keep[4]
@@ -312,14 +361,22 @@ class _LGARFunction(torch.autograd.Function):
         ctx.want_pdm = pdm is not None and ctx.needs_input_grad[3]
         ctx.in_shapes = (alpha.shape, n.shape, ksat.shape)
         ctx.mark_non_differentiable(res.status, res.crash_step, res.start_volume)
-        per_step = res.per_step if res.per_step is not None else torch.zeros(0, dtype=F64, device=ens.device)
-        return per_step, res.sums, res.start_volume, res.status, res.crash_step
+        # an output the loss does not use gets no gradient (None): the soil-moisture outputs then pass NULL to the
+        # reverse pass, which leaves it exactly as without them; per_step and sums keep their zero gradients
+        ctx.set_materialize_grads(False)
+        empty = lambda x: x if x is not None else torch.zeros(0, dtype=F64, device=ens.device)
+        return (empty(res.per_step), res.sums, res.start_volume, res.status, res.crash_step, empty(res.moisture),
+                empty(res.layer_water))
 
     @staticmethod
-    def backward(ctx, g_per_step, g_sums, _gsv, _gst, _gcs):
+    def backward(ctx, g_per_step, g_sums, _gsv, _gst, _gcs, g_moisture, g_layer_water):
         L_ = _capi.lib()
         ens: ColumnEnsemble = ctx.ens
         alpha, n, ksat = ctx.saved_tensors
+        if g_per_step is None:
+            g_per_step = torch.zeros(bin(ctx.mask).count("1"), ens.num_steps, ens.num_columns, dtype=F64, device=ens.device)
+        if g_sums is None:
+            g_sums = torch.zeros(NUM_OUTPUTS, ens.num_columns, dtype=F64, device=ens.device)
         dev = ens.device
         Lr, B = ens.num_layers, ens.num_columns
         p = ens.problem(alpha, n, ksat, ctx.pdm_b)
@@ -341,6 +398,10 @@ class _LGARFunction(torch.autograd.Function):
         g.grad_per_step = gps.data_ptr() if gps is not None else None
         g.grad_mask = ctx.mask
         g.grad_sums = gs.data_ptr() if gs is not None else None
+        gm = g_moisture.contiguous() if (g_moisture is not None and g_moisture.numel()) else None
+        gl = g_layer_water.contiguous() if (g_layer_water is not None and g_layer_water.numel()) else None
+        g.grad_moisture = gm.data_ptr() if gm is not None else None
+        g.grad_layer_water = gl.data_ptr() if gl is not None else None
         g.grad_alpha, g.grad_n, g.grad_ksat = ga.data_ptr(), gn.data_ptr(), gk.data_ptr()
         g.tape_overflow = overflow.data_ptr()
         partials = None
@@ -365,7 +426,7 @@ class _LGARFunction(torch.autograd.Function):
         gp_out = None
         if gp is not None:
             gp_out = (gp.sum() if (pdm_shared and gp.numel() > 1) else gp).reshape(ctx.pdm_shape)
-        return shape_back(ga, sa), shape_back(gn, sn), shape_back(gk, sk), gp_out, None, None
+        return shape_back(ga, sa), shape_back(gn, sn), shape_back(gk, sk), gp_out, None, None, None, None
 
 
 def lgar_columns(alpha, n, ksat, ens: ColumnEnsemble, outputs=("runoff", "percolation"), ponded_depth_max=None):
@@ -373,7 +434,15 @@ def lgar_columns(alpha, n, ksat, ens: ColumnEnsemble, outputs=("runoff", "percol
     ponded_depth_max (optional): a scalar (shared) or `[B]` tensor that replaces ens.ponded_depth_max; if it requires
     grad it is a gradient leaf like alpha/n/ksat (the reference's commented-out parameter, models/dpLGAR.py:48-49).
     Returns a dict: every requested output as `[T,B]`, plus `sums[NOUT,B]`, `start_volume[B]`,
-    `status[B]`, `crash_step[B]`."""
+    `status[B]`, `crash_step[B]`.
+    Soil moisture (definitions in lgar_b200.h), also differentiable: "moisture" in `outputs` adds `moisture[D,T,B]`,
+    theta at ens.moisture_depths; "layer_water" adds `layer_water[L,T,B]` (cm) and `layer_theta[L,T,B]` = layer_water /
+    thickness, the layer-average water content."""
+    outputs = tuple(outputs)
+    moisture, layer_water = "moisture" in outputs, "layer_water" in outputs
+    if moisture and ens.num_depths == 0:
+        raise ValueError('"moisture" needs ColumnEnsemble(moisture_depths=...)')
+    outputs = tuple(nm for nm in outputs if nm not in ("moisture", "layer_water"))
     mask = output_mask(outputs)
     dev = ens.device
     a = torch.as_tensor(alpha, dtype=F64).to(dev)
@@ -384,7 +453,13 @@ def lgar_columns(alpha, n, ksat, ens: ColumnEnsemble, outputs=("runoff", "percol
         nn_ = nn_ if nn_.dim() == 2 else nn_.unsqueeze(1).expand(ens.num_layers, ens.num_columns)
         k = k if k.dim() == 2 else k.unsqueeze(1).expand(ens.num_layers, ens.num_columns)
     pdm = None if ponded_depth_max is None else torch.as_tensor(ponded_depth_max, dtype=F64).to(dev)
-    per_step, sums, sv, st, cs = _LGARFunction.apply(a.contiguous(), nn_.contiguous(), k.contiguous(), pdm, ens, mask)
+    per_step, sums, sv, st, cs, moist, lw = _LGARFunction.apply(a.contiguous(), nn_.contiguous(), k.contiguous(), pdm,
+                                                                ens, mask, moisture, layer_water)
     out = {name: per_step[bin(mask & ((1 << OUT_NAMES.index(name)) - 1)).count("1")] for name in outputs}
     out.update(sums=sums, start_volume=sv, status=st, crash_step=cs)
+    if moisture:
+        out["moisture"] = moist
+    if layer_water:
+        out["layer_water"] = lw
+        out["layer_theta"] = lw / ens.thickness[:, None, :]
     return out

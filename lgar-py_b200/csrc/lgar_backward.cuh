@@ -65,6 +65,8 @@ struct BParams {
   double* grad_n;
   double* grad_ksat;
   double* grad_pdm;             // [B] (or [1] with reduce) dL/d ponded_depth_max, or NULL
+  const double* grad_moisture;  // [num_depths][T][B] dL/d(theta at the sensor depths) or NULL
+  const double* grad_layer_water;  // [L][T][B] dL/d(layer water) or NULL
   // per resident warp scratch
   TapeEntry* tape;              // [slots][arena_cap][32]: the tapes of all sub-steps of one chunk, back to back
   unsigned char* meta;          // [slots][ring_steps][32] StepMeta
@@ -92,6 +94,32 @@ template <int FM>
 constexpr size_t backward_smem_bytes() {
   return (size_t)5 * FM * NT * sizeof(double) + (size_t)WARPS * NODEBUF * sizeof(double) +
          (size_t)5 * FM * NT * sizeof(short) + (size_t)FM * NT;
+}
+
+// Soil-moisture outputs of a forcing step whose gradient is requested (lgar_b200.h), read off the END state of its last
+// sub-step and appended to that sub-step's tape as one entry each, in a fixed order: theta at every sensor depth
+// (a copy of the selected front's theta; the selection carries no gradient, no front: an entry without input), then the
+// water of every layer (a copy of W_l, formed on the tape by the same routine as the mass balance).  The reverse sweep
+// seeds dL/d(output) into these last entries of the sub-step, which therefore need no record of their ids.
+template <int FM>
+__device__ void tape_soil_moisture(const BParams& P, Column<FM, Var, 2>& C) {
+  const lgar_problem& p = P.K.p;
+  // the layer sums first (their own entries), so that the copies below are the last entries of the sub-step
+  int id_w[MAXL];
+  if (P.grad_layer_water) {
+    int o = 0;
+    for (int l = 0; l < C.L; l++) {
+      id_w[l] = C.template layer_water_t<Var>(l, o).id;
+      o += C.cnt(l);
+    }
+  }
+  if (P.grad_moisture)
+    for (int d = 0; d < p.num_depths; d++) {
+      const int i = C.front_at_depth(p.moisture_depths[d]);
+      tape_append(i >= 0 ? C.g(F_THETA, i) : Var(0.0));
+    }
+  if (P.grad_layer_water)
+    for (int l = 0; l < C.L; l++) tape_append(Var(0.0, id_w[l]));
 }
 
 // GM = 0: trapezoid Geff only (closed-form branch compiled out of the taped sub-step); GM = 2: run-time switch
@@ -131,6 +159,8 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
   Tv.ctx.iter_cap = K.iter_cap;
   Column<FM, Var, 2>& C = Tv.col;
   const unsigned long long nitems = (unsigned long long)K.ntiles * K.nchunks;
+  // tape entries of the soil-moisture outputs at the end of every forcing step (tape_soil_moisture)
+  const int nsm = (P.grad_moisture ? p.num_depths : 0) + (P.grad_layer_water ? p.num_layers : 0);
 
   for (;;) {
     if (lane == 0) sm_item[warp] = atomicAdd(P.next_tile, 1ULL);
@@ -228,6 +258,7 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
 #pragma unroll
           for (int k = 0; k < NOUT; k++) Tv.acc[k] = Var(0.0);
           substep<FM, Var, GM>(Tv, alive, x.x, x.y, K, nodebuf);
+          if (sc == S - 1 && nsm > 0 && alive && Tv.ctx.st == 0) tape_soil_moisture(P, C);
           __syncwarp();
           if (tc.n > tc.cap) overflow = true;
           const int ne = min(tc.n, tc.cap);
@@ -287,6 +318,14 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
             else if (k == LGAR_OUT_PONDED_WATER) id = (sc == S - 1) ? M.id_ponded : -1;
             else id = M.id_acc[k];
             if (id >= 0) adj[(size_t)id * 32] += g;
+          }
+          // dL / d(soil-moisture outputs of this forcing step): the last nsm entries of its last sub-step's tape
+          if (sc == S - 1 && nsm > 0) {
+            double* a = adj + (size_t)(NL + ne - nsm) * 32;
+            if (P.grad_moisture)
+              for (int d = 0; d < p.num_depths; d++, a += 32) *a += __ldg(P.grad_moisture + ((size_t)d * Tn + t) * B + b);
+            if (P.grad_layer_water)
+              for (int l = 0; l < p.num_layers; l++, a += 32) *a += __ldg(P.grad_layer_water + ((size_t)l * Tn + t) * B + b);
           }
           // the tape comes back from DRAM (the arenas of all resident warps are far larger than L2): fetch eight
           // entries at a time, independently of the adjoints, so that the misses overlap instead of queueing behind

@@ -4,6 +4,7 @@
 // There is no CPU fallback: without an sm_100 device every compute entry point fails.
 // =====================================================================================
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -81,8 +82,15 @@ int check_args(Entry entry, const lgar_problem* p, int with_grad, const lgar_out
   if (with_grad && (s.t_begin != 0 || s.t_end != s.T))
     return fail(LGAR_E_INVALID, "a step window (step_begin, step_end) is forward-only: checkpoints and lgar_backward "
                                 "need the whole record");
+  if (p->num_depths < 0 || p->num_depths > LGAR_MAX_DEPTHS)
+    return fail(LGAR_E_INVALID, "num_depths must be in [0, LGAR_MAX_DEPTHS]");
+  for (int d = 0; d < p->num_depths; d++)
+    if (!(std::isfinite(p->moisture_depths[d]) && p->moisture_depths[d] > 0.0))
+      return fail(LGAR_E_INVALID, "moisture_depths: every used depth must be finite and > 0");
   if (entry == BACKWARD) {
     if (!g) return fail(LGAR_E_INVALID, "gradients is NULL");
+    if (g->grad_moisture && p->num_depths == 0)
+      return fail(LGAR_E_INVALID, "grad_moisture needs num_depths > 0");
     if (!g->grad_alpha || !g->grad_n || !g->grad_ksat)
       return fail(LGAR_E_INVALID, "a gradient output array (grad_alpha, grad_n, grad_ksat) is NULL");
     if (g->reduce && !g->partials) return fail(LGAR_E_INVALID, "reduce needs the partials scratch array");
@@ -99,6 +107,7 @@ int check_args(Entry entry, const lgar_problem* p, int with_grad, const lgar_out
   if (p->pipeline_seq > 0 && with_grad) return fail(LGAR_E_INVALID, "pipeline_seq > 0 is forward-only");
   if (p->pipeline_seq > 1 && !p->resume) return fail(LGAR_E_INVALID, "pipeline_seq > 1 needs resume = 1");
   if (out->fronts && s.FM != 16) return fail(LGAR_E_INVALID, "front dumps (outputs.fronts) need max_fronts = 16");
+  if (out->moisture && p->num_depths == 0) return fail(LGAR_E_INVALID, "outputs.moisture needs num_depths > 0");
   return 0;
 }
 
@@ -356,6 +365,8 @@ int lgar_backward_ex(const lgar_problem* p, const lgar_gradients* g, void* works
   P.grad_n = g->grad_n;
   P.grad_ksat = g->grad_ksat;
   P.grad_pdm = g->grad_ponded_depth_max;
+  P.grad_moisture = g->grad_moisture;
+  P.grad_layer_water = g->grad_layer_water;
   P.tape_overflow = g->tape_overflow;
   P.reduce = g->reduce ? 1 : 0;
   P.partials = g->partials;
@@ -396,6 +407,7 @@ int lgar_forward_host(const lgar_problem* ph, const lgar_outputs* oh) {
   OUT(start_volume, B) OUT(status, B) OUT(crash_step, B) OUT(num_fronts, T * B) OUT(fronts, T * LGAR_MAX_FRONTS * 5 * B)
   OUT(front_layer, T * LGAR_MAX_FRONTS * B) OUT(front_to_bottom, T * LGAR_MAX_FRONTS * B) OUT(counters, 16)
   OUT(tile_cycles, (size_t)(oh->tile_diag_rows == 3 ? 3 : 1) * s.ntiles)
+  OUT(moisture, (size_t)ph->num_depths * T * B) OUT(layer_water, LB * T)
 #undef OUT
   const size_t wsb = lgar_workspace_bytes(&p, 0);
   void* ws = nullptr;

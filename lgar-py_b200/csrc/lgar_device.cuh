@@ -1039,20 +1039,27 @@ struct Column {
 
   // ---- Layer.mass_balance (Layer.py:795-824); association S0 + (S1 + (S2 ...)).
   //      Q = double evaluates values only (root-finder loops), Q = R is on the tape.
+  //      layer_water_t: the inner sum of layer l, whose list starts at flat index o (the soil-moisture output W_l,
+  //      lgar_b200.h); 0 for an empty list.
+  template <class Q>
+  __device__ __forceinline__ Q layer_water_t(int l, int o) {
+    const double base = (l == 0) ? 0.0 : (cum[l] - thick[l]);
+    const int nf = cnt(l);
+    Q sum(0.0);
+    for (int i = 0; i < nf - 1; i++)
+      sum = sum + (gq<Q>(F_DEPTH, o + i) - base) * (gq<Q>(F_THETA, o + i) - gq<Q>(F_THETA, o + i + 1));
+    if (nf > 0) sum = sum + (gq<Q>(F_DEPTH, o + nf - 1) - base) * gq<Q>(F_THETA, o + nf - 1);
+    return sum;
+  }
   template <class Q>
   __device__ Q mass_balance_t() {
     Q s_l[MAXL];
     empty_list = false;
     int o = 0;
     for (int l = 0; l < L; l++) {
-      const double base = (l == 0) ? 0.0 : (cum[l] - thick[l]);
       const int nf = cnt(l);
-      Q sum(0.0);
-      for (int i = 0; i < nf - 1; i++)
-        sum = sum + (gq<Q>(F_DEPTH, o + i) - base) * (gq<Q>(F_THETA, o + i) - gq<Q>(F_THETA, o + i + 1));
-      if (nf > 0) sum = sum + (gq<Q>(F_DEPTH, o + nf - 1) - base) * gq<Q>(F_THETA, o + nf - 1);
-      else empty_list = true;  // wetting_fronts[0] of an empty list: IndexError in the reference
-      s_l[l] = sum;
+      s_l[l] = layer_water_t<Q>(l, o);
+      if (nf == 0) empty_list = true;  // wetting_fronts[0] of an empty list: IndexError in the reference
       o += nf;
     }
     Q tot = s_l[L - 1];
@@ -1060,6 +1067,23 @@ struct Column {
     return tot;
   }
   __device__ __forceinline__ R mass_balance() { return mass_balance_t<R>(); }
+
+  // ---- soil-moisture output theta(z) (lgar_b200.h): flat index of the first front of the list of the layer holding
+  //      depth z (cum[l-1] < z <= cum[l]) whose depth >= z; -1 if z lies below the column or no front qualifies.
+  //      A selection: no arithmetic, nothing on the tape.
+  __device__ __forceinline__ int front_at_depth(double z) const {
+    int o = 0;
+    for (int l = 0; l < L; l++) {
+      const int nf = cnt(l);
+      if (z <= cum[l]) {
+        for (int i = o; i < o + nf; i++)
+          if (fb[(F_DEPTH * FM + i) * NT] >= z) return i;
+        return -1;
+      }
+      o += nf;
+    }
+    return -1;
+  }
 
   // ---- free-drainage front (models/dpLGAR.py:328-338, Layer.py:134-162): arg-min psi, ties ->
   //      deeper; else-branch torch.isclose(psi_i, psi, atol=1e-8) with default rtol 1e-5

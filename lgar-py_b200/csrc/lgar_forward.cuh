@@ -572,6 +572,27 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       : "memory");
 }
 
+// soil-moisture outputs of forcing step t (lgar_b200.h): theta at the sensor depths and the water of every layer, read
+// off the END state of the step; NaN where the column has crashed (ok == false) or no front qualifies
+template <int FM, class R, int LM>
+__device__ void store_soil_moisture(const KParams& K, Column<FM, R, LM>& C, bool ok, int t, int b) {
+  const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+  const size_t B = K.p.num_columns, Tn = K.p.num_steps;
+  if (K.o.moisture) {
+    for (int d = 0; d < K.p.num_depths; d++) {
+      const int i = ok ? C.front_at_depth(K.p.moisture_depths[d]) : -1;
+      K.o.moisture[((size_t)d * Tn + t) * B + b] = (i >= 0) ? C.f(F_THETA, i) : qnan;
+    }
+  }
+  if (K.o.layer_water) {
+    int o = 0;
+    for (int l = 0; l < C.L; l++) {
+      K.o.layer_water[((size_t)l * Tn + t) * B + b] = ok ? C.template layer_water_t<double>(l, o) : qnan;
+      o += C.cnt(l);
+    }
+  }
+}
+
 // dynamic shared memory of lgar_forward_kernel<FM>: the carve at the top of the kernel
 template <int FM>
 constexpr size_t forward_smem_bytes() {
@@ -743,6 +764,7 @@ __global__ void __launch_bounds__(NT, (FM == 32) ? 1 : ((FM == 16) ? 2 : ((FM ==
             T.sums[k] = (k == LGAR_OUT_ENDING_VOLUME || k == LGAR_OUT_PONDED_WATER) ? T.acc[k] : T.sums[k] + T.acc[k];
         }
         if (K.o.num_fronts) K.o.num_fronts[(size_t)t * B + b] = ok ? T.col.n : 0;
+        if (K.o.moisture || K.o.layer_water) store_soil_moisture(K, T.col, ok, t, b);
         if (DUMP && K.o.fronts) {
           for (int i = 0; i < LGAR_MAX_FRONTS; i++) {
             const bool has = ok && i < T.col.n;

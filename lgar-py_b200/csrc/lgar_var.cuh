@@ -56,6 +56,16 @@ __device__ __forceinline__ Var tape_record(double v, int a, double da, int b, do
   t.base[(size_t)k * 32] = e;
   return Var(v, t.first_id + k);
 }
+// one entry "copy of x" even when x is a constant (a < 0): callers that find entries by their position on the tape
+__device__ __forceinline__ void tape_append(const Var& x) {
+  TapeCtl& t = g_tapectl[threadIdx.x];
+  const int k = t.n;
+  t.n = k + 1;
+  if (k >= t.cap) return;  // overflow: detected by the kernel through n > cap
+  TapeEntry e;
+  e.a = x.id; e.b = -1; e.da = 1.0; e.db = 0.0;
+  t.base[(size_t)k * 32] = e;
+}
 // value = sum_j d_j * x_j over up to 6 inputs (macro closures)
 __device__ __forceinline__ Var tape_record_n(double v, int n, const int* ids, const double* d) {
   Var acc(0.0);

@@ -12,7 +12,11 @@ Mirrors the public surface of dpLGAR/models/dpLGAR.py:30-430 that its callers us
     accumulators `.precip .PET .AET .infiltration .runoff .percolation .giuh_runoff .discharge
     .groundwater_discharge`, `.ponded_water`, `.ending_volume` are kept and must be zeroed by the caller exactly like
     MassBalance.change_mass does;
-  * `set_internal_states()` resets the column to its initial state with the current parameters.
+  * `set_internal_states()` resets the column to its initial state with the current parameters;
+  * soil moisture (definitions in include/lgar_b200.h): with `moisture_depths` (ctor kwarg, else
+    cfg.data.moisture_depths) `forward_record` also returns `moisture[T,D]` (theta at those depths), `layer_water[T,L]`
+    (cm) and `layer_theta[T,L]`; after every one-row `forward`, `.soil_moisture[D]` and `.layer_water[L]` hold the
+    state at the end of that row (plain state, not accumulators: the caller's resets leave them alone).
 
 Differences (by design): one-row `forward` is a no-grad convenience; training uses `forward_record(x[T,2])`, which runs
 the whole record in one persistent launch and is differentiable through the reverse-mode kernel
@@ -28,7 +32,7 @@ import torch
 import torch.nn as nn
 
 from . import _capi
-from .columns import ColumnEnsemble, forward_raw, lgar_columns
+from .columns import ColumnEnsemble, check_moisture_depths, forward_raw, lgar_columns
 from ._capi import OUT_NAMES, STATUS_NAMES
 
 # data/utils.py:108-180 read_test_params (== alpha, n, Ks columns of data/vG_default_params.dat; rows 12-17 are
@@ -67,7 +71,7 @@ def read_soil_table(path):
 
 
 class dpLGAR(nn.Module):
-    def __init__(self, cfg, theta_r=None, theta_e=None, columns: int = 1, device="cuda") -> None:
+    def __init__(self, cfg, theta_r=None, theta_e=None, columns: int = 1, device="cuda", moisture_depths=None) -> None:
         super().__init__()
         self.cfg = cfg
         soil_types = list(_get(cfg, "data.layer_soil_type"))
@@ -95,6 +99,10 @@ class dpLGAR(nn.Module):
             subcycle_length_h=self.dt_h, num_subcycles=self.num_subcycles, nint=int(_get(cfg, "constants.nint", 120)),
             wilting_point_psi=float(_get(cfg, "data.wilting_point_psi", 15495.0)), frozen_factor=ff, giuh_ordinates=giuh,
             use_closed_form_G=bool(_get(cfg, "data.use_closed_form_G", False)))
+        if moisture_depths is None:
+            moisture_depths = _get(cfg, "data.moisture_depths")
+        self.moisture_depths = check_moisture_depths(moisture_depths)
+        self._ens_kw["moisture_depths"] = self.moisture_depths
         self._step_ens = None
         self._ws = None
         self.set_internal_states()
@@ -127,6 +135,8 @@ class dpLGAR(nn.Module):
             setattr(self, name, self._zero())
         self._started = False
         self._ws = None
+        self.soil_moisture = None  # [D] theta at moisture_depths after the last one-row forward
+        self.layer_water = None    # [L] cm
         # initial water volume: a zero-length-forcing run is not allowed, so use one dry row and read start_volume
         a, n, k = self._params()
         ens = self._ensemble(np.zeros((1, 2)))
@@ -140,7 +150,8 @@ class dpLGAR(nn.Module):
         f = torch.as_tensor(x, dtype=torch.float64).reshape(1, 1, 2)
         ens = self._ensemble(f, resume=self._started)
         with torch.no_grad():
-            res, self._ws = forward_raw(ens, a.detach(), n.detach(), k.detach(), outputs=OUT_NAMES, workspace=self._ws)
+            res, self._ws = forward_raw(ens, a.detach(), n.detach(), k.detach(), outputs=OUT_NAMES, workspace=self._ws,
+                                        moisture=len(self.moisture_depths) > 0, layer_water=True)
         self._started = True
         st = int(res.status[0])
         if st != 0:
@@ -150,14 +161,22 @@ class dpLGAR(nn.Module):
             setattr(self, name, getattr(self, name) + v[name])
         self.ponded_water = v["ponded_water"]
         self.ending_volume = v["ending_volume"]
+        self.soil_moisture = (res.moisture[:, 0, 0].cpu() if res.moisture is not None
+                              else torch.zeros(0, dtype=torch.float64))
+        self.layer_water = res.layer_water[:, 0, 0].cpu()
         return self.runoff, self.percolation
 
     def forward_record(self, x, outputs=("runoff", "percolation"), on_status="raise"):
         """Whole record `x[T,2]` in one persistent launch, from the initial state; differentiable in alpha/n/ksat.
         Returns a dict of `[T]` tensors (or `[T, columns]`).  on_status: what to do when a column ends with a non-zero
         status (its series are NaN from the crash step on): "raise" (default: the reference raises out of model(x)),
-        "warn" or "ignore" (the caller inspects out["status"] itself, like the agent does)."""
+        "warn" or "ignore" (the caller inspects out["status"] itself, like the agent does).
+        With moisture_depths configured the soil-moisture outputs are added: `moisture[T,D]`, `layer_water[T,L]`,
+        `layer_theta[T,L]` (with `columns > 1`: `[T,D,columns]` and `[T,L,columns]`)."""
         a, n, k = self._params()
+        outputs = tuple(outputs)
+        if self.moisture_depths:
+            outputs += tuple(nm for nm in ("moisture", "layer_water") if nm not in outputs)
         ens = self._ensemble(torch.as_tensor(x, dtype=torch.float64))
         self.last_ensemble = ens  # (the reverse pass leaves its tape-overflow flags there)
         # ponded_depth_max as a learnable parameter (models/dpLGAR.py:48, commented out upstream): make it one with
@@ -176,6 +195,9 @@ class dpLGAR(nn.Module):
                     raise RuntimeError(msg)
                 import warnings
                 warnings.warn(msg)
+        for key in ("moisture", "layer_water", "layer_theta"):  # [D or L, T, B] -> time first, like the other series
+            if key in out:
+                out[key] = out[key].permute(1, 0, 2)
         if self.columns == 1:
             out = {key: (val[..., 0] if val.dim() >= 1 and val.shape[-1] == 1 else val) for key, val in out.items()}
         return out
