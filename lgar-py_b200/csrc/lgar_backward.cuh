@@ -122,6 +122,71 @@ __device__ void tape_soil_moisture(const BParams& P, Column<FM, Var, 2>& C) {
     for (int l = 0; l < C.L; l++) tape_append(Var(0.0, id_w[l]));
 }
 
+// derived parameter on the tape: m = 1 - 1/n (data/utils.py:75)
+template <int FM>
+__device__ __forceinline__ void tape_m(Column<FM, Var, 2>& C) {
+  for (int l = 0; l < C.L; l++) {
+    SoilT<Var>& sl = C.soil[l];
+    Var mV = 1.0 - (1.0 / Var(sl.n, sl.id_n));
+    sl.id_m = mV.id;
+  }
+}
+
+// the tape ids the column state ended up with: the END state of a sub-step, or the initial state
+template <int FM>
+__device__ __forceinline__ void record_state(StepMeta<FM>& M, Column<FM, Var, 2>& C) {
+  M.n_fronts = C.n;
+  M.id_ponded = (int16_t)C.ponded_water.id;
+  M.id_endvol = (int16_t)C.ending_volume.id;
+  for (int i = 0; i < NGIUH; i++) M.id_giuh[i] = (int16_t)C.giuh[i].id;
+  for (int i = 0; i < C.n; i++)
+#pragma unroll
+    for (int k = 0; k < 5; k++) M.id_field[k * FM + i] = C.fid(k, i);
+}
+
+// zero the adjoints of the leaves and of the ne entries of a tape, then seed lambda (the adjoint of the state the tape
+// ends in) into the ids recorded for that state
+template <int FM>
+__device__ __forceinline__ void seed_state(double* adj, const double* lam, const StepMeta<FM>& M, int ne) {
+  for (int q = 0; q < num_leaves<FM>() + ne; q++) adj[(size_t)q * 32] = 0.0;
+  for (int i = 0; i < M.n_fronts; i++)
+#pragma unroll
+    for (int k = 0; k < 5; k++) {
+      const int id = M.id_field[k * FM + i];
+      if (id >= 0) adj[(size_t)id * 32] += __ldcg(lam + (size_t)(leaf_fields<FM>() + k * FM + i) * 32);
+    }
+  if (M.id_ponded >= 0) adj[(size_t)M.id_ponded * 32] += __ldcg(lam + (size_t)leaf_ponded<FM>() * 32);
+  if (M.id_endvol >= 0) adj[(size_t)M.id_endvol * 32] += __ldcg(lam + (size_t)leaf_endvol<FM>() * 32);
+  for (int i = 0; i < NGIUH; i++)
+    if (M.id_giuh[i] >= 0) adj[(size_t)M.id_giuh[i] * 32] += __ldcg(lam + (size_t)(leaf_giuh<FM>() + i) * 32);
+}
+
+// sweep the ne entries of a tape backwards.  The tape comes back from DRAM (the arenas of all resident warps are far
+// larger than L2): fetch eight entries at a time, independently of the adjoints, so that the misses overlap instead of
+// queueing behind the dependent chain adj -> entry -> adj.  Out of line so that the sub-step sweep and the initial-state
+// sweep share one copy of the unrolled loop; its arguments are scalars, so the call adds no stack traffic.
+template <int FM>
+__device__ __noinline__ void sweep_tape(double* adj, const TapeEntry* tape, int ne) {
+  for (int e0 = ne - 1; e0 >= 0; e0 -= 8) {
+    TapeEntry te8[8];
+#pragma unroll
+    for (int k = 0; k < 8; k++)
+      if (e0 - k >= 0) te8[k] = tape[(size_t)(e0 - k) * 32];
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+      const int e = e0 - k;
+      if (e >= 0) {
+        const double g = adj[(size_t)(num_leaves<FM>() + e) * 32];
+        if (g != 0.0) {
+          const TapeEntry te = te8[k];
+          if (te.a >= 0) adj[(size_t)te.a * 32] += g * te.da;
+          if (te.b >= 0) adj[(size_t)te.b * 32] += g * te.db;
+        }
+      }
+    }
+  }
+}
+
 // GM = 0: trapezoid Geff only (closed-form branch compiled out of the taped sub-step); GM = 2: run-time switch
 template <int FM, int GM>
 __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel(const BParams P) {
@@ -183,7 +248,6 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
     const bool valid = (size_t)slot_c < B;
     const int slot_cc = valid ? slot_c : (int)B - 1;
     const int b = p.column_order ? __ldg(p.column_order + slot_cc) : slot_cc;
-    const int bb = b;
     double* lam = P.lam + (size_t)tile * NL * 32 + lane;
     double* gsave = P.gpar + (size_t)tile * NPAR_IDS * 32 + lane;
 
@@ -192,7 +256,7 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
     const int final_crash = __ldcg(K.state_i + ((size_t)K.nchunks * NI_STATE + 3) * K.Bp + slot_cc);
     const int t_end = (final_st == 0) ? Tn : final_crash;  // steps [0, t_end) produced outputs
 
-    load_params(K, bb, Tv);
+    load_params(K, b, Tv);
     for (int l = 0; l < C.L; l++) {
       C.soil[l].id_alpha = 3 * l;
       C.soil[l].id_n = 3 * l + 1;
@@ -248,12 +312,8 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
           tc.base = arena + (size_t)arena_used * 32;
           tc.n = 0;
           tc.cap = min(P.step_cap, P.arena_cap - arena_used);
-          // derived parameters on the tape: m = 1 - 1/n (data/utils.py:75), psi_wp (aet.py:37-43)
-          for (int l = 0; l < C.L; l++) {
-            SoilT<Var>& sl = C.soil[l];
-            Var mV = 1.0 - (1.0 / Var(sl.n, sl.id_n));
-            sl.id_m = mV.id;
-          }
+          // derived parameters on the tape: m, psi_wp (aet.py:37-43)
+          tape_m(C);
           if (x.y > 0.0) precompute_psi_wp(Tv, p.wilting_point_psi);
 #pragma unroll
           for (int k = 0; k < NOUT; k++) Tv.acc[k] = Var(0.0);
@@ -268,16 +328,10 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
           }
           StepMeta<FM>& M = metas[(size_t)j * 32];
           M.n_entries = ne;
-          M.n_fronts = C.n;
           M.alive = (int16_t)(alive && Tv.ctx.st == 0 && !overflow);
-          M.id_ponded = (int16_t)C.ponded_water.id;
-          M.id_endvol = (int16_t)C.ending_volume.id;
-          for (int i = 0; i < NGIUH; i++) M.id_giuh[i] = (int16_t)C.giuh[i].id;
 #pragma unroll
           for (int k = 0; k < NOUT; k++) M.id_acc[k] = (int16_t)Tv.acc[k].id;
-          for (int i = 0; i < C.n; i++)
-#pragma unroll
-            for (int k = 0; k < 5; k++) M.id_field[k * FM + i] = C.fid(k, i);
+          record_state(M, C);
           arena_used += ne;
         }
       }
@@ -292,26 +346,14 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
           const int ne = M.n_entries;
           arena_used -= ne;
           if (!M.alive) continue;
-          const TapeEntry* tape = arena + (size_t)arena_used * 32;
-          for (int q = 0; q < NL + ne; q++) adj[(size_t)q * 32] = 0.0;
-          for (int i = 0; i < M.n_fronts; i++)
-#pragma unroll
-            for (int k = 0; k < 5; k++) {
-              const int id = M.id_field[k * FM + i];
-              if (id >= 0) adj[(size_t)id * 32] += __ldcg(lam + (size_t)(leaf_fields<FM>() + k * FM + i) * 32);
-            }
-          if (M.id_ponded >= 0) adj[(size_t)M.id_ponded * 32] += __ldcg(lam + (size_t)leaf_ponded<FM>() * 32);
-          if (M.id_endvol >= 0) adj[(size_t)M.id_endvol * 32] += __ldcg(lam + (size_t)leaf_endvol<FM>() * 32);
-          for (int i = 0; i < NGIUH; i++)
-            if (M.id_giuh[i] >= 0) adj[(size_t)M.id_giuh[i] * 32] += __ldcg(lam + (size_t)(leaf_giuh<FM>() + i) * 32);
+          seed_state(adj, lam, M, ne);
           // dL / d(outputs of this forcing step)
 #pragma unroll
           for (int k = 0; k < NOUT; k++) {
             double g = 0.0;
-            const bool state_out = (k == LGAR_OUT_ENDING_VOLUME || k == LGAR_OUT_PONDED_WATER);
             if (P.grad_per_step && (P.grad_mask & (1u << k)))
               g += __ldg(P.grad_per_step + ((size_t)__popc(P.grad_mask & ((1u << k) - 1u)) * Tn + t) * B + b);
-            if (P.grad_sums && (!state_out || t == Tn - 1)) g += __ldg(P.grad_sums + (size_t)k * B + b);
+            if (P.grad_sums && (!is_state_output(k) || t == Tn - 1)) g += __ldg(P.grad_sums + (size_t)k * B + b);
             if (g == 0.0) continue;
             int id = -1;
             if (k == LGAR_OUT_ENDING_VOLUME) id = (sc == S - 1) ? M.id_endvol : -1;
@@ -327,27 +369,7 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
             if (P.grad_layer_water)
               for (int l = 0; l < p.num_layers; l++, a += 32) *a += __ldg(P.grad_layer_water + ((size_t)l * Tn + t) * B + b);
           }
-          // the tape comes back from DRAM (the arenas of all resident warps are far larger than L2): fetch eight
-          // entries at a time, independently of the adjoints, so that the misses overlap instead of queueing behind
-          // the dependent chain adj -> entry -> adj
-          for (int e0 = ne - 1; e0 >= 0; e0 -= 8) {
-            TapeEntry te8[8];
-#pragma unroll
-            for (int k = 0; k < 8; k++)
-              if (e0 - k >= 0) te8[k] = tape[(size_t)(e0 - k) * 32];
-#pragma unroll
-            for (int k = 0; k < 8; k++) {
-              const int e = e0 - k;
-              if (e >= 0) {
-                const double g = adj[(size_t)(NL + e) * 32];
-                if (g != 0.0) {
-                  const TapeEntry te = te8[k];
-                  if (te.a >= 0) adj[(size_t)te.a * 32] += g * te.da;
-                  if (te.b >= 0) adj[(size_t)te.b * 32] += g * te.db;
-                }
-              }
-            }
-          }
+          sweep_tape<FM>(adj, arena + (size_t)arena_used * 32, ne);
           for (int q = NPAR_IDS; q < NL; q++) __stcg(lam + (size_t)q * 32, adj[(size_t)q * 32]);
 #pragma unroll
           for (int q = 0; q < NPAR_IDS; q++) gpar[q] += adj[(size_t)q * 32];
@@ -361,64 +383,46 @@ __global__ void __launch_bounds__(NT, BACKWARD_CTAS_PER_SM) lgar_backward_kernel
 #pragma unroll
       for (int q = 0; q < NPAR_IDS; q++) gsave[(size_t)q * 32] = gpar[q];
       P.rev_flags[(size_t)tile * 32 + lane] = overflow ? 1 : 0;
-    }
-    // ---- the initial state depends on the parameters: theta_init = theta_l(psi_init), K_init
-    //      (data/utils.py:82-84, WettingFront.py:38-48); ending_volume(0) = mass_balance()
-    if (chunk == 0) {
+    } else {
+      // ---- the initial state depends on the parameters: theta_init = theta_l(psi_init), K_init
+      //      (data/utils.py:82-84, WettingFront.py:38-48); ending_volume(0) = mass_balance().  Its ids are recorded
+      //      in the first StepMeta of the ring, free again after the sweep above.
       tc.base = arena;
       tc.n = 0;
       tc.cap = min(P.step_cap, P.arena_cap);
       Tv.ctx.st = 0;
-      for (int l = 0; l < C.L; l++) {
-        SoilT<Var>& sl = C.soil[l];
-        Var mV = 1.0 - (1.0 / Var(sl.n, sl.id_n));
-        sl.id_m = mV.id;
-      }
-      init_column(Tv, __ldg(p.initial_psi + bb), p.use_closed_form_G != 0);
+      tape_m(C);
+      init_column(Tv, __ldg(p.initial_psi + b), p.use_closed_form_G != 0);
       const int ne = min(tc.n, tc.cap);
       if (valid && Tv.ctx.st == 0) {
-        for (int q = 0; q < NL + ne; q++) adj[(size_t)q * 32] = 0.0;
-        for (int i = 0; i < C.n; i++)
-#pragma unroll
-          for (int k = 0; k < 5; k++) {
-            const int id = C.fid(k, i);
-            if (id >= 0) adj[(size_t)id * 32] += __ldcg(lam + (size_t)(leaf_fields<FM>() + k * FM + i) * 32);
-          }
-        if (C.ending_volume.id >= 0) adj[(size_t)C.ending_volume.id * 32] += __ldcg(lam + (size_t)leaf_endvol<FM>() * 32);
-        for (int e = ne - 1; e >= 0; e--) {
-          const double g = adj[(size_t)(NL + e) * 32];
-          if (g != 0.0) {
-            const TapeEntry te = arena[(size_t)e * 32];
-            if (te.a >= 0) adj[(size_t)te.a * 32] += g * te.da;
-            if (te.b >= 0) adj[(size_t)te.b * 32] += g * te.db;
-          }
-        }
+        StepMeta<FM>& M = metas[0];
+        record_state(M, C);
+        seed_state(adj, lam, M, ne);
+        sweep_tape<FM>(adj, arena, ne);
 #pragma unroll
         for (int q = 0; q < NPAR_IDS; q++) gpar[q] += adj[(size_t)q * 32];
       }
-    }
-    if (chunk > 0) {
-      // (nothing to write yet)
-    } else if (P.reduce) {
-      // shared parameters: sum over the 32 columns of the tile in a fixed (butterfly) order; overflowed and
-      // out-of-range lanes contribute 0
+      if (P.reduce) {
+        // shared parameters: sum over the 32 columns of the tile in a fixed (butterfly) order; overflowed and
+        // out-of-range lanes contribute 0
 #pragma unroll
-      for (int q = 0; q < NPAR_IDS; q++) {
-        double v = (valid && !overflow) ? gpar[q] : 0.0;
+        for (int q = 0; q < NPAR_IDS; q++) {
+          double v = (valid && !overflow) ? gpar[q] : 0.0;
 #pragma unroll
-        for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
-        if (lane == 0) P.partials[(size_t)tile * NPAR_IDS + q] = v;
+          for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+          if (lane == 0) P.partials[(size_t)tile * NPAR_IDS + q] = v;
+        }
+      } else if (valid) {
+        const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+        for (int l = 0; l < p.num_layers; l++) {
+          P.grad_alpha[(size_t)l * B + b] = overflow ? qnan : gpar[3 * l];
+          P.grad_n[(size_t)l * B + b] = overflow ? qnan : gpar[3 * l + 1];
+          P.grad_ksat[(size_t)l * B + b] = overflow ? qnan : gpar[3 * l + 2];
+        }
+        if (P.grad_pdm) P.grad_pdm[b] = overflow ? qnan : gpar[ID_PDM];
       }
-    } else if (valid) {
-      const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-      for (int l = 0; l < p.num_layers; l++) {
-        P.grad_alpha[(size_t)l * B + b] = overflow ? qnan : gpar[3 * l];
-        P.grad_n[(size_t)l * B + b] = overflow ? qnan : gpar[3 * l + 1];
-        P.grad_ksat[(size_t)l * B + b] = overflow ? qnan : gpar[3 * l + 2];
-      }
-      if (P.grad_pdm) P.grad_pdm[b] = overflow ? qnan : gpar[ID_PDM];
+      if (valid && P.tape_overflow) P.tape_overflow[b] = overflow ? 1 : 0;
     }
-    if (chunk == 0 && valid && P.tape_overflow) P.tape_overflow[b] = overflow ? 1 : 0;
     if (P.counters) {
       if (lane == 0) {
         atomicAdd(P.counters + 0, cyc_fwd);

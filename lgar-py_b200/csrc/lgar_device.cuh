@@ -287,6 +287,12 @@ __device__ __forceinline__ double2 h_from_se_x2(double se0, double se1, const So
 }
 
 __device__ __forceinline__ double shfl_d(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
+// maximum of v over the warp (butterfly); warp-convergent
+__device__ __forceinline__ int warp_max(int v) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) v = max(v, __shfl_xor_sync(0xffffffffu, v, d));
+  return v;
+}
 
 // torch.min / torch.minimum semantics (NaN propagates, unlike fmin)
 __device__ __forceinline__ double tmin(double a, double b) {
@@ -645,6 +651,30 @@ __device__ __forceinline__ Soil gather_soil(const ST* soil, int L, int owner, in
   return q;
 }
 
+// The start of one request, common to both batch evaluators: Se and h at both ends, the node spacing dh, K at node 0
+// and the status raised so far
+struct GeffStart {
+  double se_i, se_f, h_i, h_f, dh, k1;
+  int st;
+};
+__device__ __forceinline__ GeffStart geff_start(double theta_1, double theta_2, const Soil& s, int nint) {
+  Ctx c;
+  c.st = 0;
+  GeffStart g;
+  g.se_i = se_from_theta(theta_1, s, c);
+  g.se_f = se_from_theta(theta_2, s, c);
+  const double2 hh = h_from_se_x2(g.se_i, g.se_f, s, c);
+  g.h_i = hh.x;
+  g.h_f = hh.y;
+  // "Checkpoint" calls green_ampt.py:61-63: results unused, only their guards can matter
+  if (fabs(g.h_i) >= 0.1 && s.alpha * g.h_i < 0.0) raise(c, LGAR_ST_NEG_POW);
+  if (fabs(g.h_f) >= 0.1 && s.alpha * g.h_f < 0.0) raise(c, LGAR_ST_NEG_POW);
+  g.dh = (g.h_f - g.h_i) / (double)nint;
+  g.k1 = k_from_se(g.se_i, s.ksat, s.m, s.inv_m, c);
+  g.st = c.st;
+  return g;
+}
+
 // Forward (values only).  Every lane of the warp calls it; lane s evaluates slot s.
 template <class ST>
 __device__ __noinline__ void geff_batch_eval(GeffQueue* q, const ST* soil, int L, int nint) {
@@ -653,22 +683,13 @@ __device__ __noinline__ void geff_batch_eval(GeffQueue* q, const ST* soil, int L
   const bool have = meta >= 0;
   const Soil s = gather_soil(soil, L, have ? (meta & 31) : lane, have ? ((meta >> 8) & 7) : 0);
   if (have) {
-    Ctx c;
-    c.st = 0;
-    const double theta_1 = q->a[lane], theta_2 = q->b[lane];
-    const double se_i = se_from_theta(theta_1, s, c);
-    const double se_f = se_from_theta(theta_2, s, c);
-    const double2 hh = h_from_se_x2(se_i, se_f, s, c);
-    const double h_i = hh.x, h_f = hh.y;
-    // "Checkpoint" calls green_ampt.py:61-63: results unused, only their guards can matter
-    if (fabs(h_i) >= 0.1 && s.alpha * h_i < 0.0) raise(c, LGAR_ST_NEG_POW);
-    if (fabs(h_f) >= 0.1 && s.alpha * h_f < 0.0) raise(c, LGAR_ST_NEG_POW);
-    const double dh = (h_f - h_i) / (double)nint;
-    double k1 = k_from_se(se_i, s.ksat, s.m, s.inv_m, c);
+    const GeffStart g0 = geff_start(q->a[lane], q->b[lane], s, nint);
+    const double dh = g0.dh;
+    double k1 = g0.k1;
     const double half = dh / 2.0;
     double geff = 0.0;
-    double h2 = h_i + dh;
-    int st = c.st;
+    double h2 = g0.h_i + dh;
+    int st = g0.st;
     // two nodes per pass through the SAME out-of-line pair evaluator as everything else (k_nodes_core_x2 -> pow_x2):
     // the kernel is instruction-fetch sensitive (DESIGN.md), so the hot loops share one small body of pow code
 #pragma unroll 1
@@ -785,21 +806,13 @@ __device__ __noinline__ void geff_batch_eval_taped(GeffQueue* q, const ST* soil,
   const bool have = meta >= 0;
   const Soil s = gather_soil(soil, L, have ? (meta & 31) : lane, have ? ((meta >> 8) & 7) : 0);
   if (have) {
-    Ctx c;
-    c.st = 0;
-    const double theta_1 = q->a[lane], theta_2 = q->b[lane];
-    const double se_i = se_from_theta(theta_1, s, c);
-    const double se_f = se_from_theta(theta_2, s, c);
-    const double2 hh = h_from_se_x2(se_i, se_f, s, c);
-    const double h_i = hh.x, h_f = hh.y;
-    if (fabs(h_i) >= 0.1 && s.alpha * h_i < 0.0) raise(c, LGAR_ST_NEG_POW);
-    if (fabs(h_f) >= 0.1 && s.alpha * h_f < 0.0) raise(c, LGAR_ST_NEG_POW);
-    const double dh = (h_f - h_i) / (double)nint;
-    double k1 = k_from_se(se_i, s.ksat, s.m, s.inv_m, c);
-    const P4 pi = h_se_partials_core(se_i, s.alpha, s.ninv_m, s.inv_m, s.inv_n, h_i);
-    const P4 pf = h_se_partials_core(se_f, s.alpha, s.ninv_m, s.inv_m, s.inv_n, h_f);
-    const NodeFull n0 = k_node_full(h_i, true, se_i, s.alpha, s.n, s.m, s.inv_m, s.ksat);
-    int st = c.st;
+    const GeffStart g0 = geff_start(q->a[lane], q->b[lane], s, nint);
+    const double h_i = g0.h_i, dh = g0.dh;
+    double k1 = g0.k1;
+    const P4 pi = h_se_partials_core(g0.se_i, s.alpha, s.ninv_m, s.inv_m, s.inv_n, h_i);
+    const P4 pf = h_se_partials_core(g0.se_f, s.alpha, s.ninv_m, s.inv_m, s.inv_n, g0.h_f);
+    const NodeFull n0 = k_node_full(h_i, true, g0.se_i, s.alpha, s.n, s.m, s.inv_m, s.ksat);
+    int st = g0.st;
     if (st == 0 && n0.bad) st = n0.bad;
     double S = 0.5 * k1, Csei = 0.5 * n0.dk_se, Ahi = 0.0, Ahf = 0.0, Ca = 0.0, Cn = 0.0, Cm = 0.5 * n0.dk_m;
     const double half = dh / 2.0;
@@ -854,25 +867,24 @@ __device__ __forceinline__ void geffq_put(GeffQueue* q, int slot, int owner, int
   q->b[slot] = t2;
   q->meta[slot] = owner | (layer << 8);
 }
-// result of slot `slot`, owned by this lane (value + status; the taped pass records one entry with five partials)
-__device__ __forceinline__ double geffq_get(GeffQueue* q, int slot, double /*t1*/, double /*t2*/, const SoilT<double>&, int nint,
-                                            Ctx& c) {
+// result of slot `slot`, owned by this lane (value + status; the taped pass records one entry with five partials).
+// geffq_take counts the request's work and raises its status.
+__device__ __forceinline__ void geffq_take(const GeffQueue* q, int slot, int nint, Ctx& c) {
   c.cnt[C_GEFF]++;
   c.cnt[C_H_SE] += 2;
   c.cnt[C_K_SE] += 1 + nint;
   c.cnt[C_SE_H] += nint;
   const int st = q->st[slot];
   if (st) raise(c, st);
+}
+__device__ __forceinline__ double geffq_get(GeffQueue* q, int slot, double /*t1*/, double /*t2*/, const SoilT<double>&, int nint,
+                                            Ctx& c) {
+  geffq_take(q, slot, nint, c);
   return q->a[slot];
 }
 __device__ __forceinline__ Var geffq_get(GeffQueue* q, int slot, const Var& t1, const Var& t2, const SoilT<Var>& s, int nint,
                                          Ctx& c) {
-  c.cnt[C_GEFF]++;
-  c.cnt[C_H_SE] += 2;
-  c.cnt[C_K_SE] += 1 + nint;
-  c.cnt[C_SE_H] += nint;
-  const int st = q->st[slot];
-  if (st) raise(c, st);
+  geffq_take(q, slot, nint, c);
   const int ids[5] = {t1.id, t2.id, s.id_alpha, s.id_n, s.id_m};
   const double* dq = g_geffq_partials[threadIdx.x >> 5] + slot;
   const double d[5] = {dq[0 * 32], dq[1 * 32], dq[2 * 32], dq[3 * 32], dq[4 * 32]};
@@ -1062,11 +1074,16 @@ struct Column {
       if (nf == 0) empty_list = true;  // wetting_fronts[0] of an empty list: IndexError in the reference
       o += nf;
     }
-    Q tot = s_l[L - 1];
-    for (int l = L - 2; l >= 0; l--) tot = s_l[l] + tot;
-    return tot;
+    return layer_sum(s_l);
   }
   __device__ __forceinline__ R mass_balance() { return mass_balance_t<R>(); }
+  // sum of per-layer terms in the reference's association x[0] + (x[1] + (... + x[L-1]))
+  template <class Q>
+  __device__ __forceinline__ Q layer_sum(const Q* x) const {
+    Q tot = x[L - 1];
+    for (int l = L - 2; l >= 0; l--) tot = x[l] + tot;
+    return tot;
+  }
 
   // ---- soil-moisture output theta(z) (lgar_b200.h): flat index of the first front of the list of the layer holding
   //      depth z (cum[l-1] < z <= cum[l]) whose depth >= z; -1 if z lies below the column or no front qualifies.
@@ -1226,9 +1243,7 @@ struct Column {
     const unsigned FULL = 0xffffffffu;
     go = go && (c.st == 0);
     const int num_wf = go ? n : 0;
-    int rmax = num_wf;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) rmax = max(rmax, __shfl_xor_sync(FULL, rmax, d));
+    const int rmax = warp_max(num_wf);
     R old_theta_below(0.0), old_psi_below(0.0);  // previous_state of front i+1
     int l = L - 1;
     int o = go ? n - cnt(L - 1) : 0;  // flat offset of list l
@@ -1331,9 +1346,7 @@ struct Column {
       }
       // ---- P1: sums over the layers above (convergent, values only)
       double dth[MAXL - 1], dtk[MAXL - 1];
-      int nupmax = nup;
-#pragma unroll
-      for (int d = 16; d > 0; d >>= 1) nupmax = max(nupmax, __shfl_xor_sync(FULL, nupmax, d));
+      const int nupmax = warp_max(nup);
 #pragma unroll
       for (int k = 0; k < MAXL - 1; k++) {
         dth[k] = 0.0;
@@ -1763,9 +1776,7 @@ struct Column {
       }
       o += cnt(l);
     }
-    R tot = fl[L - 1];
-    for (int l = L - 2; l >= 0; l--) tot = fl[l] + tot;
-    return tot;
+    return layer_sum(fl);
   }
 
   // ---- Layer.fix_dry_over_wet_fronts (Layer.py:1055-1143): one fix per layer list per call
@@ -1793,9 +1804,7 @@ struct Column {
       }
       o += cnt(l);
     }
-    R tot = mc[L - 1];
-    for (int l = L - 2; l >= 0; l--) tot = mc[l] + tot;
-    return tot;
+    return layer_sum(mc);
   }
   // cleanup_wetting_fronts (:1098-1115): the search is by VALUE from the top of the column
   __device__ void cleanup_wetting_fronts(int nx, Ctx& c) {
@@ -1835,9 +1844,7 @@ struct Column {
   __device__ void update_psi_warp(bool go, Ctx& c) {
     go = go && (c.st == 0);
     const int my_n = go ? n - 1 : 0;
-    int nmax = my_n;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) nmax = max(nmax, __shfl_xor_sync(0xffffffffu, nmax, d));
+    const int nmax = warp_max(my_n);
     int l = 0, o_next = go ? cnt(0) : 0;
     for (int i = 0; i < nmax; i++) {
       if (i < my_n) {

@@ -26,6 +26,9 @@ enum StateSlot {
 // int state: n, cntpk, status, crash_step
 constexpr int NI_STATE = 4;
 
+// outputs that are states, not fluxes: a step's value is the END state of the step and their "sum" is the last value
+__host__ __device__ constexpr bool is_state_output(int k) { return k == LGAR_OUT_ENDING_VOLUME || k == LGAR_OUT_PONDED_WATER; }
+
 template <int FM>
 __host__ __device__ constexpr int state_doubles() { return 5 * FM + S_COUNT; }
 
@@ -301,8 +304,10 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
   if (timed) { const long long t = clock64(); c.ph[2] += (unsigned long long)(t - tph); tph = t; }
   // ---- phase 4: Layer.calc_dzdt (Layer.py:1176-1252): one Geff per moving front of every column.  All requests of
   //      the tile are known here, so they go through the per-warp queue in batches of 32, one lane per request
-  //      (geff_batch_eval); each lane then finishes dzdt of its own fronts in front order.
-  if (!(GM == 2 && nint < 0)) {
+  //      (geff_batch_eval); each lane then finishes dzdt of its own fronts in front order.  With the closed-form Geff
+  //      (nint < 0) the queue is not used: the owner lane evaluates each of its requests itself (geff_closedR).
+  {
+    const bool closed = GM == 2 && nint < 0;
     const unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31;
     const bool go = act && c.st == 0;
@@ -342,9 +347,9 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
     int rem = nreq;
     for (int lo = 0; lo < total;) {
       const int hi = lo + 32;
-      gq->meta[lane] = -1;
-      __syncwarp();
-      {
+      if (!closed) {
+        gq->meta[lane] = -1;
+        __syncwarp();
         int i = cur, gg = g, r_ = rem;
         while (r_ > 0 && gg < hi) {
           if (!C.tb(i)) {
@@ -354,9 +359,9 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
           }
           i++;
         }
+        __syncwarp();
+        geffq_eval(gq, C.soil, K.p.num_layers, nint);
       }
-      __syncwarp();
-      geffq_eval(gq, C.soil, K.p.num_layers, nint);
       while (rem > 0 && g < hi) {
         const int i = cur++;
         if (C.tb(i)) continue;
@@ -367,7 +372,7 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
         const int l = C.list_layer(i);
         const R theta_1 = C.g(F_THETA, i + 1), theta_2 = C.g(F_THETA, i);
         const SoilT<R>& s = C.soil[l];
-        const R geff = geffq_get(gq, slot, theta_1, theta_2, s, nint, c);
+        const R geff = closed ? geff_closedR(true, theta_1, theta_2, s, c) : geffq_get(gq, slot, theta_1, theta_2, s, nint, c);
         if (c.st != 0) continue;
         const R depth = C.g(F_DEPTH, i);
         const R delta_theta = theta_2 - theta_1;
@@ -387,53 +392,6 @@ __device__ void substep(Tile<FM, R, LM>& T, bool act, double precip_rate, double
       lo = hi;
     }
     if (go && c.st == 0 && pre_err) raise(c, pre_err);
-  } else {  // closed-form Geff (geff_closedR): per lane, no queue; each lane takes its own fronts in front order
-    const bool go = act && c.st == 0;
-    const int my_n = go ? C.n - 1 : 0;  // the deepest front of the domain is excluded
-    int nmax = my_n;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) nmax = max(nmax, __shfl_xor_sync(0xffffffffu, nmax, d));
-    int l = 0, o_next = go ? C.cnt(0) : 0;  // list layer of flat index i
-    for (int i = 0; i < nmax; i++) {
-      bool needG = false;
-      R theta_1(0.0), theta_2(0.0), bottom_sum(0.0);
-      const bool mine = go && (i < my_n) && (c.st == 0);
-      if (mine) {
-        while (i >= o_next) {
-          l++;
-          o_next += C.cnt(l);
-        }
-        theta_1 = C.g(F_THETA, i + 1);
-        theta_2 = C.g(F_THETA, i);
-        if (C.tb(i)) {
-          C.s(F_DZDT, i, R(0.0));
-        } else {
-          if (C.lay(i) > 0) {
-            if (l == 0) raise(c, LGAR_ST_NULL_NEIGHBOUR);  // self.previous_layer is None
-            else bottom_sum = 0.0 + (C.g(F_DEPTH, i) - C.cum[l - 1]) / C.g(F_K, i);
-          } else if (theta_1 > theta_2) {
-            raise(c, LGAR_ST_THETA_ORDER);
-          }
-          needG = (c.st == 0);
-        }
-      }
-      const R geff = geff_closedR(needG, theta_1, theta_2, C.soil[needG ? l : 0], c);
-      if (needG && c.st == 0) {
-        const SoilT<R>& s = C.soil[l];
-        const R depth = C.g(F_DEPTH, i);
-        const R delta_theta = theta_2 - theta_1;
-        R dzdt(0.0);
-        if (C.lay(i) == 0) {
-          if (delta_theta > 0.0)
-            dzdt = 1.0 / delta_theta * (s.ksatR() * (geff + ponded_depth_sub) / depth + C.g(F_K, i));
-        } else {
-          const R denominator = C.calc_bottom_sum(0, bottom_sum, C.g(F_PSI, i), C.lay(i), c);
-          if (delta_theta > 0.0)
-            dzdt = (1.0 / delta_theta) * ((depth / denominator) + s.ksatR() * (geff + ponded_depth_sub) / depth);
-        }
-        C.s(F_DZDT, i, dzdt);
-      }
-    }
   }
 
   if (timed) { const long long t = clock64(); c.ph[3] += (unsigned long long)(t - tph); tph = t; }
@@ -675,7 +633,6 @@ __global__ void __launch_bounds__(NT, (FM == 32) ? 1 : ((FM == 16) ? 2 : ((FM ==
     const bool valid = (size_t)slot_c < B;
     const int slot_cc = valid ? slot_c : (int)B - 1;  // clamp for loads; results of invalid lanes are never stored
     const int b = p.column_order ? __ldg(p.column_order + slot_cc) : slot_cc;
-    const int bb = b;
 
     // wait for the previous chunk of this tile (acquire): done[tile] = forcing rows completed (absolute row index)
     const int t0 = K.t_begin + chunk * K.chunk_steps;
@@ -698,7 +655,7 @@ __global__ void __launch_bounds__(NT, (FM == 32) ? 1 : ((FM == 16) ? 2 : ((FM ==
 #pragma unroll
     for (int k = 0; k < 3; k++) T.ctx.br[k] = 0;
     const long long clk0 = clock64();
-    load_params(K, bb, T);
+    load_params(K, b, T);
     const int slot_in = K.keep_ckpt ? chunk : 0;
     if (chunk == 0 && p.resume) {
       load_state(K, 0, slot_cc, T);  // continue from the state the previous launch left in the workspace
@@ -706,7 +663,7 @@ __global__ void __launch_bounds__(NT, (FM == 32) ? 1 : ((FM == 16) ? 2 : ((FM ==
     } else if (chunk == 0) {
       T.ctx.st = 0;
       T.crash_step = -1;
-      init_column(T, __ldg(p.initial_psi + bb), p.use_closed_form_G != 0);
+      init_column(T, __ldg(p.initial_psi + b), p.use_closed_form_G != 0);
       if (T.ctx.st) T.crash_step = 0;
       if (valid && K.o.start_volume) K.o.start_volume[b] = T.col.ending_volume;
       if (K.keep_ckpt && valid) save_state(K, 0, slot_c, T);
@@ -761,7 +718,7 @@ __global__ void __launch_bounds__(NT, (FM == 32) ? 1 : ((FM == 16) ? 2 : ((FM ==
         if (ok) {
 #pragma unroll
           for (int k = 0; k < NOUT; k++)
-            T.sums[k] = (k == LGAR_OUT_ENDING_VOLUME || k == LGAR_OUT_PONDED_WATER) ? T.acc[k] : T.sums[k] + T.acc[k];
+            T.sums[k] = is_state_output(k) ? T.acc[k] : T.sums[k] + T.acc[k];
         }
         if (K.o.num_fronts) K.o.num_fronts[(size_t)t * B + b] = ok ? T.col.n : 0;
         if (K.o.moisture || K.o.layer_water) store_soil_moisture(K, T.col, ok, t, b);
