@@ -20,6 +20,21 @@ OUT_NAMES = ("runoff", "percolation", "AET", "infiltration", "ending_volume", "p
              "giuh_runoff", "precip", "PET", "discharge")
 STATUS_NAMES = ("OK", "NEG_POW", "NAN", "THETA_ORDER", "BOTTOM_REACHED", "NULL_NEIGHBOUR",
                 "FRONT_OVERFLOW", "ITER_CAP", "INDEX_ERROR")
+FRONT_OVERFLOW = STATUS_NAMES.index("FRONT_OVERFLOW")
+# statuses that are capacity limits of this library rather than states in which the reference raises (its front lists
+# are unbounded and its root finders have no iteration cap)
+CAPACITY_STATUSES = (FRONT_OVERFLOW, STATUS_NAMES.index("ITER_CAP"))
+
+
+def status_message(column, status: int, step=None) -> str:
+    """Report of a column that ended with a non-zero status (and, if known, the forcing step it crashed at)."""
+    at = "" if step is None else f" at forcing step {step}"
+    msg = f"LGAR column {column}: status {STATUS_NAMES[status]}{at}"
+    if status in CAPACITY_STATUSES:
+        return (msg + ": a capacity limit of the CUDA library (16 wetting fronts per column in the differentiable path "
+                "/ 1e6 root-finder iterations), not a reference exception; mask the column (the agent's "
+                "on_column_error='mask') or rerun it forward-only with max_fronts=32")
+    return msg + " (the reference raises here)"
 EXPORTS = ("lgar_abi_version", "lgar_device_check", "lgar_last_error_string", "lgar_workspace_bytes",
            "lgar_forward", "lgar_backward", "lgar_backward_ex", "lgar_forward_host", "lgar_measure_fp64_flops")
 

@@ -27,16 +27,11 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
+from . import parallel
+from ._capi import OUT_NAMES, status_message
+from .model import _get
+
 log = logging.getLogger("agents.DifferentiableLGAR")
-
-
-def _get(cfg, path, default=None):
-    cur = cfg
-    for key in path.split("."):
-        if cur is None:
-            return default
-        cur = cur.get(key) if isinstance(cur, dict) else getattr(cur, key, None)
-    return default if cur is None else cur
 
 
 def _set(cfg, path, value):
@@ -135,8 +130,7 @@ class DifferentiableLGAR:
     (read from cfg.data.forcing_file when None); `y`: observations `[T]` / `[sites, T]` (the reference's seeded
     random series when None)."""
 
-    OUTPUTS = ("runoff", "percolation", "AET", "infiltration", "ending_volume", "ponded_water", "giuh_runoff", "precip",
-               "PET", "discharge")
+    OUTPUTS = OUT_NAMES
 
     def __init__(self, cfg, model=None, x=None, y=None, device="cuda", group=None, on_column_error="raise") -> None:
         """on_column_error: "raise" (reference semantics: an exception inside model(x) aborts the run) or "mask"
@@ -201,16 +195,8 @@ class DifferentiableLGAR:
         failed = st is not None and bool((st != 0).any())
         msg = ""
         if failed:
-            from ._capi import STATUS_NAMES
-            from .model import CAPACITY_STATUSES
-            first = (st.reshape(-1) != 0).nonzero()[0, 0]
-            bad, step = int(st.reshape(-1)[first]), int(out["crash_step"].reshape(-1)[first])
-            if bad in CAPACITY_STATUSES:  # a limit of this library, not a reference state (its front lists are unbounded)
-                msg = (f"LGAR column status {STATUS_NAMES[bad]} at forcing step {step}: a capacity limit of the CUDA library "
-                       "(16 wetting fronts per column in the differentiable path / 1e6 root-finder iterations), not a "
-                       "reference exception; mask the site (on_column_error='mask') or rerun it forward-only with max_fronts=32")
-            else:
-                msg = f"LGAR column status {STATUS_NAMES[bad]} at forcing step {step} (the reference raises here)"
+            first = int((st.reshape(-1) != 0).nonzero()[0, 0])
+            msg = status_message(first, int(st.reshape(-1)[first]), int(out["crash_step"].reshape(-1)[first]))
         if self.on_column_error == "raise" and self._any_rank(failed):
             # every rank leaves together: a lone raise would leave the others waiting in the gradient all-reduce
             raise RuntimeError(msg or "LGAR column failure on another rank")
@@ -248,19 +234,16 @@ class DifferentiableLGAR:
         loss.backward()
         end = time.perf_counter()
         log.info(f"Back prop took : {(end - start):.6f} seconds")
-        loss_val = self._allreduce_mean(loss.detach())
-        log.info(f"Loss: {loss_val}")
-        # never step on a broken gradient: an exhausted tape arena (ColumnEnsemble.last_tape_overflow) or a non-finite
-        # entry would poison the parameters and Adam's moments for good
-        grads = [p.grad for p in self.model.parameters() if p.grad is not None]
-        finite = all(bool(torch.isfinite(g).all()) for g in grads)
         ens = getattr(self.model, "last_ensemble", None)
         overflowed = ens.check_tape_overflow(raise_error=False) if ens is not None else 0
-        if self._any_rank((not finite) or overflowed > 0):
-            self.optimizer.zero_grad()
-            raise RuntimeError(f"gradient not usable (finite: {finite}, columns with an exhausted tape arena: {overflowed}); "
-                               "the optimiser step was skipped")
-        self.optimizer.step()
+        # one collective: the loss and the gradients averaged over the ranks (each rank counts 1), and whether any
+        # rank's gradient is unusable
+        ps = list(self.model.parameters())
+        grads = [p.grad if p.grad is not None else torch.zeros_like(p) for p in ps]
+        loss_val, mean_grads, unusable = parallel.allreduce_loss_and_grads(loss.detach(), 1, grads, self.group,
+                                                                            overflowed > 0)
+        log.info(f"Loss: {loss_val}")
+        parallel.step_if_usable(ps, mean_grads, unusable, self.optimizer, overflowed)
         self.history.append((self.current_epoch, float(loss_val), nse))
 
     def save_checkpoint(self, file_name="checkpoint.pth.tar", is_best=0):
@@ -296,23 +279,6 @@ class DifferentiableLGAR:
         t = torch.tensor([1.0 if flag else 0.0], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX, group=self.group)
         return bool(t.item() > 0)
-
-    def _allreduce_mean(self, loss):
-        """Average the loss and the parameter gradients over the ranks with ONE collective (SURVEY 8e)."""
-        if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(self.group) == 1:
-            return loss
-        ps = [p for p in self.model.parameters()]
-        dev = loss.device
-        flat = torch.cat([loss.reshape(1).to(torch.float64)] +
-                         [(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1).to(dev, torch.float64)
-                          for p in ps])
-        dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=self.group)
-        flat = flat / dist.get_world_size(self.group)
-        o = 1
-        for p in ps:
-            p.grad = flat[o:o + p.numel()].reshape(p.shape).to(p.device, p.dtype)
-            o += p.numel()
-        return flat[0]
 
     def _report_mass(self, out):
         with torch.no_grad():

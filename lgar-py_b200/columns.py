@@ -14,6 +14,7 @@ arrive on the host, and the call fails loudly if the library or an sm_100 GPU is
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 import math
 from dataclasses import dataclass, field
 from typing import Optional, Sequence
@@ -21,7 +22,7 @@ from typing import Optional, Sequence
 import torch
 
 from . import _capi
-from ._capi import NUM_OUTPUTS, OUT_NAMES, MAX_FRONTS, MAX_DEPTHS
+from ._capi import NUM_OUTPUTS, OUT_NAMES, MAX_FRONTS, MAX_DEPTHS, FRONT_OVERFLOW
 
 F64 = torch.float64
 
@@ -146,13 +147,26 @@ class ColumnEnsemble:
         on the bench ensemble: a conductive top layer sends the fronts into the deeper layers, where every move is a
         mass-balance root find).  Sets `column_order` = columns sorted by (site, ksat[0]); results do not depend on
         the placement (tests/test_gpu_properties.py)."""
-        k0 = torch.as_tensor(ksat, dtype=F64)
-        k0 = (k0[0] if k0.dim() == 2 else k0[0].expand(self.num_columns)).to(self.device)
-        order = torch.argsort(k0, stable=True)
+        (k,), _ = _param_layout(self, ksat)
+        order = torch.argsort(k[0], stable=True)
         if self.site_index is not None:
             order = order[torch.argsort(self.site_index[order].to(torch.int64), stable=True)]
         self.column_order = order.to(torch.int32).contiguous()
         return self
+
+    def subset(self, idx, **changes) -> "ColumnEnsemble":
+        """The ensemble of columns `idx` (an index tensor on the device): per-column fields (`[L,B]` and `[B]`) are
+        indexed, the forcing is shared, the placement (`column_order`), `resume`, the results of the last backward pass
+        (`last_*`) and `_keep` are not carried, every other field is copied; `changes` replace fields."""
+        B, kw = self.num_columns, {}
+        for f in dataclasses.fields(self):
+            if f.name in ("column_order", "resume", "_keep") or f.name.startswith("last_"):
+                continue
+            v = getattr(self, f.name)
+            if isinstance(v, torch.Tensor) and f.name != "forcing" and v.shape[-1:] == (B,):
+                v = v[..., idx]
+            kw[f.name] = v
+        return ColumnEnsemble(**{**kw, **changes})
 
 
 def check_moisture_depths(depths) -> tuple:
@@ -175,6 +189,11 @@ def output_mask(names) -> int:
     return m
 
 
+def output_row(mask: int, k: int) -> int:
+    """Row of output k in `per_step` ([mask.bit_count(), T, B]: the selected outputs in increasing index)."""
+    return (mask & ((1 << k) - 1)).bit_count()
+
+
 @dataclass
 class ForwardResult:
     per_step: Optional[torch.Tensor]   # [popcount(mask),T,B]: selected outputs in increasing index
@@ -195,18 +214,23 @@ class ForwardResult:
 
     def __getitem__(self, name) -> torch.Tensor:
         k = OUT_NAMES.index(name)
-        assert self.per_step is not None and (self.mask >> k) & 1, f"output {name} was not requested"
-        return self.per_step[bin(self.mask & ((1 << k) - 1)).count("1")]
+        if self.per_step is None or not (self.mask >> k) & 1:
+            raise KeyError(f"output {name} was not requested")
+        return self.per_step[output_row(self.mask, k)]
 
 
-def _param(x, ens: ColumnEnsemble):
-    t = torch.as_tensor(x, dtype=F64)
-    if t.dim() == 1:  # one parameter set shared by all columns
-        t = t.unsqueeze(1).expand(ens.num_layers, ens.num_columns)
-    return t.to(ens.device, non_blocking=True).contiguous()
+def _param_layout(ens: ColumnEnsemble, *params):
+    """alpha, n, ksat (any array type) as the launch needs them: `[L,B]` float64 on the ensemble's device.  A `[L]`
+    parameter is shared by all columns and is expanded.  Returns (the tensors, whether all of them are `[L]`): only
+    then the gradient of a shared parameter is the sum over columns formed inside the library; otherwise autograd sums
+    the per-column gradients of the `[L]` ones."""
+    ts = [torch.as_tensor(x, dtype=F64).to(ens.device, non_blocking=True) for x in params]
+    LB = (ens.num_layers, ens.num_columns)
+    return [(t if t.dim() == 2 else t.unsqueeze(1)).expand(LB).contiguous() for t in ts], all(t.dim() == 1 for t in ts)
 
 
-FRONT_OVERFLOW = 6  # lgar_status: more than max_fronts wetting fronts (capacity of the library, not a reference state)
+# the fields of a ForwardResult with one entry per column, in the last dimension
+_PER_COLUMN_RESULTS = ("per_step", "sums", "start_volume", "status", "crash_step", "num_fronts", "moisture", "layer_water")
 
 
 def _rerun_overflowed(ens: ColumnEnsemble, alpha, n, ksat, res: "ForwardResult", outputs, per_step, moisture=False,
@@ -215,31 +239,15 @@ def _rerun_overflowed(ens: ColumnEnsemble, alpha, n, ksat, res: "ForwardResult",
     The (rare: ~0.07 % of the bench ensemble over a year) columns that overflow are run again with the 32-front
     instantiation (one CTA per SM) and their results scattered into `res`.  Returns the number of columns rerun."""
     idx = (res.status == FRONT_OVERFLOW).nonzero().flatten()
-    if idx.numel() == 0 or int(ens.max_fronts) >= 32 or ens.resume:
+    if idx.numel() == 0 or int(ens.max_fronts) >= 32:
         return 0
-    sub = ColumnEnsemble(
-        theta_r=ens.theta_r[:, idx], theta_e=ens.theta_e[:, idx], thickness=ens.thickness[:, idx], forcing=ens.forcing,
-        site_index=(ens.site_index[idx] if ens.site_index is not None else None), initial_psi=ens.initial_psi[idx],
-        ponded_depth_max=ens.ponded_depth_max[idx], subcycle_length_h=ens.subcycle_length_h,
-        num_subcycles=ens.num_subcycles, nint=ens.nint, wilting_point_psi=ens.wilting_point_psi,
-        frozen_factor=ens.frozen_factor, use_closed_form_G=ens.use_closed_form_G, giuh_ordinates=ens.giuh_ordinates,
-        max_fronts=32, chunk_steps=ens.chunk_steps, iter_cap=ens.iter_cap, moisture_depths=ens.moisture_depths,
-        device=ens.device)
-    r2, _ = forward_raw(sub, alpha[:, idx].contiguous(), n[:, idx].contiguous(), ksat[:, idx].contiguous(), outputs=outputs,
-                        per_step=per_step, num_fronts=res.num_fronts is not None, overflow_fallback=False,
-                        moisture=moisture, layer_water=layer_water)
-    if res.per_step is not None:
-        res.per_step[:, :, idx] = r2.per_step
-    if moisture:
-        res.moisture[:, :, idx] = r2.moisture
-    if layer_water:
-        res.layer_water[:, :, idx] = r2.layer_water
-    res.sums[:, idx] = r2.sums
-    res.start_volume[idx] = r2.start_volume
-    res.status[idx] = r2.status
-    res.crash_step[idx] = r2.crash_step
-    if res.num_fronts is not None:
-        res.num_fronts[:, idx] = r2.num_fronts
+    r2, _ = forward_raw(ens.subset(idx, max_fronts=32), alpha[:, idx], n[:, idx], ksat[:, idx], outputs=outputs,
+                        per_step=per_step, num_fronts=res.num_fronts is not None, moisture=moisture,
+                        layer_water=layer_water)
+    for name in _PER_COLUMN_RESULTS:
+        part = getattr(r2, name)
+        if part is not None:
+            getattr(res, name)[..., idx] = part
     return int(idx.numel())
 
 
@@ -250,7 +258,8 @@ def forward_raw(ens: ColumnEnsemble, alpha, n, ksat, outputs=("runoff", "percola
                 layer_water=False) -> tuple[ForwardResult, torch.Tensor]:
     """One persistent launch over all columns and all forcing steps (no autograd).
     overflow_fallback: rerun the columns that overflowed the front list with the 32-front kernel (synchronises:
-    the status array is inspected on the host).
+    the status array is inspected on the host).  The rerun starts from the initial state at row 0, so it needs a run
+    over the whole record: a `window` other than (0, T) or a resumed ensemble is a ValueError.
     window=(t0, t1): advance only forcing rows [t0, t1) of the record (lgar_problem.step_begin/step_end); t0 > 0
     continues from the state the previous call left in `workspace` (resume).  Rows of the per-step outputs and
     crash steps stay absolute, so `into=` (the ForwardResult of the previous window) lets consecutive windows fill
@@ -264,10 +273,13 @@ def forward_raw(ens: ColumnEnsemble, alpha, n, ksat, outputs=("runoff", "percola
     per_step."""
     L_ = _capi.lib()
     dev = ens.device
+    B, T = ens.num_columns, ens.num_steps
     if moisture and ens.num_depths == 0:
         raise ValueError("moisture=True needs ColumnEnsemble(moisture_depths=...)")
-    alpha, n, ksat = _param(alpha, ens), _param(n, ens), _param(ksat, ens)
-    B, T = ens.num_columns, ens.num_steps
+    if overflow_fallback and (ens.resume or (window is not None and tuple(int(t) for t in window) != (0, T))):
+        raise ValueError("overflow_fallback reruns columns over the whole record: it needs window=None or (0, T) "
+                         "and an ensemble that does not resume")
+    (alpha, n, ksat), _ = _param_layout(ens, alpha, n, ksat)
     if ponded_depth_max is not None:  # [B] override of ens.ponded_depth_max (e.g. a learnable one)
         ponded_depth_max = _dev_f64(ponded_depth_max, dev, (B,))
     p = ens.problem(alpha, n, ksat, ponded_depth_max)
@@ -288,7 +300,7 @@ def forward_raw(ens: ColumnEnsemble, alpha, n, ksat, outputs=("runoff", "percola
         res = into
     else:
         res = ForwardResult(
-            per_step=torch.empty((bin(mask).count("1"), T, B), dtype=F64, device=dev) if mask else None, mask=mask,
+            per_step=torch.empty((mask.bit_count(), T, B), dtype=F64, device=dev) if mask else None, mask=mask,
             sums=torch.empty((NUM_OUTPUTS, B), dtype=F64, device=dev),
             start_volume=torch.empty(B, dtype=F64, device=dev),
             status=torch.empty(B, dtype=torch.int32, device=dev),
@@ -346,20 +358,15 @@ class _LGARFunction(torch.autograd.Function):
                 layer_water: bool = False):
         outputs = [OUT_NAMES[k] for k in range(NUM_OUTPUTS) if (mask >> k) & 1]
         need_grad = any(ctx.needs_input_grad[:4])
-        B = ens.num_columns
-        pdm_b = None
-        if pdm is not None:
-            pdm_b = pdm.detach().to(ens.device, F64)
-            pdm_b = (pdm_b.reshape(1).expand(B) if pdm_b.numel() == 1 else pdm_b.reshape(B)).contiguous()
-        res, ws = forward_raw(ens, alpha.detach(), n.detach(), ksat.detach(), outputs=outputs,
-                              keep_checkpoints=need_grad, ponded_depth_max=pdm_b, moisture=moisture,
-                              layer_water=layer_water)
+        (a, n_, k), ctx.params_shared = _param_layout(ens, alpha.detach(), n.detach(), ksat.detach())
+        pdm_b = None if pdm is None else _dev_f64(pdm.detach(), ens.device, (ens.num_columns,))
+        res, ws = forward_raw(ens, a, n_, k, outputs=outputs, keep_checkpoints=need_grad, ponded_depth_max=pdm_b,
+                              moisture=moisture, layer_water=layer_water)
         ctx.ens, ctx.mask, ctx.ws = ens, mask, ws
-        ctx.save_for_backward(*res._keep[:3])
-        ctx.pdm_b = res._keep[4]
+        ctx.save_for_backward(a, n_, k, pdm_b)
         ctx.pdm_shape = None if pdm is None else tuple(pdm.shape)
         ctx.want_pdm = pdm is not None and ctx.needs_input_grad[3]
-        ctx.in_shapes = (alpha.shape, n.shape, ksat.shape)
+        ctx.in_dims = (alpha.dim(), n.dim(), ksat.dim())
         ctx.mark_non_differentiable(res.status, res.crash_step, res.start_volume)
         # an output the loss does not use gets no gradient (None): the soil-moisture outputs then pass NULL to the
         # reverse pass, which leaves it exactly as without them; per_step and sums keep their zero gradients
@@ -372,17 +379,16 @@ class _LGARFunction(torch.autograd.Function):
     def backward(ctx, g_per_step, g_sums, _gsv, _gst, _gcs, g_moisture, g_layer_water):
         L_ = _capi.lib()
         ens: ColumnEnsemble = ctx.ens
-        alpha, n, ksat = ctx.saved_tensors
+        alpha, n, ksat, pdm = ctx.saved_tensors
         if g_per_step is None:
-            g_per_step = torch.zeros(bin(ctx.mask).count("1"), ens.num_steps, ens.num_columns, dtype=F64, device=ens.device)
+            g_per_step = torch.zeros(ctx.mask.bit_count(), ens.num_steps, ens.num_columns, dtype=F64, device=ens.device)
         if g_sums is None:
             g_sums = torch.zeros(NUM_OUTPUTS, ens.num_columns, dtype=F64, device=ens.device)
         dev = ens.device
         Lr, B = ens.num_layers, ens.num_columns
-        p = ens.problem(alpha, n, ksat, ctx.pdm_b)
-        sa, sn, sk = ctx.in_shapes
+        p = ens.problem(alpha, n, ksat, pdm)
         pdm_shared = ctx.pdm_shape is None or int(torch.Size(ctx.pdm_shape).numel()) == 1
-        shared = len(sa) == 1 and len(sn) == 1 and len(sk) == 1 and (pdm_shared or not ctx.want_pdm)
+        shared = ctx.params_shared and (pdm_shared or not ctx.want_pdm)
         g = _capi.Gradients()
         gshape = (Lr,) if shared else (Lr, B)
         ga = torch.zeros(gshape, dtype=F64, device=dev)
@@ -421,12 +427,12 @@ class _LGARFunction(torch.autograd.Function):
         ens.last_tape_overflow = overflow
         ens.last_reverse_counters = counters
 
-        def shape_back(gr, shp):
-            return gr.sum(dim=1) if (len(shp) == 1 and gr.dim() == 2) else gr
+        # a [L] parameter next to [L,B] ones (or next to a per-column ponded_depth_max leaf) got per-column gradients
+        ga, gn, gk = (gr.sum(dim=1) if (dim == 1 and gr.dim() == 2) else gr for gr, dim in zip((ga, gn, gk), ctx.in_dims))
         gp_out = None
         if gp is not None:
             gp_out = (gp.sum() if (pdm_shared and gp.numel() > 1) else gp).reshape(ctx.pdm_shape)
-        return shape_back(ga, sa), shape_back(gn, sn), shape_back(gk, sk), gp_out, None, None, None, None
+        return ga, gn, gk, gp_out, None, None, None, None
 
 
 def lgar_columns(alpha, n, ksat, ens: ColumnEnsemble, outputs=("runoff", "percolation"), ponded_depth_max=None):
@@ -444,18 +450,11 @@ def lgar_columns(alpha, n, ksat, ens: ColumnEnsemble, outputs=("runoff", "percol
         raise ValueError('"moisture" needs ColumnEnsemble(moisture_depths=...)')
     outputs = tuple(nm for nm in outputs if nm not in ("moisture", "layer_water"))
     mask = output_mask(outputs)
-    dev = ens.device
-    a = torch.as_tensor(alpha, dtype=F64).to(dev)
-    nn_ = torch.as_tensor(n, dtype=F64).to(dev)
-    k = torch.as_tensor(ksat, dtype=F64).to(dev)
-    if not (a.dim() == 1 and nn_.dim() == 1 and k.dim() == 1):  # mixed: expand the shared ones (autograd sums them)
-        a = a if a.dim() == 2 else a.unsqueeze(1).expand(ens.num_layers, ens.num_columns)
-        nn_ = nn_ if nn_.dim() == 2 else nn_.unsqueeze(1).expand(ens.num_layers, ens.num_columns)
-        k = k if k.dim() == 2 else k.unsqueeze(1).expand(ens.num_layers, ens.num_columns)
-    pdm = None if ponded_depth_max is None else torch.as_tensor(ponded_depth_max, dtype=F64).to(dev)
-    per_step, sums, sv, st, cs, moist, lw = _LGARFunction.apply(a.contiguous(), nn_.contiguous(), k.contiguous(), pdm,
-                                                                ens, mask, moisture, layer_water)
-    out = {name: per_step[bin(mask & ((1 << OUT_NAMES.index(name)) - 1)).count("1")] for name in outputs}
+    # on the device before autograd sees them: their gradients come back to where the caller's tensors live
+    a, n_, k = (torch.as_tensor(x, dtype=F64).to(ens.device) for x in (alpha, n, ksat))
+    pdm = None if ponded_depth_max is None else torch.as_tensor(ponded_depth_max, dtype=F64).to(ens.device)
+    per_step, sums, sv, st, cs, moist, lw = _LGARFunction.apply(a, n_, k, pdm, ens, mask, moisture, layer_water)
+    out = {name: per_step[output_row(mask, OUT_NAMES.index(name))] for name in outputs}
     out.update(sums=sums, start_volume=sv, status=st, crash_step=cs)
     if moisture:
         out["moisture"] = moist

@@ -33,7 +33,7 @@ import torch.nn as nn
 
 from . import _capi
 from .columns import ColumnEnsemble, check_moisture_depths, forward_raw, lgar_columns
-from ._capi import OUT_NAMES, STATUS_NAMES
+from ._capi import CAPACITY_STATUSES, OUT_NAMES, status_message  # noqa: F401 (CAPACITY_STATUSES: importable from here)
 
 # data/utils.py:108-180 read_test_params (== alpha, n, Ks columns of data/vG_default_params.dat; rows 12-17 are
 # Phillipsburg P-1..3 and Bushland B-1..3)
@@ -43,10 +43,6 @@ N_TABLE = (1.25, 1.42, 1.47, 1.75, 3.18, 1.21, 1.33, 1.45, 1.68, 1.32, 1.52, 1.6
            1.6858, 1.299, 1.6151, 1.3579, 1.5276, 1.4585)
 KSAT_TABLE = (0.612, 0.3348, 0.504, 4.32, 26.64, 0.468, 0.54, 1.584, 1.836, 0.432, 0.468, 0.756,
               0.45, 0.07, 0.45, 0.07, 0.02, 0.2)
-
-
-# statuses that are capacity limits of the CUDA library rather than exceptions of the reference
-CAPACITY_STATUSES = (STATUS_NAMES.index("FRONT_OVERFLOW"), STATUS_NAMES.index("ITER_CAP"))
 
 
 def _get(cfg, path, default=None):
@@ -155,7 +151,7 @@ class dpLGAR(nn.Module):
         self._started = True
         st = int(res.status[0])
         if st != 0:
-            raise RuntimeError(f"LGAR column status {STATUS_NAMES[st]} (the reference raises here)")
+            raise RuntimeError(status_message(0, st))
         v = {name: res[name][0, 0].cpu() for name in OUT_NAMES}
         for name in ("precip", "PET", "AET", "infiltration", "runoff", "percolation", "giuh_runoff", "discharge"):
             setattr(self, name, getattr(self, name) + v[name])
@@ -187,10 +183,7 @@ class dpLGAR(nn.Module):
             st = out["status"]
             if bool((st != 0).any()):
                 first = int((st != 0).nonzero()[0, 0])
-                code, step = int(st[first]), int(out["crash_step"][first])
-                kind = ("a capacity limit of the CUDA library, not a reference exception" if code in CAPACITY_STATUSES
-                        else "the reference raises here")
-                msg = f"LGAR column {first}: status {STATUS_NAMES[code]} at forcing step {step} ({kind})"
+                msg = status_message(first, int(st[first]), int(out["crash_step"][first]))
                 if on_status == "raise":
                     raise RuntimeError(msg)
                 import warnings

@@ -147,3 +147,30 @@ def test_two_ranks_equal_two_sites_in_one_process():
         for got, w in zip(out[r][:-1], want):
             np.testing.assert_allclose(got, w, rtol=1e-12, atol=1e-15)
         assert out[r][-1] == pytest.approx(ag.history[0][1], rel=1e-12)
+
+
+def _nan_worker(rank, world, port, out):
+    os.environ["MASTER_ADDR"] = "127.0.0.1"
+    os.environ["MASTER_PORT"] = str(port)
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    rng = np.random.default_rng(5)
+    x = np.abs(rng.normal(size=(2, 48, 2))) * 0.3
+    x[1, 20, 0] = np.nan                            # rank 1's record gives a NaN runoff, hence a NaN gradient
+    ag = A.DifferentiableLGAR(_cfg(epochs=1), model=ToyModel(), x=x[rank])
+    before = [p.detach().clone() for p in ag.model.parameters()]
+    try:
+        ag.train_one_epoch()
+        out[rank] = "stepped"
+    except RuntimeError as e:
+        ps = list(ag.model.parameters())
+        out[rank] = ("raised", all(torch.equal(p.detach(), b) for p, b in zip(ps, before)),
+                     all(p.grad is None for p in ps), len(ag.history), str(e))
+    dist.destroy_process_group()
+
+
+def test_two_ranks_refuse_a_nan_gradient_together():
+    port = 35000 + os.getpid() % 2000
+    out = mp.Manager().dict()
+    mp.spawn(_nan_worker, args=(2, port, out), nprocs=2, join=True)
+    for r in range(2):
+        assert out[r][:4] == ("raised", True, True, 0), out[r]

@@ -56,3 +56,30 @@ def test_calibration_step_world2_equals_single_process():
         assert abs(l - float(loss)) < 1e-12
         np.testing.assert_allclose(q0, want0, rtol=1e-12)
         assert abs(q1 - want1) < 1e-12
+
+
+def _nan_worker(rank, world, port, out):
+    os.environ["MASTER_ADDR"] = "127.0.0.1"
+    os.environ["MASTER_PORT"] = str(port)
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    data = torch.arange(8, dtype=torch.float64) / 8
+    p = [torch.nn.Parameter(torch.tensor([0.3, 0.7], dtype=torch.float64)), torch.nn.Parameter(torch.tensor(1.5, dtype=torch.float64))]
+    before = [q.detach().clone() for q in p]
+    opt = torch.optim.SGD(p, lr=0.1)
+    poison = float("nan") if rank == 1 else 1.0     # rank 1's shard produces a NaN gradient
+    ens = lambda ps: (ps[0][0] * data + ps[0][1]) ** 2 * ps[1] * poison
+    try:
+        parallel.calibration_step(p, ens, lambda y: (y.sum(), 8), opt)
+        out[rank] = "stepped"
+    except RuntimeError as e:
+        unchanged = all(torch.equal(q.detach(), b) for q, b in zip(p, before))
+        out[rank] = ("raised", unchanged, all(q.grad is None for q in p), str(e))
+    dist.destroy_process_group()
+
+
+def test_calibration_step_refuses_a_nan_gradient_on_every_rank():
+    port = 33000 + os.getpid() % 2000
+    out = mp.Manager().dict()
+    mp.spawn(_nan_worker, args=(2, port, out), nprocs=2, join=True)
+    for r in range(2):
+        assert out[r][:3] == ("raised", True, True), out[r]

@@ -132,6 +132,23 @@ def test_window_argument_checks():
         forward_raw(ens, we.alpha, we.n, we.ksat, window=(0, 25), keep_checkpoints=True)
 
 
+def test_overflow_fallback_needs_the_whole_record():
+    """The 32-front rerun starts at row 0: with a window that is not the whole record forward_raw raises before it
+    launches anything, so the previous window's results and state are left as they were."""
+    from lgar_b200 import forward_raw
+    we, ens = _setup(B=64, T=50, sites=1)
+    res, ws = forward_raw(ens, we.alpha, we.n, we.ksat, window=(0, 20), num_fronts=True)
+    torch.cuda.synchronize()
+    before = [t.clone() for t in (res.per_step, res.sums, res.start_volume, res.status, res.crash_step, res.num_fronts, ws)]
+    for window in ((20, 50), (0, 20)):
+        with pytest.raises(ValueError):
+            forward_raw(ens, we.alpha, we.n, we.ksat, window=window, num_fronts=True, workspace=ws, into=res,
+                        overflow_fallback=True)
+    torch.cuda.synchronize()
+    after = (res.per_step, res.sums, res.start_volume, res.status, res.crash_step, res.num_fronts, ws)
+    assert all(torch.equal(a.view(torch.uint8), b.view(torch.uint8)) for a, b in zip(after, before))
+
+
 def test_forward_host_entry_point():
     """lgar_forward_host: every pointer is a HOST pointer; the library stages, runs and copies back."""
     from lgar_b200 import forward_raw, _capi, output_mask, OUT_NAMES

@@ -161,6 +161,39 @@ def test_front_overflow_fallback():
     assert torch.equal(fb["runoff"][:, ok].contiguous().view(torch.int64), ref["runoff"][:, ok].contiguous().view(torch.int64))
 
 
+def test_subset_carries_every_field():
+    """ColumnEnsemble.subset (the 32-front rerun's sub-ensemble): per-column fields are those of the indexed columns,
+    the forcing is shared, the placement, resume and the last backward pass's results are not carried, every other
+    field equals the parent's.  A field added to ColumnEnsemble that subset does not handle fails here."""
+    import dataclasses
+    from lgar_b200 import workloads
+    B = 100
+    we = workloads.synthetic_sites_ensemble(B=B, T=20, sites=3, rank=0)
+    ens = _ens(we, initial_psi=np.linspace(1000.0, 3000.0, B), ponded_depth_max=0.5, moisture_depths=(5.0, 30.0),
+               nint=60, iter_cap=12345, use_closed_form_G=True, reverse_counters=True, resume=True)
+    ens.balance(we.ksat)
+    ens.last_tape_overflow = torch.zeros(B, dtype=torch.int32, device="cuda")
+    idx = torch.tensor([3, 17, 64, 99], device="cuda")
+    sub = ens.subset(idx, max_fronts=32)
+    default = {f.name: (f.default_factory() if f.default_factory is not dataclasses.MISSING else f.default)
+               for f in dataclasses.fields(ens)}
+    for f in dataclasses.fields(ens):
+        got, parent = getattr(sub, f.name), getattr(ens, f.name)
+        if f.name in ("column_order", "resume", "_keep") or f.name.startswith("last_"):
+            assert not isinstance(got, torch.Tensor) and got == default[f.name], f.name
+        elif f.name == "max_fronts":
+            assert got == 32
+        elif f.name == "forcing":
+            assert got.data_ptr() == parent.data_ptr()
+        elif isinstance(parent, torch.Tensor) and parent.shape[-1:] == (B,):
+            assert torch.equal(got, parent[..., idx]), f.name
+        elif isinstance(parent, torch.Tensor):
+            assert torch.equal(got, parent), f.name
+        else:
+            assert got == parent, f.name
+    assert sub.num_columns == 4 and sub.num_layers == ens.num_layers
+
+
 def test_flat_column_mass_run_ends_with_iter_cap_quickly():
     """A column whose free-drainage front has the theta of the front below it: the column mass does not depend on the
     depth check_column_mass steps (Layer.py:681-701), the reference never leaves that loop, this library answers with

@@ -119,3 +119,25 @@ def test_valid_calls_get_past_the_argument_rules():
     assert _backward(_problem(S=6, chunk_steps=85)) in (E_NO_DEVICE, E_WORKSPACE)
     assert _capi.lib().lgar_workspace_bytes(C.byref(_problem(S=6, chunk_steps=85)), 1) > 0
     assert _capi.lib().lgar_workspace_bytes(C.byref(_problem(max_fronts=32)), 1) > 0
+
+
+def test_output_rows_are_the_popcount_below_k():
+    from lgar_b200.columns import output_row
+    for mask in range(1 << _capi.NUM_OUTPUTS):
+        rows = [sum((mask >> j) & 1 for j in range(k)) for k in range(_capi.NUM_OUTPUTS)]
+        assert [output_row(mask, k) for k in range(_capi.NUM_OUTPUTS)] == rows
+
+
+def test_status_policy():
+    names = _capi.STATUS_NAMES
+    assert _capi.FRONT_OVERFLOW == names.index("FRONT_OVERFLOW") == 6
+    assert set(_capi.CAPACITY_STATUSES) == {names.index("FRONT_OVERFLOW"), names.index("ITER_CAP")}
+    from lgar_b200 import model
+    assert model.CAPACITY_STATUSES == _capi.CAPACITY_STATUSES
+    for code in range(1, len(names)):
+        msg = _capi.status_message(17, code, 42)
+        assert msg.startswith(f"LGAR column 17: status {names[code]} at forcing step 42")
+        capacity = names[code] in ("FRONT_OVERFLOW", "ITER_CAP")
+        assert ("capacity limit" in msg and "max_fronts=32" in msg and "mask" in msg) == capacity
+        assert ("the reference raises here" in msg) == (not capacity)
+    assert _capi.status_message(0, names.index("NAN")) == "LGAR column 0: status NAN (the reference raises here)"
